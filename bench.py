@@ -1,7 +1,10 @@
 #!/usr/bin/env python
 """bench.py -- env-steps/s of the TaskEnv step on B200 (BASELINE.json metric), one JSON line on stdout.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W]            our arm (CUDA path through the C ABI)
+  python bench.py [--gpus N] [--steps K] [--warmup W]            our arm (CUDA path through the C ABI); --steps / --warmup are its
+                                                                  timed / untimed passes and are refused by the other arms below
+  python bench.py --dump-outputs DIR [...]                        our arm, then what its last timed pass returned, as DIR/<name>.npy
+                                                                  (this arm only: rollout / train / reference have no dump)
   python bench.py --impl reference [...]                          the reference's CPU implementation of the path
   torchrun --nproc-per-node N bench.py --gpus N ...               N > 1 (one rank per GPU, env shards, no collective on the data path);
                                                                   launched plainly with --gpus N > 1 it re-executes itself under torchrun
@@ -47,8 +50,8 @@ FALLBACK_HBM_GBS = 6650.0           # /opt/skills/guides/B200_PROFILING.md fallb
 def parse():
     p = argparse.ArgumentParser()
     p.add_argument("--gpus", type=int, default=1)
-    p.add_argument("--steps", type=int, default=2000)
-    p.add_argument("--warmup", type=int, default=200)
+    p.add_argument("--steps", type=int, help="timed passes of the env step (default 2000; --mode env, --impl ours only)")
+    p.add_argument("--warmup", type=int, help="untimed passes before them (default 200; --mode env, --impl ours only)")
     p.add_argument("--impl", default="ours", choices=["ours", "reference"])
     p.add_argument("--envs", type=int, default=65536, help="envs per GPU (weak scaling)")
     p.add_argument("--total-envs", type=int, default=0, help="BASELINE configs[3]: this many envs in total, sharded evenly over the GPUs "
@@ -72,7 +75,19 @@ def parse():
     p.add_argument("--no-compact", action="store_true", help="--mode rollout/train: every decision forwards the whole batch (default: only the envs "
                    "that are still playing, at the fractions of the batch TrainerConfig.rollout_fractions names)")
     p.add_argument("--eager", action="store_true", help="--mode rollout/train: eager decision loop instead of the CUDA-graph replay")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one returned to its caller as DIR/<name>.npy "
+                   "(float32; a fixed sample of the envs of rank 0 when the batch would exceed 64 MB), so that two builds can be compared output for output.  "
+                   "--mode env, --impl ours only: the rollout / train modes and the reference arm have no dump")
+    args = p.parse_args()
+    if args.mode != "env" or args.impl != "ours":
+        # the rollout / train modes time --iters iterations and the reference arm runs for --cpu-seconds
+        given = [f for f, v in (("--steps", args.steps), ("--warmup", args.warmup), ("--dump-outputs", args.dump_outputs)) if v is not None]
+        if given:
+            p.error(f"{', '.join(given)}: --mode env --impl ours only (--mode rollout/train time --iters iterations, --impl reference "
+                    "runs for --cpu-seconds)")
+    args.steps = 2000 if args.steps is None else args.steps
+    args.warmup = 200 if args.warmup is None else args.warmup
+    return args
 
 
 def metric_name(args):
@@ -94,6 +109,28 @@ def algorithmic_bytes(A, T, M=5, w=8):
     s_dyn = T * (M * (1 + w) + 2 * w + 5) + A * (3 * w + 4) + 40
     s_obs = 4 * 6 * A + 4 * 5 * (T + 1) + (T + 1)
     return s_static + 2 * s_dyn + s_obs + 16
+
+
+DUMP_LIMIT = 64_000_000
+
+
+def dump_outputs(out_dir, env, first_gid):
+    """What BatchedTaskEnv.step() hands its caller, as left by the last timed step: the next leader's agent / task observation and
+    mask, the next leader, the step reward and done flag, and the action the in-kernel policy took.  All float32 (the integer and
+    uint8 outputs are small enough to be exact).  When the whole batch would pass DUMP_LIMIT, the same envs are kept every run: a
+    sample drawn from a fixed seed; env_index.npy (float64) holds their global ids."""
+    import numpy as np
+    import torch
+    outs = {"agent_obs": env.agent_obs, "task_obs": env.task_obs, "mask": env.mask_u8, "next_leader": env.leader,
+            "reward": env.reward, "done": env.done_u8, "action": env.used_action}
+    per_env = 8 + 4 * sum(t[0].numel() for t in outs.values())
+    n = min(env.B, (DUMP_LIMIT - 4096) // per_env)                 # 4 KB of room for the .npy headers
+    idx = np.arange(env.B) if n == env.B else np.sort(np.random.default_rng(0).choice(env.B, n, replace=False))
+    sel = torch.from_numpy(idx).to(env.device)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "env_index.npy"), (idx + first_gid).astype(np.float64))
+    for name, t in outs.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.index_select(0, sel).float().cpu().numpy())
 
 
 class ClockSampler:
@@ -194,12 +231,12 @@ def run_reference(args):
     t0 = time.perf_counter()
     # warm-up
     cpu_rollout(args.agents, args.tasks, args.policy, 0.5)
-    # K "steps", each a bounded sample of the workload: the whole run is sized to ~args.cpu_seconds of wall time on all host
-    # threads, i.e. one "step" = total/K decisions spread over the thread pool
+    # a bounded sample of the workload: the run is sized to ~args.cpu_seconds of wall time on all host threads (it has no passes to
+    # count, so the line reports no steps / ms_per_step)
     rate, cores, total, dt, rate1 = cpu_rollout(args.agents, args.tasks, args.policy, args.cpu_seconds)
     line = {
-        "metric": metric_name(args), "value": rate, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup,
-        "ms_per_step": 1e3 * dt / max(args.steps, 1), "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
+        "metric": metric_name(args), "value": rate, "unit": UNIT, "n_gpus": args.gpus, "steps": None, "warmup": None,
+        "ms_per_step": None, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
         "dtype": "f64", "data": "synthetic", "impl": "reference",
         "config": {"workload": f"synthetic {args.agents}A/{args.tasks}T TaskEnv, {args.policy} policy, obs+mask built every decision",
                    "env_steps_timed": total, "threads": cores},
@@ -272,6 +309,8 @@ def run_ours(args):
     barrier()
     ms = ev0.elapsed_time(ev1)
     clocks = sampler.stop(w0, w1) if rank == 0 else None
+    if args.dump_outputs and rank == 0:                              # before the e2e legs re-seed and reset the env
+        dump_outputs(args.dump_outputs, env, first_gid)
     env_steps = env.total_steps() - steps0
     episodes_timed = env.total_episodes() - episodes0
     total_steps, ms_max = reduce_job_totals(env_steps, ms)          # env-steps summed over the ranks, time = max over the ranks

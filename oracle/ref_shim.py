@@ -1,6 +1,6 @@
-"""oracle/ref_shim.py -- import the REAL reference TaskEnv (read-only tree at /root/reference) in the build
-container.  TEST INFRASTRUCTURE ONLY; it cannot travel to the GPU box (the reference tree is absent there), so
-only oracle/make_golden.py and the `reference`-marked CPU tests use it.
+"""oracle/ref_shim.py -- import the REAL reference TaskEnv (a read-only checkout of the original project, found at
+$DCMRTA_REFERENCE).  TEST INFRASTRUCTURE ONLY: the tests do not use it; the oracle/make_*golden.py generators record
+tests/golden/ from the reference through it.
 
 Shims (SURVEY.md App. B): (1) stub matplotlib, which env/task_env.py:2-5 imports at module top and this image
 lacks; (2) remap the pickles' `__main__.TaskEnv` to env.task_env.TaskEnv; (3) normalise an unpickled env

@@ -11,19 +11,14 @@ if str(ROOT) not in sys.path:
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box with -m gpu)")
-    config.addinivalue_line("markers", "reference: needs the read-only reference tree at /root/reference (build container only)")
 
 
 def pytest_collection_modifyitems(config, items):
-    from oracle import ref_shim
-    have_ref = ref_shim.available()
     try:
         import torch
         have_gpu = torch.cuda.is_available()
     except Exception:
         have_gpu = False
     for item in items:
-        if "reference" in item.keywords and not have_ref:
-            item.add_marker(pytest.mark.skip(reason="reference tree not present on this box"))
         if "gpu" in item.keywords and not have_gpu:
             item.add_marker(pytest.mark.skip(reason="no CUDA device"))

@@ -100,29 +100,6 @@ def test_sweep_traces_digest_exact():
         assert np.array_equal(fin, tr.z[f"finished/{ep['name']}"])
 
 
-@pytest.mark.reference
-def test_oracle_live_against_reference():
-    """Build container only: step the real reference and the C oracle in lock-step (fresh draw, not a stored vector)."""
-    from oracle import ref_shim as R
-    for i, policy, seed in ((3, "random", 77), (11, "greedy", 78)):
-        env = R.load_pickle(i)
-        ia = R.instance_arrays(env)
-        recs = []
-        trace, reward, fin = R.run_reference_episode(
-            env, policy, seed, on_decision=lambda e, l, m, a, t: recs.append((l, m.copy(), a.copy(), t.copy(), R.canonical_state(e))))
-        o = OracleEnv.make(**ia)
-        n = len(trace["leader"])
-        o.fused_reset(trace["leader"][0])
-        for k in range(n):
-            l, m, a, t, st = recs[k]
-            assert np.array_equal(o.mask(), m) and np.array_equal(o.agent_status(l), a) and np.array_equal(o.task_status(l), t)
-            assert not canon.diff_states(o.export(8), st)
-            rc, r, done, _, _ = o.fused_step(trace["action"][k], trace["followers"][k], trace["leader"][k + 1] if k + 1 < n else -1)
-            assert rc == 0 and r == trace["reward"][k]
-        m, f = o.episode_metrics()
-        assert m["reward"] == reward and np.array_equal(f.astype(bool), fin)
-
-
 def test_builtin_policies_terminate_and_are_deterministic():
     inst = pickle_instances()[5]
     runs = []
