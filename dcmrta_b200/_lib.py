@@ -14,7 +14,8 @@ _LIB = None
 STATUS = {0: "DCM_OK", -1: "DCM_ERR_ARG", -2: "DCM_ERR_SHAPE", -3: "DCM_ERR_DEVICE", -4: "DCM_ERR_CUDA", -5: "DCM_ERR_STATE",
           -6: "DCM_ERR_NOMEM"}
 
-FLAG_AUTO_RESET, FLAG_REGENERATE = 1, 2
+FLAG_AUTO_RESET, FLAG_REGENERATE, FLAG_INDIVIDUAL = 1, 2, 4
+PROTOCOL = {"LF": 0, "IA": FLAG_INDIVIDUAL}     # leader-follower (worker.py:45-85) / individual agent (worker.py:159-198)
 POLICY = {"external": 0, "random": 1, "greedy": 2}
 ENV_DONE, ENV_FINISHED, ENV_STUCK = 1, 2, 4
 ENV_ERR_OVERFLOW, ENV_ERR_ACTION, ENV_ERR_FOLLOW, ENV_ERR_LEADER = 16, 32, 64, 128

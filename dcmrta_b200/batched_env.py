@@ -3,7 +3,8 @@
 `BatchedTaskEnv` owns one dcm_env handle (include/dcmrta.h) and the policy-input tensors the step kernel writes
 into: agent rows [B,A,6] fp32, task rows [B,T+1,5] fp32, mask [B,T+1] bool -- exactly what
 AttentionNet.forward(tasks, agents, mask) consumes (reference attention.py:288, worker.py:62-69).  One `step()`
-is one leader decision for every env (reference worker.py:45-85).  PyTorch is used only for device memory and
+is one leader decision for every env (reference worker.py:45-85) -- or, with protocol="IA", one individual decision
+(worker.py:159-198 run_test_IS: every decider acts alone, in ascending id order).  PyTorch is used only for device memory and
 streams; all simulation work happens in the CUDA library.  There is no CPU fallback.
 """
 from __future__ import annotations
@@ -33,16 +34,24 @@ def _ptr(t):
 
 
 class BatchedTaskEnv:
-    """B environments of A agents / T tasks stepped in lock-step on one GPU."""
+    """B environments of A agents / T tasks stepped in lock-step on one GPU.
+
+    protocol: "LF" leader-follower (worker.py:45-85, what training plays) or "IA" individual agent (worker.py:159-198,
+    DCM_FLAG_INDIVIDUAL): `leader` is then the agent that acts next, followers must not be given, and an episode takes one
+    step per individual decision: with the greedy policy on the bundled 20A/50T instances 185 on average (at most 259) against
+    99 (at most 190) under LF, so size rollout horizons accordingly."""
 
     def __init__(self, B, A, T, M=5, device=0, auto_reset=False, regenerate=False, velocity=0.2, max_wait=10.0,
-                 max_time=100.0, seed=0, first_gid=0):
+                 max_time=100.0, seed=0, first_gid=0, protocol="LF"):
+        if protocol not in _lib.PROTOCOL:
+            raise ValueError(f"protocol must be 'LF' or 'IA', not {protocol!r}")
         if not torch.cuda.is_available():
             raise _lib.DcmError(-3, "BatchedTaskEnv needs a CUDA device; there is no CPU fallback")
         self.B, self.A, self.T, self.M = int(B), int(A), int(T), int(M)
         self.device = torch.device("cuda", int(device) if not isinstance(device, torch.device) else device.index or 0)
         self.auto_reset = bool(auto_reset)
-        flags = (_lib.FLAG_AUTO_RESET if auto_reset else 0) | (_lib.FLAG_REGENERATE if regenerate else 0)
+        self.protocol = protocol
+        flags = (_lib.FLAG_AUTO_RESET if auto_reset else 0) | (_lib.FLAG_REGENERATE if regenerate else 0) | _lib.PROTOCOL[protocol]
         h = C.c_void_p()
         check(lib().dcm_create(C.byref(h), self.device.index, self.B, self.A, self.T, self.M, flags))
         self._h = h

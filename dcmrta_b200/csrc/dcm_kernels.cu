@@ -4,6 +4,7 @@
 //   k_step          dcm_step: one leader decision per env per launch, thread / env -- action application, coalition update, agent
 //                   update, slot advance, leader choice; two rounds of loads, the rest from registers and a per-thread shared-memory
 //                   scratch filled with cp.async (step_env)                                                          (hot path 1/3)
+//   k_step_ia       the same step for handles created with DCM_FLAG_INDIVIDUAL: one individual decision per env (worker.py:159-198)
 //   k_episode_list  episode accounting + restart of the envs whose episode just ended, warp / env, beside k_obs_tile  (hot path 2/3)
 //   k_obs_tile      observation + mask builder, block / tile: TMA bulk loads of the tile's arrays, rows from shared memory, TMA bulk
 //                   stores straight into the policy's input tensors; launched programmatically after k_step           (hot path 3/3)
@@ -124,7 +125,9 @@ template <int TW> __device__ __forceinline__ void st_state_all(const TC& c, cons
 // The members join, the joined task is evaluated (t_eval_task with the head in registers) and the movers' next_decision is set
 // (t_agent_update with `known`) from registers; the slot advance scans next_decision in shared memory.  What still goes to memory
 // are the rare paths: a re-visit, a removal, the waiting-coalition scan when the earliest waiting member may give up.
-template <int TW>
+// IA: the individual-agent protocol of handles created with DCM_FLAG_INDIVIDUAL (worker.py:159-198), a compile-time switch so that the
+// leader-follower kernel is the same code with or without it.
+template <int TW, bool IA>
 __device__ __forceinline__ unsigned step_env(const EnvArgs& E, const StepArgs& F, int b, double* nds, unsigned* nws, double* tmp) {
     TC c = make_tc(E, b); c.nds = F.use_nds ? nds : nullptr; c.nws = nws; c.tmp = tmp;
     const int A = c.A, T = c.T;
@@ -172,7 +175,9 @@ __device__ __forceinline__ unsigned step_env(const EnvArgs& E, const StepArgs& F
             tr.n = (int)(ip.y & 0xffu); tr.status = (int)(signed char)((ip.y >> 8) & 0xffu); tr.req = (int)((ip.y >> 16) & 0xffu);
         } else { tx = EL(c, s_dep, 2, 0); ty = EL(c, s_dep, 2, 1); }
     }
-    int want = 0; u64 g = group & ~(1ull << leader);                          // task_env.py:328
+    // task_env.py:328.  Individual agent (DCM_FLAG_INDIVIDUAL, worker.py:170-186): the leader moves alone whatever the stored group
+    // holds (dcm_import_state may install a leader-follower record in the middle of a slot): no followers, and the depot takes only it
+    int want = 0; u64 g = IA ? 0ull : group & ~(1ull << leader);
     const int* fp = F.followers ? F.followers + (size_t)b * F.fstride : nullptr;
     if (ok) {
         const int vacancy = action == 0 ? __popcll(group) : tr.status;        // :327
@@ -269,7 +274,8 @@ __device__ __forceinline__ unsigned step_env(const EnvArgs& E, const StepArgs& F
         t_update_and_advance<TW>(c, st, now, pending, flags, node_of, tr, movers, arrival);    // worker.py:74-76, then :85 / :45-51 while nobody is pending
         if (flags & ENV_DONE) { leader = -1; group = 0; }                     // episode accounting / restart: k_episode
         else {
-            group = f_current_group(c, node_of, pending);                     // task_env.py:291-298
+            group = IA ? pending & (0ull - pending)                           // the lowest pending id acts next (worker.py:170)
+                       : f_current_group(c, node_of, pending);                // task_env.py:291-298
             if (inj >= 0) {
                 if (inj < A && ((group >> inj) & 1ull)) leader = inj;
                 else { flags |= ENV_ERR_LEADER; leader = ctz64(group); }
@@ -284,7 +290,8 @@ __device__ __forceinline__ unsigned step_env(const EnvArgs& E, const StepArgs& F
         // The episode kernel restarts this env; the first leader of the new episode (episode_env, worker.py:54) is a function of the
         // RNG contract alone, so the OUTPUT carries it already: next_leader, reward and done are then final when k_step ends and
         // dcm_step_host sends them to the host while the episode and observation kernels run.  (The stored leader stays -1.)
-        if (inj >= 0) leader_out = inj < A ? inj : 0;
+        if (IA) leader_out = 0;                                               // agent 0 starts (episode_env flags any other injected leader)
+        else if (inj >= 0) leader_out = inj < A ? inj : 0;
         else if (A == 1) leader_out = 0;
         else leader_out = kth_bit(A >= 64 ? ~0ull : ((1ull << A) - 1), pick(draw_block(rng, episode + 1, 0, 0).y, A));
     }
@@ -304,9 +311,8 @@ __device__ __forceinline__ unsigned step_env(const EnvArgs& E, const StepArgs& F
 #define STEP_NDS_MAX_AGENTS 24
 __host__ __device__ inline size_t step_smem_bytes(int A, int ANB, bool nds) { return (size_t)STEP_THREADS * (8 * (size_t)(SCR_TMP + (nds ? A : 0)) + (size_t)ANB); }
 
-template <int TW>
-__global__ void __launch_bounds__(STEP_THREADS, 7) k_step(const __grid_constant__ EnvArgs E, const __grid_constant__ StepArgs F) {
-    extern __shared__ __align__(16) unsigned char step_smem[];
+template <int TW, bool IA>
+__device__ __forceinline__ void step_pass(const EnvArgs& E, const StepArgs& F, unsigned char* step_smem) {
     const int b = blockIdx.x * STEP_THREADS + threadIdx.x;
     unsigned flags = 0;
     // programmatic dependent launch: the observation kernel that follows in the stream may become resident (and run its prologue) as SM
@@ -314,7 +320,7 @@ __global__ void __launch_bounds__(STEP_THREADS, 7) k_step(const __grid_constant_
     asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
     if (F.trace && threadIdx.x == 0) { unsigned long long t; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t)); atomicMin(F.trace, t); }
     double* const tmp = (double*)step_smem + threadIdx.x; double* const nds = tmp + SCR_TMP * STEP_THREADS;
-    if (b < E.S.B) flags = step_env<TW>(E, F, b, nds, (unsigned*)(nds - threadIdx.x + (size_t)STEP_THREADS * (F.use_nds ? E.S.A : 0)) + threadIdx.x, tmp);
+    if (b < E.S.B) flags = step_env<TW, IA>(E, F, b, nds, (unsigned*)(nds - threadIdx.x + (size_t)STEP_THREADS * (F.use_nds ? E.S.A : 0)) + threadIdx.x, tmp);
     if (F.elist) {                                                            // envs whose episode just ended: one warp-aggregated append per warp that has any
         const bool need = (flags & ENV_DONE) && !(flags & ENV_ACCOUNTED);
         const unsigned m = __ballot_sync(0xffffffffu, need), lane = threadIdx.x & 31u;
@@ -327,6 +333,19 @@ __global__ void __launch_bounds__(STEP_THREADS, 7) k_step(const __grid_constant_
         if (b == 0) *F.ecount_next = 0;
     }
     if (F.trace && (threadIdx.x & 31) == 0) { unsigned long long t; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t)); atomicMax(F.trace + 1, t); }
+}
+
+template <int TW>
+__global__ void __launch_bounds__(STEP_THREADS, 7) k_step(const __grid_constant__ EnvArgs E, const __grid_constant__ StepArgs F) {
+    extern __shared__ __align__(16) unsigned char step_smem[];
+    step_pass<TW, false>(E, F, step_smem);
+}
+
+// dcm_step of a DCM_FLAG_INDIVIDUAL handle: one individual decision per env
+template <int TW>
+__global__ void __launch_bounds__(STEP_THREADS, 7) k_step_ia(const __grid_constant__ EnvArgs E, const __grid_constant__ StepArgs F) {
+    extern __shared__ __align__(16) unsigned char step_smem[];
+    step_pass<TW, true>(E, F, step_smem);
 }
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -535,13 +554,15 @@ __device__ __forceinline__ void episode_env(const EnvArgs& E, const EpiArgs& P, 
         AREC2(c, i, 0) = make_double2(dx, dy); AREC2(c, i, 1) = make_double2(0.0, 0.0);
         EL(c, a_nd, A, i) = 0.0; ANODE(c, i) = DCM_NODE_DEPOT; EL(c, a_nab, A, i) = 0;
     }
-    // ---- first slot (worker.py:45-51): every agent decides at t = 0 from the depot, nothing to update; one group
+    // ---- first slot (worker.py:45-51): every agent decides at t = 0 from the depot, nothing to update; one group (individual
+    // agent: every agent decides, agent 0 first, worker.py:170)
     const u64 all = A >= 64 ? ~0ull : ((1ull << A) - 1);
     unsigned nflags = P.mode == 0 ? ENV_FRESH : 0u; u64 pending = all, group = all; int leader;
     if (!alive) { nflags = ENV_DONE | ENV_ACCOUNTED; pending = 0; group = 0; leader = -1; }
     else {
         const int inj = P.leader_in ? P.leader_in[be] : -1;
-        if (inj >= 0) { if (inj < A) leader = inj; else { nflags |= ENV_ERR_LEADER; leader = 0; } }
+        if (E.cflags & DCM_FLAG_INDIVIDUAL) { group = 1; leader = 0; if (inj > 0) nflags |= ENV_ERR_LEADER; }
+        else if (inj >= 0) { if (inj < A) leader = inj; else { nflags |= ENV_ERR_LEADER; leader = 0; } }
         else if (A == 1) leader = 0;
         else { const Rng rng{E.seed, gid}; leader = kth_bit(all, pick(draw_block(rng, episode, 0, 0).y, A)); }   // worker.py:54
     }
@@ -1553,7 +1574,12 @@ int dcm_step(dcm_env* v, const int32_t* action, const int32_t* followers, int fs
     {
         F.use_nds = v->E.S.A <= STEP_NDS_MAX_AGENTS && !v->sw_step_no_nds;
         const int grid = grid_env(v, STEP_THREADS); const size_t smem = step_smem_bytes(v->E.S.A, v->E.S.ANB, F.use_nds != 0);
-        if (v->E.S.TW == 1) k_step<1><<<grid, STEP_THREADS, smem, s>>>(v->E, F);
+        if (v->E.cflags & DCM_FLAG_INDIVIDUAL) {
+            if (v->E.S.TW == 1) k_step_ia<1><<<grid, STEP_THREADS, smem, s>>>(v->E, F);
+            else if (v->E.S.TW == 2) k_step_ia<2><<<grid, STEP_THREADS, smem, s>>>(v->E, F);
+            else k_step_ia<4><<<grid, STEP_THREADS, smem, s>>>(v->E, F);
+        }
+        else if (v->E.S.TW == 1) k_step<1><<<grid, STEP_THREADS, smem, s>>>(v->E, F);
         else if (v->E.S.TW == 2) k_step<2><<<grid, STEP_THREADS, smem, s>>>(v->E, F);
         else k_step<4><<<grid, STEP_THREADS, smem, s>>>(v->E, F);
     }

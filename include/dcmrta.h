@@ -46,6 +46,12 @@ enum dcm_status {
 /* dcm_create flags */
 #define DCM_FLAG_AUTO_RESET  1u   /* an env that finishes inside dcm_step starts its next episode in the same call */
 #define DCM_FLAG_REGENERATE  2u   /* ... on a freshly generated instance (needs dcm_generate to have set the distribution) */
+/* Individual-agent decision protocol (worker.py:159-198 run_test_IS; RL_test.py METHOD = 'IA') instead of leader-follower
+ * (worker.py:45-85): every decider of a slot acts alone, in ascending id order -- no location groups, no leader draw, no
+ * followers.  One dcm_step call is then one INDIVIDUAL decision per env; the slot boundary (check_finished, next_decision,
+ * task_update, agent_update) is unchanged.  The flag belongs to the handle: restarted episodes follow it too.  The contract
+ * under this flag is stated at dcm_reset and dcm_step; the granular entry points and dcm_execute_by_route ignore it. */
+#define DCM_FLAG_INDIVIDUAL  4u
 
 /* built-in policies for dcm_step(policy=...) */
 #define DCM_POLICY_EXTERNAL  0    /* action_d supplies the actions (the attention policy of attention.py) */
@@ -97,7 +103,9 @@ int dcm_get_instances(dcm_env* env, double* task_xy_d, double* depot_xy_d, int32
  * that leader (worker.py:57-64).
  *   which_d        [B] u8, 1 = reset this env; NULL = all
  *   leader_in_d    [B] i32 leader to use (trace replay), NULL = Philox
- * outputs as for dcm_step (any may be NULL). */
+ * outputs as for dcm_step (any may be NULL).
+ * DCM_FLAG_INDIVIDUAL: the first agent to act is agent 0 and no random word is drawn; an injected leader other than 0 sets
+ * DCM_ENV_ERR_LEADER and agent 0 acts (a negative entry injects nothing, as in leader-follower mode). */
 int dcm_reset(dcm_env* env, const uint8_t* which_d, const int32_t* leader_in_d,
               float* agent_obs_d, float* task_obs_d, uint8_t* mask_d, int32_t* next_leader_d, void* stream);
 
@@ -112,13 +120,25 @@ int dcm_reset(dcm_env* env, const uint8_t* which_d, const int32_t* leader_in_d,
  *   next_leader_d [B] i32 (-1 when done; with DCM_FLAG_AUTO_RESET the first leader of the restarted episode)
  *   reward_d [B] f32 (task_env.py:341)   done_d [B] u8
  *   used_action_d [B] i32 or NULL: the action that was applied (what a built-in policy chose; -1 if the env did not step)
- * Envs already done (and not auto-reset) are left untouched and report done=1. */
+ * Envs already done (and not auto-reset) are left untouched and report done=1.
+ * DCM_FLAG_INDIVIDUAL (one call = one individual decision, worker.py:170-186):
+ *   - exactly one agent moves, the current leader, whatever the stored group holds (also for the depot action);
+ *   - next_leader is the lowest-id pending decider of the slot, or the first decider of the next slot; a restarted episode
+ *     (DCM_FLAG_AUTO_RESET) starts with agent 0.  No random word is drawn for leaders or followers; the built-in random policy
+ *     draws word 0 of block 0, as in leader-follower mode;
+ *   - followers_d must be NULL or all -1 for an env that moves to a task: otherwise DCM_ENV_ERR_FOLLOW is set and the env does
+ *     not step (as in leader-follower mode, the depot action ignores followers_d);
+ *   - an injected next_leader_in_d entry >= 0 must be that agent: otherwise DCM_ENV_ERR_LEADER is set and that agent acts
+ *     anyway (for a restart: agent 0);
+ *   - reward is -travel_time of the one mover (task_env.py:315);
+ *   - dcm_total_steps and the `decisions` metric count individual decisions. */
 int dcm_step(dcm_env* env, const int32_t* action_d, const int32_t* followers_d, int fstride,
              const int32_t* next_leader_in_d, int policy,
              float* agent_obs_d, float* task_obs_d, uint8_t* mask_d,
              int32_t* next_leader_d, float* reward_d, uint8_t* done_d, int32_t* used_action_d, void* stream);
 
-/* Same call with HOST buffers (pageable or pinned): actions are copied in -- or, from pinned memory, read in place by the step
+/* Same call with HOST buffers (pageable or pinned), under the same protocol as dcm_step (DCM_FLAG_INDIVIDUAL included: the next
+ * leader is then the agent that acts next): actions are copied in -- or, from pinned memory, read in place by the step
  * kernel --, outputs copied out, the call returns when the outputs are valid.  Any output pointer may be NULL (then it is not copied).  next_leader, reward and done are final when the
  * step kernel ends and are copied on a second stream while the episode and observation kernels still run.  The call runs on a
  * stream of the handle; it first waits (on the device, through an event) for the asynchronous work earlier calls on this handle
