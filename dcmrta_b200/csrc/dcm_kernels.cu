@@ -386,10 +386,18 @@ __device__ __forceinline__ double g_np_sum_le128(const double* v, int base, int 
     for (; i < n; ++i) res += v[base + i];
     return res;                                                               // valid in lane8 == 0
 }
-__device__ __forceinline__ double g_np_sum(const double* v, int n, unsigned lane8, unsigned gmask) {   // n <= 256
-    if (n <= 128) return g_np_sum_le128(v, 0, n, lane8, gmask);
-    int n2 = n / 2; n2 -= n2 % 8;
-    return g_np_sum_le128(v, 0, n2, lane8, gmask) + g_np_sum_le128(v, n2, n - n2, lane8, gmask);
+// n <= 256: numpy's recursion, blocks of np_blocks (dcm_thread.cuh) summed as b0 + (b1 + b2), one copy of the block sum
+__device__ __forceinline__ double g_np_sum(const double* v, int n, unsigned lane8, unsigned gmask) {
+    int n2, m2; np_blocks(n, n2, m2);
+    double head = 0.0, tail = 0.0;
+#pragma unroll 1
+    for (int s = 0; s < 3; ++s) {
+        const int b = s == 0 ? 0 : (s == 1 ? n2 : m2), e = s == 0 ? n2 : (s == 1 ? m2 : n);
+        if (b >= e) continue;
+        const double r = g_np_sum_le128(v, b, e - b, lane8, gmask);
+        if (s == 0) head = r; else if (s == 1) tail = r; else tail += r;
+    }
+    return n2 < n ? head + tail : head;
 }
 
 // out[8]: reward, success_rate, makespan, time_cost, waiting_time, travel_dist, efficiency, decisions.  Returns the final clock.

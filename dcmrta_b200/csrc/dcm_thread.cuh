@@ -668,10 +668,27 @@ template <class F> __device__ __forceinline__ double np_sum_le128(F val, int bas
     for (; i < n; ++i) res += val(base + i);
     return res;
 }
-template <class F> __device__ __forceinline__ double np_sum(F val, int n) {                   // n <= 256
-    if (n <= 128) return np_sum_le128(val, 0, n);
-    int n2 = n / 2; n2 -= n2 % 8;
-    return np_sum_le128(val, 0, n2) + np_sum_le128(val, n2, n - n2);
+// n <= 256: numpy splits a block longer than 128 at n/2 - (n/2) % 8 and recurses into each half.  The first half is at most 128
+// long; the second is longer than 128 for n = 249..256 and is split once more: blocks [0, n2), [n2, m2), [m2, n) summed as
+// b0 + (b1 + b2).  One loop over the blocks keeps one copy of the block sum in the kernel.
+__device__ __forceinline__ void np_blocks(int n, int& n2, int& m2) {
+    n2 = m2 = n;
+    if (n <= 128) return;
+    n2 = n / 2; n2 -= n2 % 8;
+    const int m = n - n2;
+    if (m > 128) { m2 = m / 2; m2 = n2 + m2 - m2 % 8; }
+}
+template <class F> __device__ __forceinline__ double np_sum(F val, int n) {
+    int n2, m2; np_blocks(n, n2, m2);
+    double head = 0.0, tail = 0.0;
+#pragma unroll 1
+    for (int s = 0; s < 3; ++s) {
+        const int b = s == 0 ? 0 : (s == 1 ? n2 : m2), e = s == 0 ? n2 : (s == 1 ? m2 : n);
+        if (b >= e) continue;
+        const double r = np_sum_le128(val, b, e - b);
+        if (s == 0) head = r; else if (s == 1) tail = r; else tail += r;
+    }
+    return n2 < n ? head + tail : head;
 }
 
 // Thread-per-env version (granular dcm_compute_metrics).  out[8] (plain global): reward, success_rate, makespan, time_cost,

@@ -64,6 +64,7 @@ def lib() -> C.CDLL:
             "orc_route": (None, [vp, i32, vp, vp]),
             "orc_agent_scalars": (None, [vp, vp, vp]),
             "orc_philox": (None, [vp, vp, vp]),
+            "orc_np_sum": (f64, [vp, i32]),
             "orc_seed": (None, [vp, u64, u64, u32]),
             "orc_fused_reset": (i32, [vp, i32]),
             "orc_policy_action": (i32, [vp, i32]),
@@ -265,6 +266,12 @@ def philox(ctr, key):
     o = np.zeros(4, np.uint32)
     lib().orc_philox(_p(c), _p(k), _p(o))
     return o
+
+
+def np_sum(a):
+    """the oracle's restatement of np.add.reduce on a float64 vector (pairwise summation)"""
+    a = np.ascontiguousarray(a, np.float64)
+    return lib().orc_np_sum(_p(a), len(a))
 
 
 def synthetic_instance(A, T, M, seed, max_duration=5.0, random_duration=False):

@@ -536,6 +536,7 @@ static void philox4x32_10(const uint32_t ctr[4], const uint32_t key[2], uint32_t
     out[0] = c0; out[1] = c1; out[2] = c2; out[3] = c3;
 }
 void orc_philox(const uint32_t *ctr, const uint32_t *key, uint32_t *out) { philox4x32_10(ctr, key, out); }
+double orc_np_sum(const double *a, int n) { return np_sum(a, n); }
 
 /* Random stream contract shared with the CUDA path (DESIGN.md "RNG contract"):
  *   key  = (seed_lo, seed_hi)

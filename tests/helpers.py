@@ -78,3 +78,149 @@ def quirk_instance(tr: Traces, name: str):
 
 def quirk_census(tr: Traces, name: str):
     return dict(zip(tr.census_keys, (int(x) for x in tr.z[f"census/{name}"])))
+
+
+# ---- the supported shape range (include/dcmrta.h: 1 <= A <= 64, 1 <= T <= 254, 1 <= M <= 8) -------------------------------------
+# Shapes at which the CUDA path changes code path, shared by tests/test_gpu_shape_envelope.py (CUDA against the oracle) and
+# tests/test_shape_envelope_oracle.py (the same trajectories on the oracle alone, so the census below cannot become vacuous).
+class EnvelopeShape:
+    """A, T, M, batch size B, the in-kernel policy, the decisions a test plays (`steps`; `ia_steps` for the individual-agent
+    protocol, None where it is not run) and the census events (envelope_census) its sampled trajectories must reach."""
+
+    def __init__(self, A, T, M, B, policy, steps, ia_steps, reaches, census):
+        self.A, self.T, self.M, self.B, self.policy, self.steps, self.ia_steps = A, T, M, B, policy, steps, ia_steps
+        self.reaches, self.census = reaches, tuple(census)
+        self.seed = 100 + A + 7 * T + 11 * M
+
+    @property
+    def name(self):
+        return f"{self.A}A_{self.T}T_{self.M}M_B{self.B}_{self.policy}"
+
+    @property
+    def random_duration(self):
+        return self.policy == "greedy"
+
+    def sample(self):
+        """env 0, the last env, and the first and last env of the last (partial) tile of 32 envs"""
+        return sorted({0, min(31, self.B - 1), 32 * ((self.B - 1) // 32), self.B - 1})
+
+    def first_gid(self):
+        return 1000 * self.A + self.T
+
+
+ENVELOPE_SHAPES = [
+    EnvelopeShape(1, 1, 1, 33, "random", 40, None, "the smallest instance; a second tile holding one env", ["leader_last", "task_last", "full_coalition"]),
+    EnvelopeShape(2, 3, 3, 100, "random", 60, None, "requirements above A: episodes end by the clock cap or stuck",
+                  ["leader_last", "task_last", "give_up", "clock_cap_or_stuck"]),
+    EnvelopeShape(7, 63, 2, 100, "greedy", 240, 300, "A < 8; ragged agent chunk; T just below a word", ["leader_last", "task_last", "full_coalition"]),
+    EnvelopeShape(24, 64, 8, 100, "random", 280, None, "last shape with the next_decision scratch; word 0 full; 8-member coalitions",
+                  ["leader_last", "task_last", "task_63", "full_coalition"]),
+    EnvelopeShape(25, 65, 8, 100, "greedy", 420, None, "first shape without the scratch; TW = 2 with one bit in word 1",
+                  ["leader_last", "task_last", "task_64", "full_coalition"]),
+    EnvelopeShape(32, 128, 4, 100, "random", 500, None, "ANB = 32; TW = 2 full", ["leader_last", "task_last", "task_63", "task_64", "task_127", "full_coalition"]),
+    EnvelopeShape(33, 129, 5, 100, "greedy", 600, 1100, "ANB = 64; TW = 4",
+                  ["leader_last", "task_last", "task_63", "task_64", "task_127", "task_128", "full_coalition", "depot16"]),
+    EnvelopeShape(20, 55, 5, 100, "random", 270, None, "largest T of the k_obs_tile path at A = 20 (228 kB of shared memory per SM)", ["leader_last", "task_last"]),
+    EnvelopeShape(20, 56, 5, 100, "random", 270, None, "smallest T of the chunked k_obs path at A = 20 (228 kB of shared memory per SM)", ["leader_last", "task_last"]),
+    EnvelopeShape(64, 249, 3, 100, "greedy", 450, None, "agent bit 63; the first T whose metric sums split twice",
+                  ["leader_last", "task_last", "task_63", "task_64", "task_127", "task_128", "full_coalition", "depot16"]),
+    EnvelopeShape(64, 254, 8, 100, "random", 800, 650, "the largest shape",
+                  ["leader_last", "task_last", "task_63", "task_64", "task_127", "task_128", "full_coalition", "wait16", "clock_cap"]),
+    EnvelopeShape(64, 254, 8, 1, "greedy", 600, None, "the largest shape in a batch of one", ["leader_last", "task_last", "full_coalition"]),
+]
+
+
+def envelope_shape(name):
+    return next(s for s in ENVELOPE_SHAPES if s.name == name)
+
+
+def device_instance(A, T, M, seed, gid, instance=0, max_duration=5.0, random_duration=False):
+    """The instance dcm_generate draws for global env `gid` (dcm_kernels.cu t_generate): Philox counter (gid_lo, gid_hi, instance,
+    0x80000000 + 2 j + {0, 1}) for task j and 0xFFFFFFFF for the depot, key = seed, uniforms of 53 bits."""
+    from oracle.oracle import philox
+    key = [seed & 0xFFFFFFFF, seed >> 32]
+    g = [gid & 0xFFFFFFFF, gid >> 32, instance]
+    u01 = lambda hi, lo: float(((int(hi) >> 5) << 26) | (int(lo) >> 6)) * (1.0 / 9007199254740992.0)
+    xy, req, dur = np.empty((T, 2)), np.empty(T, np.int32), np.full(T, float(max_duration))
+    for j in range(T):
+        a, b = philox(g + [0x80000000 + 2 * j], key), philox(g + [0x80000001 + 2 * j], key)
+        xy[j] = u01(a[0], a[1]), u01(a[2], a[3])
+        req[j] = 1 + ((int(b[0]) * M) >> 32)
+        if random_duration:
+            dur[j] = u01(b[1], b[2]) * max_duration
+    a = philox(g + [0xFFFFFFFF], key)
+    return dict(A=A, task_xy=xy, depot_xy=np.array([u01(a[0], a[1]), u01(a[2], a[3])]), req=req, dur=dur)
+
+
+def envelope_census(ev, o, A, T, M, leader, used_action, done=False, env=None):
+    """Add to the set `ev` what one decision of the oracle reached.  `o` is the OracleEnv after the decision, `leader` the agent that
+    decided and `used_action` its action (0 = depot, j + 1 = task j); `env` the OracleEnv whose episode ended (`done`), for its cause."""
+    if leader == A - 1:
+        ev.add("leader_last")
+    for j, key in ((T - 1, "task_last"), (63, "task_63"), (64, "task_64"), (127, "task_127"), (128, "task_128")):
+        if j < T and used_action == j + 1:
+            ev.add(key)
+    s = o.export(M)
+    if (s["n_mem"] == M).any():
+        ev.add("full_coalition")
+    waiting = (s["n_mem"] > 0) & (s["feasible"] == 0)
+    if any(waiting[w:w + 64].sum() > 16 for w in range(0, T, 64)):
+        ev.add("wait16")                                              # a second SCR_TMP chunk of the waiting-coalition scan
+    if ((s["has_route"] > 0) & (s["node"] < 0) & (s["returned"] == 0)).sum() > 16 and (s["feasible"] > 0).all():
+        ev.add("depot16")                                             # ... and of the depot-return scan, which runs once all tasks are feasible
+    if s["n_aband_task"].any():
+        ev.add("give_up")
+    if done:
+        e = env if env is not None else o
+        if e.stuck:
+            ev.add("stuck")
+            ev.add("clock_cap_or_stuck")
+        elif not e.export(M)["env_finished"]:
+            ev.add("clock_cap")
+            ev.add("clock_cap_or_stuck")
+    return ev
+
+
+class EnvelopeOracle:
+    """One sampled env of an envelope shape on the CPU reference, restarted as an auto-reset handle restarts it: the oracle's
+    leader-follower driver (protocol "LF") or the individual-agent loop of tests/ia_oracle.py ("IA"), with the Philox draws of
+    (shape.seed, gid, episode)."""
+
+    def __init__(self, shape, b, inst, protocol="LF"):
+        from oracle.oracle import OracleEnv
+        self.shape, self.gid, self.protocol = shape, shape.first_gid() + b, protocol
+        if protocol == "IA":
+            from ia_oracle import IAOracle
+            self.o = IAOracle(shape.A, inst["task_xy"], inst["depot_xy"], inst["req"], inst["dur"])
+            self.env = self.o.env
+        else:
+            self.o = self.env = OracleEnv.make(shape.A, inst["task_xy"], inst["depot_xy"], inst["req"], inst["dur"])
+        self.episodes, self.last_metrics, self.first_end, self.census = 0, None, None, set()
+        self._restart()
+
+    def _restart(self):
+        self.o.seed(self.shape.seed, gid=self.gid, episode=self.episodes)
+        self.o.reset() if self.protocol == "IA" else self.o.fused_reset()
+
+    @property
+    def leader(self):
+        return self.o.leader
+
+    def step(self):
+        """one decision of the shape's built-in policy -> (reward, done, used_action); restarts a finished episode"""
+        code = -1 if self.shape.policy == "random" else -2
+        leader = self.o.leader
+        if self.protocol == "IA":
+            r, d, ua, _ = self.o.step(code)
+        else:
+            rc, r, d, ua, _ = self.o.fused_step(code)
+            assert rc == 0, (self.shape.name, self.gid, rc)
+        s = self.shape
+        envelope_census(self.census, self.env, s.A, s.T, s.M, leader, ua, d, self.o)
+        if d:
+            if self.first_end is None:
+                self.first_end = (bool(self.o.export(s.M)["env_finished"]), bool(self.o.stuck))
+            self.last_metrics = np.array([self.o.episode_metrics()[0][k] for k in METRIC_KEYS])
+            self.episodes += 1
+            self._restart()
+        return r, d, ua
