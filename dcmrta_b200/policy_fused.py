@@ -17,7 +17,8 @@ Re-layout of the parameters (done in `refresh`, into buffers whose addresses nev
   * compressed_task = mean_t(task_embedding) (attention.py:268-270) = task_embedding(mean_t(tasks)), the layer being affine.
 
 `forward_torch` is the same dataflow in plain torch ops on the same re-laid-out weights: the CPU tests pin it to `AttentionNet`
-(fp32, 1e-5), the GPU tests pin the CUDA path to it.  The CUDA path has no fallback: without libdcmrta_policy.so it raises.
+(fp32, 1e-5; float64, 1e-12), the GPU tests pin the CUDA path to it and each kernel to its float64 form.  The CUDA path has no
+fallback: without libdcmrta_policy.so it raises.
 """
 from __future__ import annotations
 
@@ -82,6 +83,8 @@ class CudaOps:
     """Each method launches one kernel of libdcmrta_policy.so on the current stream.  Column slices of a wider row-major matrix are
     passed as views (data_ptr() carries the offset, stride(0) the row stride)."""
 
+    acc = torch.float32                                                      # the dtype of the log-probabilities dcmp_pointer writes
+
     @staticmethod
     def _rows(t):
         assert t.dim() == 2 and t.stride(1) == 1 and t.is_cuda
@@ -135,16 +138,17 @@ class CudaOps:
 
 class TorchOps:
     """The same six ops in torch (any device / dtype, any embedding size): what each kernel must compute.  Test infrastructure and
-    documentation, never called by the product path."""
+    documentation, never called by the product path.  Every op computes in `acc` (fp32 as the kernels do, or float64 for a reference
+    that rounds nothing the tests can see)."""
 
-    def __init__(self, e=E, h=H, hid=HID):
-        self.E, self.H, self.D, self.HID = e, h, e // h, hid
+    def __init__(self, e=E, h=H, hid=HID, acc=torch.float32):
+        self.E, self.H, self.D, self.HID, self.acc = e, h, e // h, hid, acc
 
     def embed(self, x, w, b, out):
-        return out.copy_(F.linear(x.to(w.dtype), w, b))
+        return out.copy_(F.linear(x.to(self.acc), w.to(self.acc), b.to(self.acc)))
 
     def _heads(self, t, B, n):
-        return t.reshape(B, n, self.H, self.D).transpose(1, 2).float()       # [B,H,n,D]
+        return t.reshape(B, n, self.H, self.D).transpose(1, 2).to(self.acc)  # [B,H,n,D]
 
     def attention(self, q, k, v, out, B, nq, nk):
         s = self._heads(q, B, nq) @ self._heads(k, B, nk).transpose(2, 3) / math.sqrt(self.D)
@@ -161,13 +165,14 @@ class TorchOps:
         return out.copy_((p @ self._heads(v, B, nk)).transpose(1, 2).reshape(B, self.E))
 
     def add_layernorm(self, x, res, gamma, beta, out, eps):
-        return out.copy_(F.layer_norm(x.float() + res.float(), (self.E,), gamma, beta, eps))
+        a = self.acc
+        return out.copy_(F.layer_norm(x.to(a) + res.to(a), (self.E,), gamma.to(a), beta.to(a), eps))
 
     def gate(self, wv, out):
-        return out.copy_(torch.sigmoid(wv[:, :self.HID].float()) * wv[:, self.HID:].float())
+        return out.copy_(torch.sigmoid(wv[:, :self.HID].to(self.acc)) * wv[:, self.HID:].to(self.acc))
 
     def pointer(self, qk, feat, mask, out, B, n, norm, clip):
-        u = clip * torch.tanh(norm * torch.einsum("be,bne->bn", qk.float(), feat.float().view(B, n, self.E)))
+        u = clip * torch.tanh(norm * torch.einsum("be,bne->bn", qk.to(self.acc), feat.to(self.acc).view(B, n, self.E)))
         if mask is not None:
             u = u.masked_fill(mask.bool(), -1e4)
         return out.copy_(torch.log_softmax(u, -1))
@@ -194,8 +199,9 @@ def _layer_names(net):
 
 def pack_parameters(net, dtype=torch.bfloat16, into: dict | None = None) -> dict:
     """The re-laid-out copy of `net`'s parameters (see the module docstring).  GEMM operands in `dtype`; embedding, LayerNorm and
-    nothing else in fp32.  into: refresh these tensors in place instead of allocating."""
+    nothing else in fp32 (float64 when `dtype` is).  into: refresh these tensors in place instead of allocating."""
     P = {}
+    f32 = torch.promote_types(dtype, torch.float32)
 
     def put(name, t, dt=dtype):
         t = t.detach().to(dt).contiguous()
@@ -206,8 +212,8 @@ def pack_parameters(net, dtype=torch.bfloat16, into: dict | None = None) -> dict
             P[name] = t.clone()
 
     with torch.no_grad():
-        put("task_embedding.w", net.task_embedding.weight, torch.float32); put("task_embedding.b", net.task_embedding.bias, torch.float32)
-        put("agent_embedding.w", net.agent_embedding.weight, torch.float32); put("agent_embedding.b", net.agent_embedding.bias, torch.float32)
+        put("task_embedding.w", net.task_embedding.weight, f32); put("task_embedding.b", net.task_embedding.bias, f32)
+        put("agent_embedding.w", net.agent_embedding.weight, f32); put("agent_embedding.b", net.agent_embedding.bias, f32)
         for name, layer, self_attn in _layer_names(net):
             mha = layer.multiHeadAttention
             wq, wk, wv = _flat_heads(mha.w_query), _flat_heads(mha.w_key), _flat_heads(mha.w_value)
@@ -221,9 +227,9 @@ def pack_parameters(net, dtype=torch.bfloat16, into: dict | None = None) -> dict
             ffn, ln2 = layer.feedForward.DenseReluDense, layer.feedForward.layer_norm.normalizer
             put(name + ".wv", torch.cat([ffn.W.weight.t(), ffn.V.weight.t()], 1)); put(name + ".w2", ffn.W2.weight.t())
             for tag, ln in (("ln1", ln1), ("ln2", ln2)):
-                put(f"{name}.{tag}.g", ln.weight, torch.float32); put(f"{name}.{tag}.b", ln.bias, torch.float32)
+                put(f"{name}.{tag}.g", ln.weight, f32); put(f"{name}.{tag}.b", ln.bias, f32)
                 P[f"{name}.{tag}.eps"] = ln.eps
-        put("pointer.m", net.pointer.w_query.detach().float() @ net.pointer.w_key.detach().float().t())
+        put("pointer.m", net.pointer.w_query.detach().to(f32) @ net.pointer.w_key.detach().to(f32).t())
         P["pointer.norm"], P["pointer.clip"] = net.pointer.norm_factor, float(net.pointer.tanh_clipping)
         P["E"], P["HID"] = mha.embedding_dim, ffn.W.out_features
     return P
@@ -279,7 +285,7 @@ def _forward(ops, P, W, tasks, agents, mask_u8, names):
         if name.startswith("globalDecoder2"):
             cs = decoder(name, cs, 1, taf, nt, mask_u8)
     qk = ops.mm(cs, P["pointer.m"], W("qk", B, E))
-    return ops.pointer(qk, taf, mask_u8, W("logp", B, nt, torch.float32), B, nt, P["pointer.norm"], P["pointer.clip"])
+    return ops.pointer(qk, taf, mask_u8, W("logp", B, nt, ops.acc), B, nt, P["pointer.norm"], P["pointer.clip"])
 
 
 class FusedPolicy:
@@ -332,12 +338,14 @@ class FusedPolicy:
 
 @torch.no_grad()
 def forward_torch(net, tasks, agents, mask, dtype=torch.float32):
-    """The fused dataflow in torch ops on the re-laid-out parameters (activations and GEMM operands in `dtype`)."""
+    """The fused dataflow in torch ops on the re-laid-out parameters (activations and GEMM operands in `dtype`; every op computes in
+    fp32, or in float64 when `dtype` is float64: then, on `net.double()`, this is a float64 reference of the whole forward)."""
     P = pack_parameters(net, dtype)
+    acc = torch.promote_types(dtype, torch.float32)
     names = [(n, s) for n, _, s in _layer_names(net)]
 
     def W(name, rows, cols, dt=None):
         return torch.empty(rows, cols, dtype=dt or dtype, device=tasks.device)
     mask_u8 = mask.view(torch.uint8) if mask.dtype == torch.bool else mask
     mha = net.taskEncoder.layers[0].multiHeadAttention
-    return _forward(TorchOps(P["E"], mha.n_heads, P["HID"]), P, W, tasks.float(), agents.float(), mask_u8, names).clone()
+    return _forward(TorchOps(P["E"], mha.n_heads, P["HID"], acc), P, W, tasks.to(acc), agents.to(acc), mask_u8, names).clone()

@@ -4,7 +4,8 @@ CPU: the re-laid-out dataflow (`forward_torch`) against `AttentionNet` and again
 reference attention.py (tests/golden/policy_golden.npz); libdcmrta_policy.so builds for sm_100a only and exports exactly what
 include/dcmrta_policy.h declares; no CPU fallback.
 GPU (-m gpu): every kernel against its torch specification (`TorchOps`) on the same bf16 inputs, the whole fused forward against the
-fp32 module, and the rollout loops calling it."""
+fp32 module, and the rollout loops calling it.  Each kernel against a float64 reference with derived bounds, exact cases and guard
+memory: tests/test_gpu_policy_kernels.py."""
 import ctypes as C
 import math
 import re
@@ -48,6 +49,23 @@ def test_relayout_matches_the_module(A, T):
         ref = net(tasks, agents, mask)
     out = forward_torch(net, tasks, agents, mask)
     assert out.shape == ref.shape and torch.allclose(out, ref, atol=2e-5, rtol=0), float((out - ref).abs().max())
+
+
+@pytest.mark.parametrize("A,T", [(20, 50), (3, 4)])
+def test_float64_relayout_matches_the_float64_module(A, T):
+    """forward_torch in float64 is a float64 reference (every op computes in float64, the log-probabilities too): the reference the
+    GPU kernel tests (test_gpu_policy_kernels.py) compare with.  The re-layout reorders sums (heads, the folded pointer matrix, the
+    embedding of the mean task), so it agrees with the module to float64 rounding, far below anything fp32 could reach."""
+    from dcmrta_b200.policy_fused import forward_torch
+    net = _net().double()
+    tasks, agents, mask = _obs(9, A, T)
+    mask[4] = True
+    tasks, agents = tasks.double(), agents.double()
+    with torch.no_grad():
+        ref = net(tasks, agents, mask)
+    out = forward_torch(net, tasks, agents, mask, torch.float64)
+    assert out.dtype == torch.float64 and out.shape == ref.shape
+    assert float((out - ref).abs().max()) < 1e-12
 
 
 def test_relayout_matches_the_reference_recording():
