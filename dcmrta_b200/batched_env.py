@@ -122,6 +122,7 @@ class BatchedTaskEnv:
 
     def seed(self, seed, first_gid=0):
         check(lib().dcm_seed(self._h, int(seed), int(first_gid)))
+        self.first_gid = int(first_gid)                  # global id of env 0, which the policy's action sampler keys its draws by too
 
     def load_instances(self, task_xy, depot_xy, req, dur):
         """reset(test_env=...) of the reference (task_env.py:116-127) for the whole batch.  Arrays [B,T,2], [B,2], [B,T], [B,T]."""

@@ -11,7 +11,7 @@ PKG = Path(__file__).resolve().parent
 CSRC = PKG / "csrc"
 SO = Path(os.environ["DCM_LIB"]).resolve() if os.environ.get("DCM_LIB") else PKG / "libdcmrta_b200.so"
 SOURCES = [CSRC / "dcm_kernels.cu"]
-HEADERS = [CSRC / "dcm_thread.cuh", CSRC / "dcm_soa.h", CSRC / "dcm_layout.h", PKG.parent / "include" / "dcmrta.h"]
+HEADERS = [CSRC / "dcm_thread.cuh", CSRC / "dcm_philox.cuh", CSRC / "dcm_soa.h", CSRC / "dcm_layout.h", PKG.parent / "include" / "dcmrta.h"]
 
 NVCC_FLAGS = [
     "-std=c++17", "-O3",
@@ -23,7 +23,7 @@ NVCC_FLAGS = [
 # the policy kernels: bf16 activations, fp32 arithmetic with contraction allowed (nothing there has to round like NumPy)
 POLICY_SO = PKG / "libdcmrta_policy.so"
 POLICY_SOURCES = [CSRC / "policy_kernels.cu"]
-POLICY_HEADERS = [PKG.parent / "include" / "dcmrta_policy.h"]
+POLICY_HEADERS = [CSRC / "dcm_philox.cuh", PKG.parent / "include" / "dcmrta_policy.h", PKG.parent / "include" / "dcmrta_sample.h"]
 POLICY_FLAGS = ["-std=c++17", "-O3", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-Xcompiler", "-fPIC", "-shared"]
 
 

@@ -15,6 +15,7 @@
 #include <math_constants.h>
 #include <stdint.h>
 
+#include "dcm_philox.cuh"
 #include "dcm_soa.h"
 
 namespace dcm {
@@ -170,18 +171,7 @@ template <int TW> __device__ __forceinline__ void st_state(const TC& c, const St
     if (o.xlast != st.xlast) EL(c, x_last, 1, 0) = st.xlast;
 }
 
-// Philox4x32-10 (Salmon et al. 2011)
-__device__ __forceinline__ uint4 philox(unsigned c0, unsigned c1, unsigned c2, unsigned c3, unsigned k0, unsigned k1) {
-#pragma unroll
-    for (int r = 0; r < 10; ++r) {
-        unsigned h0 = __umulhi(0xD2511F53u, c0), l0 = 0xD2511F53u * c0;
-        unsigned h1 = __umulhi(0xCD9E8D57u, c2), l1 = 0xCD9E8D57u * c2;
-        unsigned n0 = h1 ^ c1 ^ k0, n2 = h0 ^ c3 ^ k1;
-        c0 = n0; c1 = l1; c2 = n2; c3 = l0;
-        k0 += 0x9E3779B9u; k1 += 0xBB67AE85u;
-    }
-    return make_uint4(c0, c1, c2, c3);
-}
+// philox(): Philox4x32-10, dcm_philox.cuh
 struct Rng { u64 seed; u64 gid; };
 // decision stream: ctr = (gid_lo, gid_hi, episode, decision*8 + block), block < 8
 // block 0: [0] action  [1] leader of this decision  [2],[3] followers 0,1 ; block 1: followers 2..5 ; ...

@@ -11,6 +11,8 @@
 #include <stdio.h>
 
 #include "../../include/dcmrta_policy.h"
+#include "../../include/dcmrta_sample.h"
+#include "dcm_philox.cuh"
 
 namespace {
 
@@ -378,6 +380,62 @@ __global__ void __launch_bounds__(256) k_pointer(const uint2* __restrict__ qk, c
     for (int r = 0; r < R; ++r) if (r * 32 + lane < n) logp[(size_t)b * n + r * 32 + lane] = (u[r] - m) - logl;   // in this order: -1e4 entries keep their low bits
 }
 
+// ---- action sampler: warp per row, the draw a function of (seed, gid, stream, decision) alone (DESIGN.md 5, include/dcmrta_sample.h) -------
+// Pass 1 keeps the row in registers (lane <-> columns 32 r + lane), pass 2 turns it into weights and an inclusive prefix sum (a shuffle
+// scan per 32-column chunk, carried from chunk to chunk), pass 3 finds the first crossing of the threshold by ballot.
+constexpr int SMP_MAX_N = 256;
+
+__global__ void __launch_bounds__(256) k_sample(const float* __restrict__ x, int ldx, const uint8_t* __restrict__ mask,
+                                                const int64_t* __restrict__ rows, long long first_gid, const uint32_t* __restrict__ draw,
+                                                int32_t* __restrict__ action, int B, int n) {
+    const int lane = threadIdx.x & 31;
+    const int b = blockIdx.x * 8 + (threadIdx.x >> 5);
+    if (b >= B) return;
+    const unsigned long long gid = (unsigned long long)(first_gid + (rows ? rows[b] : (long long)b));
+    const uint4 r4 = dcm::philox((unsigned)gid, (unsigned)(gid >> 32), draw[2], 0xC0000000u + draw[3], draw[0], draw[1]);
+    constexpr int R = SMP_MAX_N / 32;
+    float v[R];
+    float m = -INFINITY;
+#pragma unroll
+    for (int r = 0; r < R; ++r) {
+        const int j = r * 32 + lane;
+        v[r] = -INFINITY;                                                    // no such column, or forbidden: weight 0
+        if (j < n && !(mask && mask[(size_t)b * n + j])) v[r] = x[(size_t)b * ldx + j];
+        m = fmaxf(m, v[r]);
+    }
+    m = wmaxf(m);
+    float c[R];
+    float carry = 0.f, S = 0.f;
+#pragma unroll
+    for (int r = 0; r < R; ++r) {
+        c[r] = 0.f;
+        if (r * 32 < n) {                                                    // warp-uniform
+            const float w = v[r] > -INFINITY ? expf(v[r] - m) : 0.f;         // (m is finite whenever some v is)
+            v[r] = w;
+            float s = w;
+#pragma unroll
+            for (int o = 1; o < 32; o <<= 1) {
+                const float t = __shfl_up_sync(0xffffffffu, s, o);
+                if (lane >= o) s += t;
+            }
+            c[r] = carry + s;
+            carry = __shfl_sync(0xffffffffu, c[r], 31);
+            const unsigned pos = __ballot_sync(0xffffffffu, w > 0.f);
+            if (pos) S = __shfl_sync(0xffffffffu, c[r], 31 - __clz(pos));    // C at the last entry of positive weight so far
+        }
+    }
+    int a = 0;                                                               // nothing of positive weight: 0 (the step ignores it)
+    if (S > 0.f) {
+        const double theta = (double)(r4.x >> 8) * (double)S * 0x1p-24;      // exact: 24 x 24 significant bits
+#pragma unroll
+        for (int r = 0; r < R; ++r) {
+            const unsigned hit = __ballot_sync(0xffffffffu, r * 32 + lane < n && v[r] > 0.f && (double)c[r] > theta);
+            if (hit) { a = r * 32 + __ffs(hit) - 1; break; }
+        }
+    }
+    if (lane == 0) action[b] = a;
+}
+
 int row_grid(long rows) {                                                     // 8 rows (warps) per block, at most 8 resident blocks per SM
     const long want = (rows + 7) / 8, cap = (long)sm_count() * 8;
     return (int)(want < cap ? want : cap);
@@ -473,6 +531,17 @@ int dcmp_pointer(const uint16_t* qk, const uint16_t* feat, const uint8_t* mask, 
     k_pointer<<<(B + 7) / 8, 256, 0, static_cast<cudaStream_t>(stream)>>>(reinterpret_cast<const uint2*>(qk), reinterpret_cast<const uint2*>(feat),
                                                                          mask, logp, B, n, norm, clip);
     return launched("k_pointer");
+}
+
+int dcmp_sample(const float* x, int ldx, const uint8_t* mask, const int64_t* rows, long long first_gid, const uint32_t* draw, int32_t* action,
+                int B, int n, void* stream) {
+    if (!x || !draw || !action) return fail(-1, "dcmp_sample: null pointer");
+    if (first_gid < 0) return fail(-1, "dcmp_sample: first_gid must be >= 0");
+    if (B < 0 || n < 1 || n > SMP_MAX_N || ldx < n) return fail(-2, "dcmp_sample: need B >= 0, 1 <= n <= 256, ldx >= n");
+    if (B == 0) return 0;
+    if (!sm_count()) return fail(-3, "dcmp_sample: no CUDA device (there is no CPU fallback)");
+    k_sample<<<(B + 7) / 8, 256, 0, static_cast<cudaStream_t>(stream)>>>(x, ldx, mask, rows, first_gid, draw, action, B, n);
+    return launched("k_sample");
 }
 
 const char* dcmp_last_error(void) { return g_err; }

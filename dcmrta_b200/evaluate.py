@@ -12,6 +12,11 @@ follower draws come from the Philox contract (DESIGN.md 5) keyed by `seed`, inst
         --method IA --out REINFORCE_IA.csv
 
 The default forward is the fp32 module, as in the reference; --amp fused (policy_fused.FusedPolicy) or --amp bf16 are opt-in.
+
+--samples K (which the reference does not have) plays K sampled episodes per instance instead, all N K of them on the device, and reports
+the best of the K per instance: the usual second number after greedy decoding for a learned routing / allocation policy.  Actions come from
+the Philox sampler (policy_fused.sample, DESIGN.md 5) keyed by --sample-seed and the global env id, so the result does not depend on how
+the N K envs are split into batches (--max-envs).
 """
 from __future__ import annotations
 
@@ -113,6 +118,54 @@ def evaluate(net, instances: dict, method: str = "LF", amp=False, seed: int = 0,
         env.close()
 
 
+def evaluate_sampled(net, instances: dict, samples: int, method: str = "LF", amp=False, seed: int = 0, sample_seed: int = 0,
+                     device: int = 0, graphed: bool = False, horizon: int | None = None, max_envs: int = 32768) -> np.ndarray:
+    """K = `samples` sampled episodes per instance.  Returns the [N,K,8] f64 metrics (columns as `evaluate`).
+
+    Env e = i K + k plays instance i, with global id e: LF leader and follower draws come from `seed` as in `evaluate` (so K = 1 keys
+    everything exactly as the greedy run does), action draws from `sample_seed`, stream 0.  The N K envs run in contiguous chunks of at most
+    `max_envs`, each with first_gid = its first env, so the table does not depend on the chunk size.  An episode the horizon would cut
+    raises, as in `evaluate`."""
+    import torch
+
+    from .batched_env import BatchedTaskEnv
+    from .rollout import BatchedRollout, GraphedRollout
+
+    if method not in ("LF", "IA"):
+        raise ValueError(f"method must be 'LF' or 'IA', not {method!r}")
+    K, max_envs = int(samples), int(max_envs)
+    if K < 1 or max_envs < 1:
+        raise ValueError("samples and max_envs must be >= 1")
+    N, T = instances["task_xy"].shape[:2]
+    A = int(instances["A"])
+    M = max(5, int(np.max(instances["req"])))
+    horizon = int(horizon or 8 * (A + T))
+    out = np.empty((N * K, 8), np.float64)
+    R = GraphedRollout if graphed else BatchedRollout
+    for e0 in range(0, N * K, max_envs):
+        n = min(max_envs, N * K - e0)
+        inst = np.arange(e0, e0 + n) // K
+        env = BatchedTaskEnv(n, A, T, M=M, device=device, auto_reset=False, max_wait=float(MAX_WAITING_TIME), max_time=MAX_TIME,
+                             seed=seed, first_gid=e0, protocol=method)
+        try:
+            env.load_instances(instances["task_xy"][inst], instances["depot_xy"][inst], instances["req"][inst], instances["dur"][inst])
+            ep = R(env, horizon, record=False, check_every=8).run(net, "sample", amp=amp, sampler=(sample_seed, 0))
+            if not bool(ep.ended.all()):
+                cut = (e0 + torch.logical_not(ep.ended).nonzero().flatten()).tolist()
+                raise RuntimeError(f"{len(cut)} episode(s) not over after {ep.length} decisions (envs {cut[:8]}): raise `horizon`")
+            out[e0:e0 + n] = ep.metrics.cpu().numpy()
+        finally:
+            env.close()
+    return out.reshape(N, K, 8)
+
+
+def best_of(metrics):
+    """[N,K,8] -> (best [N,8], k [N]): the sample of highest reward per instance, ties to the lowest k."""
+    m = np.asarray(metrics, np.float64)
+    k = np.argmax(m[:, :, 0], axis=1)                           # first maximum
+    return m[np.arange(m.shape[0]), k], k
+
+
 def metric_rows(metrics) -> list:
     """[N,8] metrics -> the per-instance perf_metrics dicts RL_test.py collects (worker.py:103-108)."""
     m = np.asarray(metrics, np.float64)
@@ -128,14 +181,19 @@ def summary(metrics) -> str:
 # ---- command line ----------------------------------------------------------------------------------------------------------
 def parse_args(argv=None):
     ap = argparse.ArgumentParser(prog="python -m dcmrta_b200.evaluate",
-                                 description="Play a checkpoint greedily on a test set, one batch (the reference's RL_test.py).")
+                                 description="Play a checkpoint greedily on a test set, one batch (the reference's RL_test.py), "
+                                             "or best of K sampled episodes per instance (--samples K).")
     ap.add_argument("--checkpoint", required=True, help="torch checkpoint with a 'model' state dict (reference or ReinforceTrainer.save)")
     ap.add_argument("--test-set", required=True, help="instances .npz, or a directory of reference env_<i>.pkl files")
     ap.add_argument("--method", choices=("LF", "IA"), default="LF", help="leader-follower (run_test) or individual agent (run_test_IS)")
     ap.add_argument("--amp", choices=("none", "bf16", "fused"), default="none", help="policy forward: fp32 module (default), bf16 copy, fused kernels")
     ap.add_argument("--seed", type=int, default=0, help="Philox key of the LF leader / follower draws")
     ap.add_argument("--device", type=int, default=0)
-    ap.add_argument("--out", required=True, help="per-instance metrics CSV (e.g. REINFORCE_IA.csv)")
+    ap.add_argument("--out", required=True, help="per-instance metrics CSV (e.g. REINFORCE_IA.csv); with --samples, each instance's best sample")
+    ap.add_argument("--samples", type=int, default=0, help="K sampled episodes per instance, best of K reported (default 0: one greedy episode)")
+    ap.add_argument("--sample-seed", type=int, default=0, help="Philox key of the action draws of --samples")
+    ap.add_argument("--max-envs", type=int, default=32768, help="envs per batch of --samples (the result does not depend on it)")
+    ap.add_argument("--samples-out", help="optional .npz for the whole [N, K, 8] table of --samples (key 'metrics', plus 'best_k')")
     return ap.parse_args(argv)
 
 
@@ -157,6 +215,17 @@ def main(argv=None) -> int:
     amp = {"none": False, "bf16": True, "fused": "fused"}[args.amp]
     net = load_net(args.checkpoint, args.device)
     inst = load_test_set(args.test_set)
+    if args.samples > 0:
+        table = evaluate_sampled(net, inst, args.samples, method=args.method, amp=amp, seed=args.seed, sample_seed=args.sample_seed,
+                                 device=args.device, max_envs=args.max_envs)
+        best, k = best_of(table)
+        write_metrics_csv(args.out, metric_rows(best))
+        if args.samples_out:
+            np.savez(args.samples_out, metrics=table, best_k=k)
+        print(f"{args.method}: {table.shape[0]} instances x {args.samples} samples, {int(table[:, :, 7].sum())} decisions -> {args.out}")
+        print(f"best of {args.samples}:\n{summary(best)}")
+        print(f"all samples:\n{summary(table.reshape(-1, 8))}")
+        return 0
     metrics = evaluate(net, inst, method=args.method, amp=amp, seed=args.seed, device=args.device)
     write_metrics_csv(args.out, metric_rows(metrics))
     print(f"{args.method}: {metrics.shape[0]} instances, {int(metrics[:, 7].sum())} decisions -> {args.out}")

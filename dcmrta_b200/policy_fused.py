@@ -45,6 +45,10 @@ SIGNATURES = {
     "dcmp_last_error": (C.c_char_p, []),
     "dcmp_version": (C.c_char_p, []),
 }
+# every symbol include/dcmrta_sample.h declares (the action sampler, in the same library)
+SAMPLE_SIGNATURES = {
+    "dcmp_sample": (i32, [vp, i32, vp, vp, C.c_longlong, vp, vp, i32, i32, vp]),
+}
 
 
 class PolicyKernelError(RuntimeError):
@@ -62,7 +66,7 @@ def lib() -> C.CDLL:
             if not so.exists():
                 raise PolicyKernelError(f"libdcmrta_policy.so is missing and cannot be built ({e}); there is no CPU fallback")
         L = C.CDLL(str(so))
-        for name, (res, args) in SIGNATURES.items():
+        for name, (res, args) in {**SIGNATURES, **SAMPLE_SIGNATURES}.items():
             fn = getattr(L, name)
             fn.restype, fn.argtypes = res, args
         _LIB = L
@@ -334,6 +338,38 @@ class FusedPolicy:
         mask_u8 = mask.view(torch.uint8) if mask.dtype == torch.bool else mask
         return _forward(self.ops, self.P, self._workspace(tasks.device), tasks.float().contiguous(), agents.float().contiguous(),
                         mask_u8.contiguous(), self.names)
+
+
+# ---- the action sampler --------------------------------------------------------------------------------------------------------------
+def draw_tensor(seed: int, stream: int = 0, decision: int = 0, device=None) -> torch.Tensor:
+    """The device-side draw words {seed_lo, seed_hi, stream, decision} that `sample` reads when its kernel runs (int32 storage of the u32
+    words).  A captured graph that samples from it serves any seed, stream and decision written into it between replays."""
+    if not (0 <= seed < 2 ** 64 and 0 <= stream < 2 ** 32 and 0 <= decision < 2 ** 30 - 1):
+        raise ValueError("need 0 <= seed < 2^64, 0 <= stream < 2^32, 0 <= decision < 2^30 - 1")
+    words = [seed & 0xFFFFFFFF, seed >> 32, stream, decision]
+    return torch.tensor([w - (1 << 32) if w >= 1 << 31 else w for w in words], dtype=torch.int32, device=device)
+
+
+def sample(logw: torch.Tensor, mask: torch.Tensor | None, draw: torch.Tensor, rows: torch.Tensor | None = None, first_gid: int = 0,
+           out: torch.Tensor | None = None) -> torch.Tensor:
+    """Categorical(softmax(logw)).sample() per row by dcmp_sample (include/dcmrta_sample.h, the contract of DESIGN.md 5): one int32 action
+    per row, on the current stream.  logw [B, n] fp32 log-weights (row stride free, columns contiguous; what any of the three forwards
+    returns, the bf16 module's after .float()), mask [B, n] bool / u8 (True = forbidden) or None, draw: `draw_tensor`, rows [B] int64 env
+    index of each row (None: row r is env r), the env's global id being first_gid + env index."""
+    assert logw.dim() == 2 and logw.dtype == torch.float32 and logw.stride(1) == 1 and logw.is_cuda
+    B, n = logw.shape
+    if mask is not None:
+        mask = mask.view(torch.uint8) if mask.dtype == torch.bool else mask
+        assert mask.dtype == torch.uint8 and mask.is_contiguous() and mask.shape == (B, n)
+    assert draw.dtype == torch.int32 and draw.numel() == 4 and draw.is_contiguous() and draw.device == logw.device
+    if rows is not None:
+        assert rows.dtype == torch.int64 and rows.is_contiguous() and rows.shape == (B,) and rows.device == logw.device
+    if out is None:
+        out = torch.empty(B, dtype=torch.int32, device=logw.device)
+    _check(lib().dcmp_sample(logw.data_ptr(), logw.stride(0) if B > 1 else n, None if mask is None else mask.data_ptr(),
+                             None if rows is None else rows.data_ptr(), int(first_gid), draw.data_ptr(), out.data_ptr(), B, n,
+                             _stream(logw)))
+    return out
 
 
 @torch.no_grad()

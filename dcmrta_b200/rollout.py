@@ -88,8 +88,11 @@ class BatchedRollout:
 
     @torch.no_grad()
     def run(self, net, mode: str = "sample", generator: torch.Generator | None = None, amp: bool | str = False, replay: dict | None = None,
-            keep_logp: bool = False) -> Episodes:
+            keep_logp: bool = False, sampler: tuple | None = None) -> Episodes:
         """Play one episode per env with `net` (sampling: worker.py:70; greedy: worker.py:222).  The env must not auto-reset.
+
+        sampler=(seed, stream): sample with the Philox kernel (policy_fused.sample, DESIGN.md 5) instead of torch.multinomial on `generator`:
+        the action of env b at decision t is a function of (seed, global env id, stream, t) and of its own log-probabilities alone.
 
         replay (tests: pins this loop to a recorded reference episode): the draws the reference made OUTSIDE the env, injected instead of
         drawn here -- "leader" [L+1,B] int32 (np.random.choice(group), worker.py:54; -1 where the env is done), "followers" [L,B,F] int32
@@ -103,6 +106,11 @@ class BatchedRollout:
         env.set_output_buffers(self.agent_obs[s], self.task_obs[s], self.mask[s])
         env.reset(leaders=replay["leader"][0] if replay else None)
         horizon = min(self.horizon, replay["followers"].shape[0]) if replay else self.horizon
+        draw = None
+        if sampler is not None:
+            assert mode == "sample" and generator is None, "sampler= replaces the torch generator of a sampled rollout"
+            from .policy_fused import draw_tensor, sample
+            draw = draw_tensor(int(sampler[0]), int(sampler[1]), 0, env.device)
         logps = [] if keep_logp else None
         t = 0
         while t < horizon:
@@ -112,6 +120,9 @@ class BatchedRollout:
                 logps.append(logp.float().clone())
             if replay is not None and "action" in replay:
                 act = torch.where(env.done, torch.zeros_like(replay["action"][t]), replay["action"][t]).to(torch.int32)
+            elif draw is not None:
+                draw[3].fill_(t)                                     # the decision word: Episodes.action[t]
+                act = sample(logp.float(), self.mask[s], draw, first_gid=env.first_gid)
             else:
                 act = sample_actions(logp.float(), generator) if mode == "sample" else greedy_actions(logp)
             if self.record:
@@ -167,7 +178,9 @@ class GraphedRollout(BatchedRollout):
     The env writes each observation into one of two fixed ping-pong slots (graph nodes have fixed addresses); a captured index_copy_
     files it into the episode buffer at a decision counter that lives on the device.  `unroll` is even: the env alternates two
     ended-episode counters from pass to pass, and a replay must leave that parity where the capture found it.  Sampling uses the default
-    CUDA generator (graph-safe Philox offsets); seed it with torch.cuda.manual_seed.
+    CUDA generator (graph-safe Philox offsets; seed it with torch.cuda.manual_seed) or, with run(sampler=(seed, stream)), the Philox kernel
+    of policy_fused.sample, which reads its draw words from a device tensor: they are set at the start of a run and the decision word is
+    bumped inside the graph, and a compacted forward passes its index list, so every env draws what the eager loop would draw for it.
 
     `fractions`: forward only the envs that are still playing.  Episodes of one batch end at different decisions (20A/50T: 120 +- 9, the
     longest of 8,192 near 150), so late in a rollout most rows of a full-batch forward belong to finished envs.  For every fraction f < 1
@@ -187,18 +200,28 @@ class GraphedRollout(BatchedRollout):
         self.t_dev = torch.zeros(1, dtype=torch.int64, device=dev)
         self.sizes = sub_batch_sizes(B, fractions)                                                           # rows per forward, ascending
         self.live = {n: torch.zeros(n, dtype=torch.int64, device=dev) for n in self.sizes if n < B}            # the index lists
+        self.draw = torch.zeros(4, dtype=torch.int32, device=dev)                                             # run(sampler=...): the draw words
         self._graphs = {}
 
-    def _decision(self, net, mode, amp, s, rows=None):
+    def _act(self, logp, mask, mode, philox, idx=None):
+        if mode != "sample":
+            return greedy_actions(logp)
+        if philox:
+            from .policy_fused import sample
+            return sample(logp.float(), mask, self.draw, idx, self.env.first_gid)
+        return sample_actions(logp.float())
+
+    def _decision(self, net, mode, amp, s, rows=None, philox=False):
         env = self.env
         a, k, m = self.pp[s]
         if rows is None or rows == env.B:
             logp = self._logp(net, amp, k, a, m.view(torch.bool))
-            act = sample_actions(logp.float()) if mode == "sample" else greedy_actions(logp)
+            act = self._act(logp, m, mode, philox)
         else:
             idx = self.live[rows]
-            logp = self._logp(net, amp, k.index_select(0, idx), a.index_select(0, idx), m.index_select(0, idx).view(torch.bool))
-            sub = sample_actions(logp.float()) if mode == "sample" else greedy_actions(logp)
+            ms = m.index_select(0, idx)
+            logp = self._logp(net, amp, k.index_select(0, idx), a.index_select(0, idx), ms.view(torch.bool))
+            sub = self._act(logp, ms, mode, philox, idx)
             # Envs off the list are done and the step ignores their action -- except in the warm-up before the capture, where the list is
             # arbitrary: give them their first legal action there too (a forbidden depot move would send the whole team home, end the
             # episode and advance the env's Philox episode index, so the recorded rollout would no longer replay on a fresh env).
@@ -211,12 +234,15 @@ class GraphedRollout(BatchedRollout):
         env.set_output_buffers(*self.pp[1 - s])
         env.step(act)
         self.t_dev.add_(1)
+        if philox:
+            self.draw[3:].add_(1)
 
-    def _graph(self, net, mode, amp, rows=None):
+    def _graph(self, net, mode, amp, rows=None, philox=False):
         """net: the module the loop calls (the bf16 shadow / FusedPolicy when amp); its parameters keep their addresses, so refreshing them
-        between replays is all an update of the policy needs.  rows: policy rows per decision (None = every env)."""
+        between replays is all an update of the policy needs.  rows: policy rows per decision (None = every env).  philox: sample with
+        the Philox kernel (its launch holds the env's first global id)."""
         rows = self.env.B if rows is None else rows
-        key = (id(net), mode, amp, rows)
+        key = (id(net), mode, amp, rows, self.env.first_gid if philox else None)
         if key not in self._graphs:
             env = self.env
             if rows < env.B:
@@ -228,19 +254,23 @@ class GraphedRollout(BatchedRollout):
                 env.reset()
                 self.t_dev.zero_()
                 for u in range(2):
-                    self._decision(net, mode, amp, u % 2, rows)
+                    self._decision(net, mode, amp, u % 2, rows, philox)
             torch.cuda.current_stream(env.device).wait_stream(side)
             g = torch.cuda.CUDAGraph()
             self.t_dev.zero_()
             with torch.cuda.graph(g):
                 for u in range(self.unroll):
-                    self._decision(net, mode, amp, u % 2, rows)
+                    self._decision(net, mode, amp, u % 2, rows, philox)
             self._graphs[key] = g
         return self._graphs[key]
 
     @torch.no_grad()
-    def run(self, net, mode: str = "sample", generator=None, amp: bool | str = False, replay=None, keep_logp: bool = False) -> Episodes:
-        assert replay is None and not keep_logp and generator is None, "the graphed loop draws from the default CUDA generator and replays nothing"
+    def run(self, net, mode: str = "sample", generator=None, amp: bool | str = False, replay=None, keep_logp: bool = False,
+            sampler: tuple | None = None) -> Episodes:
+        assert replay is None and not keep_logp and generator is None, \
+            "the graphed loop draws from the default CUDA generator or from sampler=(seed, stream), and replays nothing"
+        philox = sampler is not None
+        assert not philox or mode == "sample"
         env = self.env
         assert not env.auto_reset
         was_training = net.training
@@ -248,10 +278,13 @@ class GraphedRollout(BatchedRollout):
         fnet = self._forward_net(net, amp)
         # all captured before the episode starts (a warm-up resets the env), the full batch FIRST: the policy's workspaces are allocated by
         # the largest forward and only sliced by the smaller ones, so no capture ever holds a buffer that a later one replaced
-        graphs = {n: self._graph(fnet, mode, amp, n) for n in sorted(self.sizes, reverse=True)}
+        graphs = {n: self._graph(fnet, mode, amp, n, philox) for n in sorted(self.sizes, reverse=True)}
         env.set_output_buffers(*self.pp[0])
         env.reset()
         self.t_dev.zero_()
+        if philox:
+            from .policy_fused import draw_tensor
+            self.draw.copy_(draw_tensor(int(sampler[0]), int(sampler[1]), 0, env.device))
         t, rows, forwarded = 0, env.B, 0
         while t < self.horizon:
             graphs[rows].replay()
