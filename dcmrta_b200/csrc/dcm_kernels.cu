@@ -9,7 +9,7 @@
 //   k_obs_tile      observation + mask builder, block / tile: TMA bulk loads of the tile's arrays, rows from shared memory, TMA bulk
 //                   stores straight into the policy's input tensors; launched programmatically after k_step           (hot path 3/3)
 //   k_obs           the same rows by register-staged chunks (granular dcm_build_obs, shapes whose tile does not fit twice per SM)
-//   k_episode       dcm_reset (and the dense variant of the episode pass)
+//   k_episode       dcm_reset
 //   k_granular      the individual TaskEnv methods (facade path)
 //   k_routes        execute_by_route: a whole preset-route episode per env in one launch
 //   k_generate      synthetic instances (generate_env distributions) with Philox
@@ -272,7 +272,7 @@ __device__ __forceinline__ unsigned step_env(const EnvArgs& E, const StepArgs& F
         reward_out = __double2float_rn(reward / (double)nm);                  // :337-341
         ++n_steps; EL(c, total, 1, 0) = total + 1;
         t_update_and_advance<TW>(c, st, now, pending, flags, node_of, tr, movers, arrival);    // worker.py:74-76, then :85 / :45-51 while nobody is pending
-        if (flags & ENV_DONE) { leader = -1; group = 0; }                     // episode accounting / restart: k_episode
+        if (flags & ENV_DONE) { leader = -1; group = 0; }                     // episode accounting / restart: k_episode_list
         else {
             group = IA ? pending & (0ull - pending)                           // the lowest pending id acts next (worker.py:170)
                        : f_current_group(c, node_of, pending);                // task_env.py:291-298
@@ -352,11 +352,16 @@ __global__ void __launch_bounds__(STEP_THREADS, 7) k_step_ia(const __grid_consta
 // k_episode: episode accounting (worker.py:87, :103-108) and restart (clear_decisions + first slot + first leader) for
 // the envs that need it -- about 1 env in 125 per step -- done WARP-COOPERATIVELY (lanes over tasks / agents) by the
 // warp that owns the tile, so that this rare, long path stays off the critical path of k_step.
-//   mode 0: envs that k_step just finished (DONE and not yet ACCOUNTED); restart only with DCM_FLAG_AUTO_RESET
-//   mode 1: dcm_reset (every env, or those selected by `which`)
+//   mode 0: envs that k_step just finished (DONE and not yet ACCOUNTED); restart only with DCM_FLAG_AUTO_RESET (k_episode_list)
+//   mode 1: dcm_reset (every env, or those selected by `which`) (k_episode)
 // ---------------------------------------------------------------------------------------------------------------
 #define EPI_WARPS 4
-#define EPI_LIST_MAX_WARPS 4
+// k_episode_list runs EPI_LIST_WARPS envs (warps) per block and EPI_LIST_WARPS_PER_SM warps per SM.  Its __launch_bounds__ are
+// sized for blocks of EPI_LIST_REG_BUDGET_WARPS warps, five per SM: that caps it at 96 registers, which is what lets its warps stay
+// co-resident with two k_obs_tile blocks (DESIGN.md section 4, late round-1 findings (1)).
+#define EPI_LIST_REG_BUDGET_WARPS 4
+#define EPI_LIST_WARPS 2
+#define EPI_LIST_WARPS_PER_SM 8
 struct EpiArgs { int mode; const unsigned char* which; const int* leader_in; int* next_leader; double* metrics;
                  ObsArgs obs; int write_obs; /* mode 0 + auto-reset: write the restarted env's observation (k_obs runs beside this kernel and skips it) */ };
 
@@ -590,9 +595,8 @@ __device__ __forceinline__ void episode_env(const EnvArgs& E, const EpiArgs& P, 
     __syncwarp();
 }
 
-// EPI_WARPS single-warp blocks per tile: block (tile, r) takes the tile's r-th, (r + EPI_WARPS)-th, ... env that needs work.
-// One warp per block, because the blocks that do have work (about one tile in four has an env that ended, rarely two) run
-// for tens of microseconds beside k_obs and must hold as few registers as possible meanwhile; the others exit at once.
+// dcm_reset: EPI_WARPS single-warp blocks per tile; block (tile, r) takes the tile's r-th, (r + EPI_WARPS)-th, ... selected env.
+// The mode-0 selection and the observation argument below are unreachable (dcm_reset passes mode 1, write_obs = 0); left in place.
 template <int TW>
 __global__ void __launch_bounds__(32, 16) k_episode(const __grid_constant__ EnvArgs E, const __grid_constant__ EpiArgs P) {
     extern __shared__ __align__(16) unsigned char epi_smem[];
@@ -614,9 +618,9 @@ __global__ void __launch_bounds__(32, 16) k_episode(const __grid_constant__ EnvA
     }
 }
 
-// The step path's variant: k_step appended the envs whose episode just ended to a list (about 1 env in 150 per pass), so the
-// grid is a few blocks per SM instead of EPI_WARPS blocks per tile -- dispatching 8,192 mostly empty blocks cost ~25 us beside
-// k_obs (profiles/r03a_timeline.txt).  Envs are independent: the order of the list does not matter.
+// The step path's episode pass: k_step appended the envs whose episode just ended to a list (about 1 env in 150 per pass), so
+// the grid is a few blocks per SM instead of EPI_WARPS blocks per tile -- dispatching 8,192 mostly empty blocks cost ~25 us
+// beside k_obs (profiles/r03a_timeline.txt).  Envs are independent: the order of the list does not matter.
 // Shared-memory footprint matters more than anything else here.  Two k_obs_tile blocks leave a 13 kB hole at the top of an
 // SM's shared memory; episode blocks that fit into it run beside them for free, but a block that does not is placed -- it has
 // priority -- at the BOTTOM of the 110 kB an exiting k_obs_tile block frees, after which no second k_obs_tile block fits on that SM
@@ -624,7 +628,7 @@ __global__ void __launch_bounds__(32, 16) k_episode(const __grid_constant__ EnvA
 // member data in registers (1.1 kB of scratch per env), several envs (warps) per block to share the 1 kB the hardware reserves per
 // block, and at most ~100 registers.
 template <int TW>
-__global__ void __launch_bounds__(32 * EPI_LIST_MAX_WARPS, 5) k_episode_list(const __grid_constant__ EnvArgs E, const __grid_constant__ EpiArgs P, const unsigned* elist, const unsigned* ecount,
+__global__ void __launch_bounds__(32 * EPI_LIST_REG_BUDGET_WARPS, 5) k_episode_list(const __grid_constant__ EnvArgs E, const __grid_constant__ EpiArgs P, const unsigned* elist, const unsigned* ecount,
                                                                          unsigned long long* trace) {
     extern __shared__ __align__(16) unsigned char epi_smem[];
     const unsigned n = *ecount, nw = blockDim.x >> 5, warp = threadIdx.x >> 5, lane = threadIdx.x & 31u;
@@ -846,10 +850,10 @@ __global__ void __launch_bounds__(32 * OBS_TILE_MAX_WARPS, 3) k_obs_tile(const _
     __syncthreads();
     asm volatile("griddepcontrol.wait;" ::: "memory");                        // the step kernel's writes are complete and visible (no-op without a programmatic launch)
     if (threadIdx.x == 0 && blockIdx.x < NT) issue_loads(blockIdx.x);
-    // The block walks tiles blockIdx.x, + gridDim.x, ...  Default grid: one block per tile (a single trip).  With two persistent
-    // blocks per SM (DCM_OBS_PERSISTENT=1) the inputs of tile i + 1 land while the TMA engine still reads the staged output of
-    // tile i; measured 138 vs 135 us per pass: the output drain lengthens to 3 us under the extra traffic and the hardware block
-    // scheduler balances the SMs better than a static tile walk beside the episode warps (profiles/r07_persistent_obs.txt).
+    // The block walks tiles blockIdx.x, + gridDim.x, ...; the grid is one block per tile, so it makes a single trip: the in-loop
+    // wait for the previous tile's drain and the next-tile prefetch never run (they served two persistent blocks per SM, measured
+    // slower and removed: DESIGN.md section 4).  The loop form stays because this kernel's register allocation is fragile (72-94
+    // across builds and variants) and the loop form was adopted in part for its allocation; collapsing it wants a measurement of its own.
     unsigned parity = 0; bool draining = false; unsigned prev_tile = 0;
     for (unsigned tile_id = blockIdx.x; tile_id < NT; tile_id += gridDim.x) {
         const int b = (int)(tile_id * 32 + lane);
@@ -1247,15 +1251,13 @@ static int fail_cuda(cudaError_t e, const char* where) {
     g_err = buf; return DCM_ERR_CUDA;
 }
 #define CK(call) do { cudaError_t _e = (call); if (_e != cudaSuccess) return fail_cuda(_e, #call); } while (0)
-// kernels are instantiated for 1, 2 and 4 mask words (T <= 64 / 128 / 254)
-#define LAUNCH_TW(v, kern, grid, block, stream, ...) do { \
-    if ((v)->E.S.TW == 1) kern<1><<<(grid), (block), 0, (stream)>>>(__VA_ARGS__); \
-    else if ((v)->E.S.TW == 2) kern<2><<<(grid), (block), 0, (stream)>>>(__VA_ARGS__); \
-    else kern<4><<<(grid), (block), 0, (stream)>>>(__VA_ARGS__); } while (0)
+// kernels are instantiated for 1, 2 and 4 mask words (T <= 64 / 128 / 254): TW_KERNEL is the instance for the handle's shape
+#define TW_KERNEL(v, kern) ((v)->E.S.TW == 1 ? kern<1> : (v)->E.S.TW == 2 ? kern<2> : kern<4>)
+#define LAUNCH_TW(v, kern, grid, block, smem, stream, ...) TW_KERNEL(v, kern)<<<(grid), (block), (smem), (stream)>>>(__VA_ARGS__)
 
 struct dcm_env {
     int device; EnvArgs E; DcmLayout L; bool have_instances;
-    bool serial_pass;                // DCM_PASS_SERIAL=1 at dcm_create: k_step, k_episode, k_obs one after the other on the caller's stream (cross-check)
+    bool serial_pass;                // DCM_PASS_SERIAL=1 at dcm_create: k_step, k_episode_list, k_obs one after the other on the caller's stream (cross-check)
     unsigned long long* d_trace; size_t trace_units;   // DCM_PASS_TRACE=1: globaltimer stamps of k_obs_tile blocks / k_episode_list warps (tools/obs_trace.py)
     unsigned char* arena; size_t arena_bytes;
     double* metrics;                 // [B,8]
@@ -1265,12 +1267,13 @@ struct dcm_env {
     // dcm_step_host staging
     int* d_action; float* d_agent; float* d_task; unsigned char* d_mask; int* d_leader; float* d_reward; unsigned char* d_done;
     cudaStream_t hstream, hcopy; bool forked;   // dcm_step_host: its stream; a second one for the results k_step alone produces; the last dcm_step recorded ev_fork
-    cudaStream_t side; cudaEvent_t ev_fork, ev_join;   // k_episode runs beside k_obs
-    bool obs_persistent; int sm_count;
+    cudaStream_t side; cudaEvent_t ev_fork, ev_join;   // k_episode_list runs beside k_obs
+    int sm_count;
     bool obs_ready, obs_tile, obs_resets;   // k_obs_tile applies to this handle's shape (DCM_OBS_CHUNKED=1: always k_obs); it also writes restarted envs' observations
-    unsigned* d_elist; unsigned* d_ecount; unsigned pass_no; bool dense_episode;   // ended-env list [B] + two alternating counters (k_episode_list)
-    // DCM_* experiment switches, read ONCE in dcm_create (never on the step path)
-    bool sw_obs_reset_by_episode, sw_obs_chunked, sw_episode_carveout_default, sw_step_no_nds, sw_no_pdl, sw_no_zero_copy; int epi_warps, epi_per_sm;
+    unsigned* d_elist; unsigned* d_ecount; unsigned pass_no;   // ended-env list [B] + two alternating counters (k_episode_list)
+    // DCM_* cross-checks: second implementations of default paths that the tests compare the defaults against (with serial_pass
+    // above; DCM_PASS_TRACE allocates d_trace).  Read once in dcm_create, never on the step path.
+    bool sw_obs_reset_by_episode, sw_obs_chunked, sw_step_no_nds;
     // dcm_step_host runs on its own stream: it must start after the asynchronous work earlier calls queued on the CALLER's stream
     cudaStream_t last_stream; bool last_pending; cudaEvent_t ev_order;
     uint64_t launches;
@@ -1306,7 +1309,11 @@ int dcm_create(dcm_env** out, int device, int B, int A, int T, int M, uint32_t f
     if (!v) return fail(DCM_ERR_NOMEM, "dcm_create: host allocation failed");
     memset(v, 0, sizeof *v);
     v->device = device;
-    { const char* gs = getenv("DCM_PASS_SERIAL"); v->serial_pass = gs && gs[0] == '1'; }
+    // the cross-checks and the pass trace (dcm_env), once per handle
+    auto on = [](const char* name) { const char* g = getenv(name); return g && g[0] == '1'; };
+    v->serial_pass = on("DCM_PASS_SERIAL"); v->sw_obs_chunked = on("DCM_OBS_CHUNKED"); v->sw_obs_reset_by_episode = on("DCM_OBS_RESET_BY_EPISODE");
+    v->sw_step_no_nds = on("DCM_STEP_NO_NDS");
+    const bool pass_trace = on("DCM_PASS_TRACE");
     v->L = dcm_make_layout(A, T, M);
     DcmSoa& S = v->E.S;
     S.B = B; S.NT = (B + 31) / 32; S.A = A; S.T = T; S.M = M; S.MC = M; S.TW = T <= 64 ? 1 : (T <= 128 ? 2 : 4);
@@ -1336,24 +1343,15 @@ int dcm_create(dcm_env** out, int device, int B, int A, int T, int M, uint32_t f
     int prio_lo = 0, prio_hi = 0;
     if (e == cudaSuccess) e = cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi);
     // highest priority: the few long episode chains must get their blocks in before the six waves of k_obs that run beside them
-    { const char* gp = getenv("DCM_EPISODE_PRIO"); if (gp && gp[0] == '0') prio_hi = prio_lo; }                       // experiment switch: side stream at normal priority
     if (e == cudaSuccess) e = cudaStreamCreateWithPriority(&v->side, cudaStreamNonBlocking, prio_hi);
     if (e == cudaSuccess) e = cudaEventCreateWithFlags(&v->ev_fork, cudaEventDisableTiming);
     if (e == cudaSuccess) e = cudaEventCreateWithFlags(&v->ev_join, cudaEventDisableTiming);
     if (e == cudaSuccess) e = cudaMalloc((void**)&v->d_elist, (size_t)B * sizeof(unsigned));
     if (e == cudaSuccess) e = cudaMalloc((void**)&v->d_ecount, 2 * sizeof(unsigned));
     if (e == cudaSuccess) e = cudaMemset(v->d_ecount, 0, 2 * sizeof(unsigned));
-    { const char* gs = getenv("DCM_EPISODE_DENSE"); v->dense_episode = gs && gs[0] == '1'; }
-    {   // every other experiment switch, once per handle
-        auto on = [](const char* name) { const char* g = getenv(name); return g && g[0] == '1'; };
-        v->sw_obs_reset_by_episode = on("DCM_OBS_RESET_BY_EPISODE"); v->obs_persistent = on("DCM_OBS_PERSISTENT");   // persistent: measured slower than one block per tile, DESIGN.md section 4
-        v->sw_obs_chunked = on("DCM_OBS_CHUNKED"); v->sw_episode_carveout_default = on("DCM_EPISODE_CARVEOUT_DEFAULT"); v->sw_step_no_nds = on("DCM_STEP_NO_NDS"); v->sw_no_pdl = on("DCM_NO_PDL"); v->sw_no_zero_copy = on("DCM_NO_ZERO_COPY");
-        v->epi_warps = 2; { const char* gw = getenv("DCM_EPISODE_WARPS"); if (gw && atoi(gw) >= 1 && atoi(gw) <= EPI_LIST_MAX_WARPS) v->epi_warps = atoi(gw); }   // envs (warps) per block
-        v->epi_per_sm = 8; { const char* gg = getenv("DCM_EPISODE_GRID"); if (gg && atoi(gg) > 0) v->epi_per_sm = atoi(gg); }                                  // warps per SM
-    }
     if (e == cudaSuccess) e = cudaDeviceGetAttribute(&v->sm_count, cudaDevAttrMultiProcessorCount, device);
     if (e == cudaSuccess) e = cudaEventCreateWithFlags(&v->ev_order, cudaEventDisableTiming);
-    { const char* tr = getenv("DCM_PASS_TRACE"); if (e == cudaSuccess && tr && tr[0] == '1') { v->trace_units = (size_t)NT * 64; e = cudaMalloc((void**)&v->d_trace, v->trace_units * 4 * sizeof(unsigned long long)); if (e == cudaSuccess) e = cudaMemset(v->d_trace, 0, v->trace_units * 4 * sizeof(unsigned long long)); } }
+    if (e == cudaSuccess && pass_trace) { v->trace_units = (size_t)NT * 64; e = cudaMalloc((void**)&v->d_trace, v->trace_units * 4 * sizeof(unsigned long long)); if (e == cudaSuccess) e = cudaMemset(v->d_trace, 0, v->trace_units * 4 * sizeof(unsigned long long)); }
     if (e != cudaSuccess) { dcm_destroy(v); return e == cudaErrorMemoryAllocation ? fail(DCM_ERR_NOMEM, "dcm_create: cudaMalloc failed") : fail_cuda(e, "dcm_create"); }
     unsigned char* a = v->arena;
     S.t_slot_arr = (double*)(a + o_slot_arr); S.t_rec = (double*)(a + o_t_rec); S.a_rec = (double*)(a + o_a_rec); S.a_obs = (double*)(a + o_a_obs);
@@ -1462,17 +1460,12 @@ static int launch_obs_tile(dcm_env* v, const ObsArgs& O, cudaStream_t s, bool pr
     const int warps = NA + NR < OBS_TILE_MAX_WARPS ? NA + NR : OBS_TILE_MAX_WARPS;
     const size_t smem = obs_tile_smem(A, T).total;
     const int use_bulk = (((uintptr_t)O.agent_obs | (uintptr_t)O.task_obs | (uintptr_t)O.mask) & 15u) == 0;
-    int grid = v->E.S.NT;                                                    // one block per tile (DCM_OBS_PERSISTENT=1: two persistent blocks per SM walk the tiles)
-    if (v->obs_persistent && grid > 2 * v->sm_count) grid = 2 * v->sm_count;
     cudaLaunchConfig_t cfg; memset(&cfg, 0, sizeof cfg);
-    cfg.gridDim = dim3(grid); cfg.blockDim = dim3(32 * warps); cfg.dynamicSmemBytes = smem; cfg.stream = s;
+    cfg.gridDim = dim3(v->E.S.NT); cfg.blockDim = dim3(32 * warps); cfg.dynamicSmemBytes = smem; cfg.stream = s;   // one block per tile
     cudaLaunchAttribute attr; memset(&attr, 0, sizeof attr);
     attr.id = cudaLaunchAttributeProgrammaticStreamSerialization; attr.val.programmaticStreamSerializationAllowed = 1;
-    if (programmatic && !v->sw_no_pdl) { cfg.attrs = &attr; cfg.numAttrs = 1; }   // after k_step in dcm_step: resident early, waits in griddepcontrol.wait
-    unsigned long long* trace = v->d_trace;
-    if (v->E.S.TW == 1) CK(cudaLaunchKernelEx(&cfg, k_obs_tile<1>, v->E, O, use_bulk, trace));
-    else if (v->E.S.TW == 2) CK(cudaLaunchKernelEx(&cfg, k_obs_tile<2>, v->E, O, use_bulk, trace));
-    else CK(cudaLaunchKernelEx(&cfg, k_obs_tile<4>, v->E, O, use_bulk, trace));
+    if (programmatic) { cfg.attrs = &attr; cfg.numAttrs = 1; }               // after k_step in dcm_step: resident early, waits in griddepcontrol.wait
+    CK(cudaLaunchKernelEx(&cfg, TW_KERNEL(v, k_obs_tile), v->E, O, use_bulk, v->d_trace));
     CK(cudaGetLastError());
     v->launches++;
     return DCM_OK;
@@ -1489,18 +1482,12 @@ static int prepare_obs(dcm_env* v) {
     CK(cudaDeviceGetAttribute(&per_sm, cudaDevAttrMaxSharedMemoryPerMultiprocessor, v->device));
     const size_t smem = obs_tile_smem(v->E.S.A, v->E.S.T).total;
     if (smem > (size_t)optin || 2 * (smem + 1024) > (size_t)per_sm) return DCM_OK;
-    const void* fn = v->E.S.TW == 1 ? (const void*)k_obs_tile<1> : v->E.S.TW == 2 ? (const void*)k_obs_tile<2> : (const void*)k_obs_tile<4>;
-    CK(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, optin));   // per function, not per handle: the device maximum
-    CK(cudaFuncSetAttribute(fn, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+    CK(cudaFuncSetAttribute(TW_KERNEL(v, k_obs_tile), cudaFuncAttributeMaxDynamicSharedMemorySize, optin));   // per function, not per handle: the device maximum
+    CK(cudaFuncSetAttribute(TW_KERNEL(v, k_obs_tile), cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
     // The episode kernel runs BESIDE this one and has to share SMs with it: blocks of kernels that ask for different L1 /
     // shared-memory splits do not become co-resident on an SM (measured: side by side the two kernels took as long as one
     // after the other, profiles/r03_timeline.txt), so it asks for the same split.
-    const void* fe = v->E.S.TW == 1 ? (const void*)k_episode_list<1> : v->E.S.TW == 2 ? (const void*)k_episode_list<2> : (const void*)k_episode_list<4>;
-    const void* fd = v->E.S.TW == 1 ? (const void*)k_episode<1> : v->E.S.TW == 2 ? (const void*)k_episode<2> : (const void*)k_episode<4>;
-    if (!v->sw_episode_carveout_default) {
-        CK(cudaFuncSetAttribute(fe, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-        CK(cudaFuncSetAttribute(fd, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-    }
+    CK(cudaFuncSetAttribute(TW_KERNEL(v, k_episode_list), cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
     v->obs_tile = true;
     return DCM_OK;
 }
@@ -1511,31 +1498,18 @@ static int launch_obs(dcm_env* v, const ObsArgs& O, cudaStream_t s, bool program
     const int tiles_per_block = OBS_THREADS / 32;
     const int NA = (v->E.S.A + OBS_AGENTS_PER_CHUNK - 1) / OBS_AGENTS_PER_CHUNK, NR = (v->E.S.T + 1 + OBS_ROWS_PER_CHUNK - 1) / OBS_ROWS_PER_CHUNK;
     const dim3 grid((v->E.S.NT + tiles_per_block - 1) / tiles_per_block, NA + NR);
-    LAUNCH_TW(v, k_obs, grid, OBS_THREADS, s, v->E, O);
+    LAUNCH_TW(v, k_obs, grid, OBS_THREADS, 0, s, v->E, O);
     CK(cudaGetLastError());
     v->launches++;
     return DCM_OK;
 }
 
 static int launch_episode_list(dcm_env* v, const EpiArgs& P, const unsigned* ecount, cudaStream_t s) {
-    const int nw = v->epi_warps;                                              // envs (warps) per block
+    const int nw = EPI_LIST_WARPS;
     const size_t smem = nw * ((epi_scratch_bytes(v->E.S.A, v->E.S.T, v->E.S.MC) + 15) / 16 * 16);
-    int grid = (v->sm_count * v->epi_per_sm + nw - 1) / nw; if (grid > v->E.S.B) grid = v->E.S.B;
+    int grid = (v->sm_count * EPI_LIST_WARPS_PER_SM + nw - 1) / nw; if (grid > v->E.S.B) grid = v->E.S.B;
     if (v->d_trace) CK(cudaMemsetAsync(v->d_trace + (size_t)v->E.S.NT * 8, 0, (size_t)grid * nw * 4 * sizeof(unsigned long long), s));
-    if (v->E.S.TW == 1) k_episode_list<1><<<grid, 32 * nw, smem, s>>>(v->E, P, v->d_elist, ecount, v->d_trace);
-    else if (v->E.S.TW == 2) k_episode_list<2><<<grid, 32 * nw, smem, s>>>(v->E, P, v->d_elist, ecount, v->d_trace);
-    else k_episode_list<4><<<grid, 32 * nw, smem, s>>>(v->E, P, v->d_elist, ecount, v->d_trace);
-    CK(cudaGetLastError());
-    v->launches++;
-    return DCM_OK;
-}
-
-static int launch_episode(dcm_env* v, const EpiArgs& P, cudaStream_t s) {
-    const size_t smem = epi_scratch_bytes(v->E.S.A, v->E.S.T, v->E.S.MC);
-    const int grid = v->E.S.NT * EPI_WARPS;
-    if (v->E.S.TW == 1) k_episode<1><<<grid, 32, smem, s>>>(v->E, P);
-    else if (v->E.S.TW == 2) k_episode<2><<<grid, 32, smem, s>>>(v->E, P);
-    else k_episode<4><<<grid, 32, smem, s>>>(v->E, P);
+    LAUNCH_TW(v, k_episode_list, grid, 32 * nw, smem, s, v->E, P, v->d_elist, ecount, v->d_trace);
     CK(cudaGetLastError());
     v->launches++;
     return DCM_OK;
@@ -1549,8 +1523,9 @@ int dcm_reset(dcm_env* v, const uint8_t* which, const int32_t* leader_in, float*
     cudaStream_t s = (cudaStream_t)stream;
     note_stream(v, s);
     EpiArgs P{1, which, leader_in, next_leader, v->metrics, ObsArgs{nullptr, nullptr, nullptr, nullptr, 0}, 0};
-    int rc = launch_episode(v, P, s);
-    if (rc) return rc;
+    LAUNCH_TW(v, k_episode, v->E.S.NT * EPI_WARPS, 32, epi_scratch_bytes(v->E.S.A, v->E.S.T, v->E.S.MC), s, v->E, P);
+    CK(cudaGetLastError());
+    v->launches++;
     ObsArgs O{nullptr, agent_obs, task_obs, mask, 0};
     if (agent_obs || task_obs || mask) return launch_obs(v, O, s);
     return DCM_OK;
@@ -1572,9 +1547,8 @@ int dcm_step(dcm_env* v, const int32_t* action, const int32_t* followers, int fs
     ObsArgs O{nullptr, agent_obs, task_obs, mask, 0};
     EpiArgs P{0, nullptr, next_leader_in, next_leader, v->metrics, O, 0};
     const bool want_obs = agent_obs || task_obs || mask;
-    const bool use_list = !v->dense_episode;
-    unsigned* ecount = nullptr;
-    if (use_list) { const unsigned p = v->pass_no++ & 1u; ecount = v->d_ecount + p; F.elist = v->d_elist; F.ecount = ecount; F.ecount_next = v->d_ecount + (p ^ 1u); }
+    const unsigned p = v->pass_no++ & 1u;
+    unsigned* ecount = v->d_ecount + p; F.elist = v->d_elist; F.ecount = ecount; F.ecount_next = v->d_ecount + (p ^ 1u);
     if (v->d_trace) {                                                         // the last two words of the trace buffer: k_step's first entry / last exit
         F.trace = v->d_trace + v->trace_units * 4 - 2;
         CK(cudaMemsetAsync(F.trace, 0xff, sizeof(unsigned long long), s)); CK(cudaMemsetAsync(F.trace + 1, 0, sizeof(unsigned long long), s));
@@ -1582,23 +1556,17 @@ int dcm_step(dcm_env* v, const int32_t* action, const int32_t* followers, int fs
     {
         F.use_nds = v->E.S.A <= STEP_NDS_MAX_AGENTS && !v->sw_step_no_nds;
         const int grid = grid_env(v, STEP_THREADS); const size_t smem = step_smem_bytes(v->E.S.A, v->E.S.ANB, F.use_nds != 0);
-        if (v->E.cflags & DCM_FLAG_INDIVIDUAL) {
-            if (v->E.S.TW == 1) k_step_ia<1><<<grid, STEP_THREADS, smem, s>>>(v->E, F);
-            else if (v->E.S.TW == 2) k_step_ia<2><<<grid, STEP_THREADS, smem, s>>>(v->E, F);
-            else k_step_ia<4><<<grid, STEP_THREADS, smem, s>>>(v->E, F);
-        }
-        else if (v->E.S.TW == 1) k_step<1><<<grid, STEP_THREADS, smem, s>>>(v->E, F);
-        else if (v->E.S.TW == 2) k_step<2><<<grid, STEP_THREADS, smem, s>>>(v->E, F);
-        else k_step<4><<<grid, STEP_THREADS, smem, s>>>(v->E, F);
+        if (v->E.cflags & DCM_FLAG_INDIVIDUAL) LAUNCH_TW(v, k_step_ia, grid, STEP_THREADS, smem, s, v->E, F);
+        else LAUNCH_TW(v, k_step, grid, STEP_THREADS, smem, s, v->E, F);
     }
     CK(cudaGetLastError());
     v->launches++;
     // Episode accounting (+ restart with DCM_FLAG_AUTO_RESET) of the envs that just finished; the injected leader of a
     // restarted env is the same next_leader_in entry.  The episode kernel is a few hundred long, latency-bound warp
     // chains (~30 us) and k_obs is bandwidth-bound (~60 us): they run side by side.  k_obs leaves out the envs k_step marked
-    // `ended`; k_episode writes the observation of the envs it restarts from registers (episode_env).
+    // `ended`; k_episode_list writes the observation of the envs it restarts from registers (episode_env).
     if (v->serial_pass || !want_obs) {
-        int rc = use_list ? launch_episode_list(v, P, ecount, s) : launch_episode(v, P, s);
+        int rc = launch_episode_list(v, P, ecount, s);
         if (rc) return rc;
         if (want_obs) return launch_obs(v, O, s);
         return DCM_OK;
@@ -1613,7 +1581,7 @@ int dcm_step(dcm_env* v, const int32_t* action, const int32_t* followers, int fs
     P.obs = O; P.write_obs = (auto_reset && !obs_resets) ? 1 : 0;
     O.skip_ended = obs_resets ? 2 : 1;
     CK(cudaStreamWaitEvent(v->side, v->ev_fork, 0));
-    int rc = use_list ? launch_episode_list(v, P, ecount, v->side) : launch_episode(v, P, v->side);
+    int rc = launch_episode_list(v, P, ecount, v->side);
     if (rc) return rc;
     CK(cudaEventRecord(v->ev_join, v->side));
     rc = launch_obs(v, O, s, true);
@@ -1654,7 +1622,7 @@ int dcm_step_host(dcm_env* v, const int32_t* action, int policy, float* agent_ob
     const int32_t* act_d = v->d_action;
     if (action) {
         cudaPointerAttributes pa;
-        if (!v->sw_no_zero_copy && cudaPointerGetAttributes(&pa, action) == cudaSuccess && pa.type == cudaMemoryTypeHost && pa.devicePointer)
+        if (cudaPointerGetAttributes(&pa, action) == cudaSuccess && pa.type == cudaMemoryTypeHost && pa.devicePointer)
             act_d = (const int32_t*)pa.devicePointer;
         else { cudaGetLastError(); CK(cudaMemcpyAsync(v->d_action, action, B * 4, cudaMemcpyHostToDevice, s)); }
     }
@@ -1691,7 +1659,7 @@ int dcm_episode_metrics(dcm_env* v, double* out, void* stream) {
 static int launch_gran(dcm_env* v, const GranArgs& G, void* stream) {
     if (!v->have_instances) return fail(DCM_ERR_STATE, "granular op: load or generate instances first");
     DeviceGuard g(v->device);
-    LAUNCH_TW(v, k_granular, grid_env(v, STEP_THREADS), STEP_THREADS, (cudaStream_t)stream, v->E, G);
+    LAUNCH_TW(v, k_granular, grid_env(v, STEP_THREADS), STEP_THREADS, 0, (cudaStream_t)stream, v->E, G);
     CK(cudaGetLastError());
     note_stream(v, (cudaStream_t)stream);
     v->launches++;
@@ -1749,7 +1717,7 @@ int dcm_execute_by_route(dcm_env* v, const int32_t* routes, int rstride, const i
     if (!v->have_instances) return fail(DCM_ERR_STATE, "dcm_execute_by_route: load instances first");
     DeviceGuard g(v->device);
     if (!v->d_cursor) CK(cudaMalloc(&v->d_cursor, (size_t)v->E.S.B * v->E.S.A));
-    LAUNCH_TW(v, k_routes, grid_env(v, STEP_THREADS), STEP_THREADS, (cudaStream_t)stream, v->E, routes, rstride, route_len, v->d_cursor, makespan);
+    LAUNCH_TW(v, k_routes, grid_env(v, STEP_THREADS), STEP_THREADS, 0, (cudaStream_t)stream, v->E, routes, rstride, route_len, v->d_cursor, makespan);
     CK(cudaGetLastError());
     note_stream(v, (cudaStream_t)stream);
     v->launches++;
@@ -1766,7 +1734,7 @@ int dcm_export_state(dcm_env* v, void* dst, size_t bytes, void* stream) {
     if (!v->d_record) { CK(cudaMalloc(&v->d_record, need)); }
     cudaStream_t s = (cudaStream_t)stream;
     CK(cudaMemsetAsync(v->d_record, 0, need, s));
-    LAUNCH_TW(v, k_export, grid_env(v, 128), 128, s, v->E, v->L, v->d_record);
+    LAUNCH_TW(v, k_export, grid_env(v, 128), 128, 0, s, v->E, v->L, v->d_record);
     CK(cudaGetLastError());
     v->launches++;
     CK(cudaMemcpyAsync(dst, v->d_record, need, cudaMemcpyDefault, s));
@@ -1780,7 +1748,7 @@ int dcm_import_state(dcm_env* v, const void* src, size_t bytes, void* stream) {
     if (!v->d_record) { CK(cudaMalloc(&v->d_record, need)); }
     cudaStream_t s = (cudaStream_t)stream;
     CK(cudaMemcpyAsync(v->d_record, src, need, cudaMemcpyDefault, s));
-    LAUNCH_TW(v, k_import, grid_env(v, 128), 128, s, v->E, v->L, v->d_record);
+    LAUNCH_TW(v, k_import, grid_env(v, 128), 128, 0, s, v->E, v->L, v->d_record);
     CK(cudaGetLastError());
     note_stream(v, s);
     v->launches++;

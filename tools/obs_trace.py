@@ -17,7 +17,7 @@ env.generate(); env.reset()
 for _ in range(700): env.step(policy="random")
 torch.cuda.synchronize()
 NT = (B + 31) // 32
-EB = 148 * int(os.environ.get("DCM_EPISODE_GRID", "8")) + 8   # warps of k_episode_list (one env each)
+EB = 148 * 8 + 8   # warps of k_episode_list (one env each): EPI_LIST_WARPS_PER_SM = 8 per SM (csrc/dcm_kernels.cu)
 pc = lambda x: np.percentile(x, [0, 10, 50, 90, 99, 100]).round(2)
 for p in range(PASSES):
     env.step(policy="random"); torch.cuda.synchronize()
