@@ -443,7 +443,7 @@ __device__ __forceinline__ double w_episode_metrics8(const TC& c, const St<TW>& 
             const double w_ab = (double)cur.nab * c.W;
             double v = w_ab;
             if (n) {
-                double acc = 0.0;
+                double acc = 0.0;                                             // sequential, also at 8 terms: see DESIGN.md §2
 #pragma unroll
                 for (int s2 = 0; s2 < 8; ++s2) if (s2 < n) acc += feas ? (mx - cur.a[s2]) : (now - cur.a[s2]);
                 v = acc + w_ab;
@@ -997,7 +997,7 @@ __global__ void __launch_bounds__(STEP_THREADS) k_granular(const __grid_constant
     const double now = EL(c, now, 1, 0);
     St<TW> st, st0; ld_state(c, st); st0 = st;
     switch (G.op) {
-    case OP_NEXT_DECISION: { double t; const u64 d = t_next_decision(c, t); G.deciders[b] = d; G.t[b] = t; } break;
+    case OP_NEXT_DECISION: { double t; const u64 d = t_next_decision(c, t, &st.xlast); G.deciders[b] = d; G.t[b] = t; } break;
     case OP_UNIQUE_GROUP: {
         signed char* out = G.group_rank + (size_t)b * c.A;
         for (int i = 0; i < c.A; ++i) out[i] = -1;
@@ -1036,7 +1036,7 @@ __global__ void __launch_bounds__(STEP_THREADS) k_granular(const __grid_constant
         EL(c, flags, 1, 0) = flags;
     } break;
     case OP_CHECK_FINISHED: {
-        double t; const u64 d = t_next_decision(c, t);
+        double t; const u64 d = t_next_decision(c, t, &st.xlast);
         bool fin = false;
         if (d == 0) { fin = t_all_returned_and_finished(c, st); EL(c, now, 1, 0) = t; }
         G.finished[b] = fin ? 1 : 0;
@@ -1065,17 +1065,20 @@ __global__ void __launch_bounds__(STEP_THREADS) k_routes(const __grid_constant__
     c.tmp = tmp_smem + threadIdx.x;
     double now = EL(c, now, 1, 0); unsigned flags = EL(c, flags, 1, 0); unsigned n_steps = EL(c, n_steps, 1, 0);
     unsigned char* pos = cursor + (size_t)b * c.A;
-    for (int i = 0; i < c.A; ++i) pos[i] = 0;
+    for (int i = 0; i < c.A; ++i) {
+        pos[i] = 0;
+        if (route_len[(size_t)b * c.A + i] > rstride) flags |= ENV_ERR_ACTION;   // a route longer than its row: only the row is played
+    }
     St<TW> st, st0; ld_state(c, st); st0 = st;
     bool finished = flags & ENV_FINISHED;
-    int guard = 0;
-    while (!finished && now < 200.0 && guard < 100000) {                      // :565
-        double t; const u64 dec = t_next_decision(c, t);                      // :568
+    int empty = 0;
+    while (!finished && now < 200.0) {                                        // :565
+        double t; const u64 dec = t_next_decision(c, t, &st.xlast);           // :568
         now = t;                                                              // :569
         t_task_update(c, st, now, nullptr); t_agent_update(c, st, now, st.route);   // :570-571
         for (u64 d = dec; d; d &= d - 1) {                                    // :572 ascending ids
             const int a = __ffsll((long long)d) - 1;
-            const int p = pos[a], len = route_len[(size_t)b * c.A + a];
+            const int p = pos[a], len = min(route_len[(size_t)b * c.A + a], rstride);
             int act = 0;                                                      // :573-574 empty / exhausted route -> depot
             if (p < len) { act = routes[((size_t)b * c.A + a) * rstride + p]; pos[a] = (unsigned char)(p + 1); }
             if (act < 0 || act > c.T) { flags |= ENV_ERR_ACTION; act = 0; }
@@ -1085,9 +1088,12 @@ __global__ void __launch_bounds__(STEP_THREADS) k_routes(const __grid_constant__
             t_task_update(c, st, now, nullptr); t_agent_update(c, st, now, st.route);   // :586-587
             ++n_steps;
         }
-        double t2; const u64 d2 = t_next_decision(c, t2);                     // :588 check_finished
+        double t2; const u64 d2 = t_next_decision(c, t2, &st.xlast);          // :588 check_finished
         if (d2 == 0) { now = t2; finished = t_all_returned_and_finished(c, st); }
-        ++guard;
+        // Nobody decided in this pass nor in the one before.  An agent at the depot never decides again, so nobody ever will and the
+        // reference `while` would spin forever (routes that leave a task unfinished): stop and flag it, as the fused step does.
+        empty = dec ? 0 : empty + 1;
+        if (!finished && empty >= 2) { flags |= ENV_STUCK; break; }
     }
     if (finished) flags |= ENV_FINISHED;
     flags |= ENV_DONE | ENV_ACCOUNTED;          // metrics are fetched explicitly with dcm_compute_metrics (baselines/CTAS-D.py:80-94)

@@ -58,7 +58,7 @@ struct DcmSoa {
     // ---- per env (rows: 1) ----
     double* now;
     double* x_fin; double* x_amin; double* x_asg; double* x_ret;   // conservative lower bounds that let a step skip whole scans (dcm_thread.cuh St)
-    double* x_last;            // max arrival_time[-1] over the agents (check_finished clock jump, task_env.py:286/369)
+    double* x_last;            // max over the agents of max(arrival_time) (check_finished clock jump, task_env.py:286/369)
     unsigned long long* pending;
     unsigned long long* group;
     unsigned* n_steps; unsigned* episode; unsigned* flags; unsigned* instance; unsigned* total;

@@ -99,7 +99,9 @@ template <int TW> struct St {
     double xfin;    // <= time_finish of every feasible, unfinished task
     double xamin;   // <= earliest member arrival of every non-feasible task that has members
     double xret;    // <= arrival at the depot of every agent that went there and is not `returned` yet
-    double xlast;   // == max over agents of arrival_time[-1] (an agent's arrivals never decrease: it decides at or after its last one)
+    double xlast;   // running maximum of every arrival since the reset == max over agents of max(arrival_time), what next_decision
+                    // returns when everybody is NaN (task_env.py:285-286).  It exceeds the largest LAST arrival only after a preset route
+                    // re-visits a feasible task once it has ended: that agent's next_decision lies in the past and the clock goes back.
 };
 
 __device__ __forceinline__ int ctz64(u64 m) { return __ffsll((long long)m) - 1; }
@@ -491,7 +493,7 @@ template <int TW> __device__ __forceinline__ void t_agent_update(const TC& c, St
 // ---------------------------------------------------------------------------------------------------------------
 // next_decision (task_env.py:283-289): earliest next_decision over the agents, deciders by exact equality (one pass)
 // ---------------------------------------------------------------------------------------------------------------
-__device__ __forceinline__ u64 t_next_decision(const TC& c, double& t_out, const double* xlast = nullptr) {
+__device__ __forceinline__ u64 t_next_decision(const TC& c, double& t_out, const double* xlast) {
     const int A = c.A;
     double mn = CUDART_INF; u64 mask = 0;
     if (c.nds) {                                                              // fused step: the scratch copy in shared memory, no round trip
@@ -512,12 +514,7 @@ __device__ __forceinline__ u64 t_next_decision(const TC& c, double& t_out, const
             else if (v[q] == mn) mask |= 1ull << (i0 + q);                    // :288
         }
     }
-    if (mask == 0) {                                                          // :285-286 everybody is NaN
-        if (xlast) { t_out = *xlast; return 0; }                              // fused protocol: the running maximum of all arrivals (St::xlast)
-        double la = 0.0;
-        for (int i = 0; i < A; ++i) { const double a = AREC(c, i, AR_LAST); la = a > la ? a : la; }
-        t_out = la; return 0;
-    }
+    if (mask == 0) { t_out = *xlast; return 0; }                              // :285-286 everybody is NaN: the running maximum of all arrivals (St::xlast)
     t_out = mn;
     return mask;
 }
@@ -695,9 +692,8 @@ template <int TW> __device__ __noinline__ double t_episode_metrics(const TC& c, 
         double mx = SARR(c, j, 0);
         for (int s = 1; s < n; ++s) { const double a = SARR(c, j, s); mx = a > mx ? a : mx; }
         const bool feas = tbit<TW>(st.feas, j);
-        double acc = 0.0;                                                     // np.sum of < 8 terms is sequential
-        for (int s = 0; s < n; ++s) { const double a = SARR(c, j, s); acc += feas ? (mx - a) : (now - a); }
-        return acc + w_ab;
+        // np.sum: sequential below 8 terms, eight accumulators combined pairwise at 8 (a full coalition of M = 8)
+        return np_sum_le128([&](int s) { const double a = SARR(c, j, s); return feas ? (mx - a) : (now - a); }, 0, n) + w_ab;
     };
     // per-agent sums: tasks in id order, members in list order (:358-362); the W * abandon entries are added at the end
     // (the reference interleaves them per task, :363-364 -- differs by summation order only, ~1e-16 relative)
@@ -723,7 +719,7 @@ template <int TW> __device__ __noinline__ double t_episode_metrics(const TC& c, 
     }
     if (task_wait) for (int j = 0; j < T; ++j) task_wait[j] = task_sum(j);
     // :422 check_finished side effect on the clock
-    double t; const u64 dec = t_next_decision(c, t);
+    double t; const u64 dec = t_next_decision(c, t, &st.xlast);
     if (dec == 0) now = t;
     int nfin = 0;
 #pragma unroll

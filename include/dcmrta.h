@@ -177,7 +177,13 @@ int dcm_check_finished(dcm_env* env, uint8_t* finished_d, void* stream);
  * per-element sums calculate_waiting_time leaves in the dicts: task_wait_d [B,T], agent_wait_d [B,A] f64 (or NULL) */
 int dcm_compute_metrics(dcm_env* env, double* out_d, double* task_wait_d, double* agent_wait_d, void* stream);
 /* pre_set_route + execute_by_route (task_env.py:562-599): routes_d [B,A,rstride] i32 actions (0 = depot), route_len_d [B,A];
- * runs every env to completion in one launch with max_waiting_time = 100 and the 200 clock cap; makespan_d [B] f64 */
+ * runs every env to completion in one launch with max_waiting_time = 100 and the 200 clock cap; makespan_d [B] f64.
+ *   - agent a plays the first min(route_len, rstride) entries of its row, then goes to the depot; an entry above rstride sets
+ *     DCM_ENV_ERR_ACTION on its env (route_len_d is device memory, so only the kernel can check it).  rstride <= 255;
+ *   - an entry outside [0, T] sets DCM_ENV_ERR_ACTION and is played as the depot;
+ *   - routes can leave a task unfinished once every agent is home (an agent at the depot never decides again): the reference
+ *     loop then spins forever.  The env stops after two consecutive passes in which nobody decides, with DCM_ENV_STUCK,
+ *     as dcm_step does.  Every env ends with DCM_ENV_DONE, and DCM_ENV_FINISHED if check_finished was true. */
 int dcm_execute_by_route(dcm_env* env, const int32_t* routes_d, int rstride, const int32_t* route_len_d,
                          double* makespan_d, void* stream);
 

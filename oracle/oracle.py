@@ -227,6 +227,12 @@ class OracleEnv:
             out.append((r[:n].copy(), t[:n].copy()))
         return out
 
+    def agent_scalars(self):
+        """-> (agent sum_waiting_time [A], task sum_waiting_time [T]) as the last calculate_waiting_time (task_env.py:344-364) left them"""
+        aw, tw = np.zeros(self.A, np.float64), np.zeros(self.T, np.float64)
+        lib().orc_agent_scalars(self._h, _p(aw), _p(tw))
+        return aw, tw
+
     # ---- fused driver ---------------------------------------------------------
     def seed(self, seed, gid=0, episode=0):
         lib().orc_seed(self._h, int(seed), int(gid), int(episode))

@@ -463,6 +463,7 @@ void orc_pre_set_route(orc_env *e, int agent, const int *route, int n) {
 /* task_env.py:562-593 execute_by_route (reactive_planning False).  Returns makespan. */
 double orc_execute_by_route(orc_env *e) {
     int ids[ORC_MAX_AGENTS]; double t;
+    int empty = 0;
     e->W = 100;                                                               /* :564 */
     while (!e->finished && e->now < 200) {                                    /* :565 */
         int n = orc_next_decision(e, ids, &t);                                /* :568 */
@@ -475,6 +476,10 @@ double orc_execute_by_route(orc_env *e) {
             orc_task_update(e, NULL); orc_agent_update(e);
         }
         e->finished = orc_check_finished(e);                                  /* :588 */
+        /* Nobody decided in this pass nor in the one before.  An agent at the depot never decides again, so nobody ever will and the
+         * reference `while` spins forever (routes that leave a task unfinished).  Stop and flag it, as orc_advance does. */
+        empty = n ? 0 : empty + 1;
+        if (!e->finished && empty >= 2) { e->stuck = 1; break; }
     }
     return e->now;
 }

@@ -152,6 +152,121 @@ def device_instance(A, T, M, seed, gid, instance=0, max_duration=5.0, random_dur
     return dict(A=A, task_xy=xy, depot_xy=np.array([u01(a[0], a[1]), u01(a[2], a[3])]), req=req, dur=dur)
 
 
+# ---- preset routes (dcm_execute_by_route), shared by tests/test_routes_oracle.py and tests/test_gpu_routes.py ------------------------
+ROUTE_FAMILIES = ("coalition", "short", "partial", "noisy")
+ROUTE_MAX_LEN = 255                     # dcm_execute_by_route: rstride <= 255
+ROUTE_MAX_DURATION = 0.5                # task durations of the route instances: short enough that 64 agents finish 254 tasks under the clock
+
+
+def route_family(b):
+    return ROUTE_FAMILIES[b % len(ROUTE_FAMILIES)]
+
+
+def make_routes(seed, inst, A, M, family):
+    """Preset routes of one env (lists of actions, 0 = depot, j + 1 = task j), seeded.  The tasks are handed out in one sweep of the
+    unit square (six vertical strips, up one and down the next), so no two agents wait for each other in opposite orders and the
+    hops are short enough for 64 agents to finish 254 tasks under the clock cap:
+      coalition  each task to min(req, A) distinct agents drawn at random, appended to their routes;
+      short      one agent fewer than req (at least one): members wait, give up after W = 100 and run into the 200-unit clock;
+      partial    as coalition, but about a tenth of the tasks are never routed: once every agent is home the episode is stuck;
+      noisy      as coalition, plus re-visits, a depot entry in the middle of some routes, empty routes and one route padded with
+                 re-visits of its own tasks to one more entry than any other route of the env.
+    Each task lies on the routes of at most M distinct agents, so no member list overflows and the oracle compares exactly."""
+    rng = np.random.default_rng(seed)
+    xy, req = np.asarray(inst["task_xy"]), inst["req"]
+    strip = np.minimum((xy[:, 0] * 6).astype(int), 5)
+    R = [[] for _ in range(A)]
+    for j in np.lexsort((np.where(strip % 2 == 0, xy[:, 1], -xy[:, 1]), strip)):
+        if family == "partial" and rng.random() < 0.1:
+            continue
+        k = min(int(req[j]), A, M)
+        if family == "short":
+            k = max(k - 1, 1)
+        for a in rng.choice(A, k, replace=False):
+            R[a].append(int(j) + 1)
+    if family == "noisy":
+        for a in range(A):
+            u = rng.random()
+            if u < 0.15:
+                R[a] = []                                                    # an empty route: straight home
+            elif u < 0.45 and R[a]:
+                R[a].insert(int(rng.integers(len(R[a]) + 1)), R[a][int(rng.integers(len(R[a])))])   # re-visit one of its tasks
+            elif u < 0.65 and len(R[a]) > 1:
+                R[a].insert(int(rng.integers(1, len(R[a]))), 0)               # home in the middle: the rest is never played
+        full = [a for a in range(A) if any(R[a])]
+        if full:
+            a = full[int(rng.integers(len(full)))]
+            own = [x for x in R[a] if x]
+            L = min(max(len(r) for r in R) + 1, ROUTE_MAX_LEN)
+            while len(R[a]) < L:
+                R[a].append(own[int(rng.integers(len(own)))])
+    return [r[:ROUTE_MAX_LEN] for r in R]
+
+
+def pack_routes(routes_per_env, A, L=None):
+    """list over envs of per-agent routes -> routes [B, A, L] int32 (zero padded), route_len [B, A] int32"""
+    L = L or max(1, max(len(r) for R in routes_per_env for r in R))
+    out = np.zeros((len(routes_per_env), A, L), np.int32)
+    n = np.zeros((len(routes_per_env), A), np.int32)
+    for b, R in enumerate(routes_per_env):
+        for a, r in enumerate(R):
+            out[b, a, :len(r)] = r
+            n[b, a] = len(r)
+    return out, n
+
+
+def route_oracle(A, inst, R, velocity=0.2):
+    """the oracle after execute_by_route of routes R on instance inst -> (OracleEnv, makespan)"""
+    from oracle.oracle import OracleEnv
+    o = OracleEnv.make(A, inst["task_xy"], inst["depot_xy"], inst["req"], inst["dur"], velocity=velocity)
+    for a, r in enumerate(R):
+        if len(r):
+            o.pre_set_route(np.asarray(r, np.int32), a)
+    return o, o.execute_by_route()
+
+
+def route_census(ev, o, A, T, M, R):
+    """Add to the set `ev` what one execute_by_route episode reached on the oracle `o` (routes R)."""
+    s = o.export(M)
+    ev.add("finished" if s["env_finished"] else ("stuck" if o.stuck else "clock_cap"))
+    if (s["n_mem"] == M).any():
+        ev.add("full_coalition")
+    if s["n_aband_task"].any():
+        ev.add("give_up")
+    played = [r for r, _ in o.routes()]
+    for j, key in ((T - 1, "task_last"), (63, "task_63"), (64, "task_64"), (127, "task_127"), (128, "task_128")):
+        if j < T and any((p == j).any() for p in played):
+            ev.add(key)
+    if (played[A - 1] >= 0).any():
+        ev.add("agent_last")                                          # the last agent (bit A - 1) moved to a task
+    if any((np.diff(t) < 0).any() for _, t in o.routes()):
+        ev.add("clock_back")                                          # a re-visit of an ended task: next_decision in the past, the clock goes back
+    return ev
+
+
+def route_census_needs(shape):
+    """what the route batches of a shape must reach: with M = 1 every task starts on arrival (no wait, no give-up, and one task cannot
+    take 200 units), and A < M agents cannot fill M slots"""
+    need = {"finished", "stuck", "task_last", "agent_last"} | \
+        {key for j, key in ((63, "task_63"), (64, "task_64"), (127, "task_127"), (128, "task_128")) if j < shape.T}
+    if shape.M > 1:
+        need |= {"clock_cap", "give_up"}
+    if shape.A >= shape.M:
+        need.add("full_coalition")
+    if shape.A > 1 and shape.B >= 100:                                # one to ten envs in a hundred re-visit a task after it ended
+        need.add("clock_back")
+    return need
+
+
+def route_batch_sizes(shape):
+    """the batch sizes tests/test_gpu_routes.py plays a shape at: its own B, one env, and one env past a tile of 32"""
+    return sorted({shape.B, 1, 33})
+
+
+def route_seed(shape, b):
+    return 1000 * shape.seed + b
+
+
 def envelope_census(ev, o, A, T, M, leader, used_action, done=False, env=None):
     """Add to the set `ev` what one decision of the oracle reached.  `o` is the OracleEnv after the decision, `leader` the agent that
     decided and `used_action` its action (0 = depot, j + 1 = task j); `env` the OracleEnv whose episode ended (`done`), for its cause."""
