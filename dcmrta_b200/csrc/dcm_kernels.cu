@@ -269,6 +269,8 @@ __device__ __forceinline__ unsigned step_env(const EnvArgs& E, const StepArgs& F
             tr.j = j; tr.n = n; tr.ids = ids; tr.amin = amin; tr.amax = amax;  // the head the evaluation below starts from
             tr.feas = feas_j; tr.ts = ti.x; tr.tf = ti.y;
         }
+        // the mover's next_decision is a time_finish that has passed: the clock goes back at the next slot start (t_watch_reached)
+        if (feas_j && ti.y < now && st.watch) { const u64 r = t_watch_reached(&EL(c, a_ts, A, 0), st.watch, now); st.assigned |= r; st.watch &= ~r; }
         reward_out = __double2float_rn(reward / (double)nm);                  // :337-341
         ++n_steps; EL(c, total, 1, 0) = total + 1;
         t_update_and_advance<TW>(c, st, now, pending, flags, node_of, tr, movers, arrival);    // worker.py:74-76, then :85 / :45-51 while nobody is pending
@@ -365,7 +367,6 @@ __global__ void __launch_bounds__(STEP_THREADS, 7) k_step_ia(const __grid_consta
 struct EpiArgs { int mode; const unsigned char* which; const int* leader_in; int* next_leader; double* metrics;
                  ObsArgs obs; int write_obs; /* mode 0 + auto-reset: write the restarted env's observation (k_obs runs beside this kernel and skips it) */ };
 
-__device__ __forceinline__ double wmax(double v) { for (int o = 16; o > 0; o >>= 1) { const double w = __shfl_xor_sync(0xffffffffu, v, o); v = w > v ? w : v; } return v; }
 __device__ __forceinline__ double wmin(double v) { for (int o = 16; o > 0; o >>= 1) { const double w = __shfl_xor_sync(0xffffffffu, v, o); v = w < v ? w : v; } return v; }
 
 // per-warp scratch of k_episode, carved from dynamic shared memory: the four vectors that are summed (the member data of a task
@@ -423,12 +424,12 @@ __device__ __forceinline__ double w_episode_metrics8(const TC& c, const St<TW>& 
         if (L.feas) L.ts = TINFO(c, jj, 0);
     };
     // agents (lane, lane + 32): issue these loads first as well
-    double a_nd_v[2], a_last[2], a_dist[2]; int a_nab_v[2];
+    double a_nd_v[2], a_dist[2]; int a_nab_v[2];
 #pragma unroll
     for (int r = 0; r < 2; ++r) {
         const int i = lane + 32 * r; const bool in = i < A; const int ii = in ? i : 0;
-        a_nd_v[r] = in ? EL(c, a_nd, A, ii) : CUDART_NAN; const double2 ld = AREC2(c, ii, 1);
-        a_last[r] = in ? ld.x : 0.0; a_dist[r] = ld.y; a_nab_v[r] = in ? (int)EL(c, a_nab, A, ii) : 0;
+        a_nd_v[r] = in ? EL(c, a_nd, A, ii) : CUDART_NAN;
+        a_dist[r] = AREC(c, ii, AR_DIST); a_nab_v[r] = in ? (int)EL(c, a_nab, A, ii) : 0;
     }
     double acc0 = 0.0, acc1 = 0.0;
     TL cur, nxt;
@@ -479,12 +480,13 @@ __device__ __forceinline__ double w_episode_metrics8(const TC& c, const St<TW>& 
             S.s_agent[i] = acc; S.s_dist[i] = a_dist[r];
         }
     }
-    // :422 check_finished side effect on the clock
-    double mn = CUDART_INF, la = 0.0;
+    // :422 check_finished side effect on the clock: when nobody can decide, the largest arrival any agent ever had (St::xlast; it exceeds
+    // the largest LAST arrival once an agent re-visited or joined a task after it ended)
+    double mn = CUDART_INF;
 #pragma unroll
-    for (int r = 0; r < 2; ++r) { if (a_nd_v[r] < mn) mn = a_nd_v[r]; la = a_last[r] > la ? a_last[r] : la; }
-    mn = wmin(mn); la = wmax(la);
-    if (mn == CUDART_INF) now = la;
+    for (int r = 0; r < 2; ++r) if (a_nd_v[r] < mn) mn = a_nd_v[r];
+    mn = wmin(mn);
+    if (mn == CUDART_INF) now = st.xlast;
     int nfin = 0;
 #pragma unroll
     for (int w = 0; w < TW; ++w) nfin += __popcll(st.fin[w]);

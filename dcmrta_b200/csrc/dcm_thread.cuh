@@ -735,6 +735,17 @@ template <int TW> __device__ __noinline__ double t_episode_metrics(const TC& c, 
     return now;
 }
 
+// The clock goes back when a mover joins (or re-visits) a feasible task whose time_finish has passed: its next_decision = time_finish
+// (:231) lies in the past, and the next slot starts there.  The lazy `assigned` of t_agent_update (WATCH, `now >= time_start` read at the
+// current clock) would then forget that agent_update (:232-233) had set it at the later clock already.  So the step settles every watch
+// against the clock before it goes back.  Returns the agents of `watch` whose time_start (a_ts, rows of 32 lanes from ts0) `now` has
+// reached.  Not inlined and given values only: legal play never calls it, and the step's state stays in registers.
+__device__ __noinline__ u64 t_watch_reached(const double* ts0, u64 watch, double now) {
+    u64 r = 0;
+    for (u64 m = watch; m; m &= m - 1) if (now >= ts0[(unsigned)ctz64(m) << 5]) r |= m & (0 - m);
+    return r;
+}
+
 // ---------------------------------------------------------------------------------------------------------------
 // slot boundary (worker.py:45-51, :85): check_finished, loop condition, next_decision, clock, task_update, agent_update
 // ---------------------------------------------------------------------------------------------------------------

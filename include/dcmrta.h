@@ -195,7 +195,15 @@ int dcm_export_state(dcm_env* env, void* dst, size_t bytes, void* stream);
 int dcm_import_state(dcm_env* env, const void* src, size_t bytes, void* stream);
 /* byte offsets of the record fields: out[0..n) as documented in DESIGN.md "record layout"; returns the count written */
 int dcm_layout(const dcm_env* env, int32_t* out, int n);
-/* per-env status bits, [B] u32 */
+/* per-env status bits, [B] u32.
+ * The DCM_ENV_ERR_* bits stay set for the rest of the episode: later legal steps do not clear them.  dcm_reset and an auto-reset
+ * restart clear them; a restart whose injected first leader is >= A sets DCM_ENV_ERR_LEADER for the new episode.
+ *   - DCM_ENV_ERR_ACTION, DCM_ENV_ERR_FOLLOW: dcm_step refuses the decision.  The env's record is unchanged except this word, the
+ *     outputs are reward 0, used_action -1, done 0, the next leader and observation of the unchanged state, and dcm_total_steps does
+ *     not count it.  The env may continue with a legal input.
+ *   - DCM_ENV_ERR_LEADER: the decision is applied; the lowest id of the group leads next (agent 0 at a restart).
+ *   - DCM_ENV_ERR_OVERFLOW: the agent moved to the full task but is not one of its members.
+ * An env that is done and not restarted sets no bit, whatever it is given. */
 int dcm_env_flags(dcm_env* env, uint32_t* flags_d, void* stream);
 /* total leader decisions applied by this handle since creation (device counter read back; synchronises) */
 int dcm_total_steps(dcm_env* env, uint64_t* out_h);

@@ -73,6 +73,7 @@ def lib() -> C.CDLL:
             "orc_done": (i32, [vp]),
             "orc_stuck": (i32, [vp]),
             "orc_pending": (u64, [vp]),
+            "orc_current_group": (u64, [vp]),
             "orc_nsteps": (C.c_long, [vp]),
             "orc_rollout_bench": (C.c_long, [vp, i32, C.c_long, u64, vp]),
         }
@@ -261,6 +262,10 @@ class OracleEnv:
     stuck = property(lambda s: bool(lib().orc_stuck(s._h)))
     pending = property(lambda s: int(lib().orc_pending(s._h)))
     n_steps = property(lambda s: int(lib().orc_nsteps(s._h)))
+
+    def current_group(self):
+        """bitmask of the group that decides now: the pending agents at the lexicographically smallest location (task_env.py:291-298)"""
+        return int(lib().orc_current_group(self._h))
 
     def rollout_bench(self, policy, min_steps, seed=0):
         return int(lib().orc_rollout_bench(self._h, int(policy), int(min_steps), int(seed), None))

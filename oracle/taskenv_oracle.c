@@ -604,7 +604,7 @@ static void orc_advance(orc_env *e) {
 static int choose_leader(orc_env *e, int injected) {
     uint64_t g = current_group(e, e->pending);
     if (!g) return -1;
-    if (injected >= 0) return (g >> injected & 1) ? injected : -2;
+    if (injected >= 0) return (injected < e->A && (g >> injected & 1)) ? injected : -2;
     return kth_bit(g, pick(draw(e, (uint32_t)e->n_steps, 1), popcnt(g)));
 }
 
@@ -658,7 +658,7 @@ int orc_fused_step(orc_env *e, int action, const int *followers, int n_followers
         if (followers) {
             if (n_followers != want) return -4;
             uint64_t gg = g;
-            for (int k = 0; k < want; k++) { if (followers[k] < 0 || !(gg >> followers[k] & 1)) return -5; gg &= ~(1ull << followers[k]); }
+            for (int k = 0; k < want; k++) { if (followers[k] < 0 || followers[k] >= e->A || !(gg >> followers[k] & 1)) return -5; gg &= ~(1ull << followers[k]); }
             for (int k = 0; k < want; k++) { members[nm++] = followers[k]; g &= ~(1ull << followers[k]); }
         } else if (action == 0) {
             /* depot: the whole group follows (Q11); order is irrelevant for the depot, take ascending ids */
@@ -684,6 +684,7 @@ int orc_fused_step(orc_env *e, int action, const int *followers, int n_followers
     return 0;
 }
 
+uint64_t orc_current_group(const orc_env *e) { return current_group(e, e->pending); }
 int orc_leader(const orc_env *e) { return e->leader; }
 int orc_done(const orc_env *e) { return e->done; }
 int orc_stuck(const orc_env *e) { return e->stuck; }

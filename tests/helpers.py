@@ -313,9 +313,9 @@ class EnvelopeOracle:
         self.episodes, self.last_metrics, self.first_end, self.census = 0, None, None, set()
         self._restart()
 
-    def _restart(self):
+    def _restart(self, leader=-1):
         self.o.seed(self.shape.seed, gid=self.gid, episode=self.episodes)
-        self.o.reset() if self.protocol == "IA" else self.o.fused_reset()
+        self.o.reset() if self.protocol == "IA" else self.o.fused_reset(leader)
 
     @property
     def leader(self):
@@ -339,3 +339,136 @@ class EnvelopeOracle:
             self.episodes += 1
             self._restart()
         return r, d, ua
+
+
+# ---- caller-supplied actions (DCM_POLICY_EXTERNAL), shared by tests/test_external_actions_oracle.py (the oracle alone) and
+# tests/test_gpu_external_actions.py (CUDA against the oracle).  The kernel plays any action in [0, T] it is given, as
+# TaskEnv.step does (task_env.py:326-342): masked ones too.  A masked task has status <= 0, so its vacancy moves the leader alone.
+EXTERNAL_EVENTS = ("join_running", "join_finished", "join_satisfied", "clock_back", "revisit_feasible", "depot_masked",
+                   "inject_want_ge2", "follower_last")
+EXT_DEPOT, EXT_REVISIT, EXT_JOIN = 0.04, 0.10, 0.30     # cumulative probabilities of the three masked kinds; the rest is a legal action
+
+
+def external_words(seed, gid, k):
+    """four uniform words of decision k of global env gid: Philox counter (gid_lo, gid_hi, 0xE0000000, k), key = seed, a region the
+    env's own draws (episode numbers) never reach"""
+    from oracle.oracle import philox
+    return [int(x) for x in philox([gid & 0xFFFFFFFF, gid >> 32, 0xE0000000, k], [seed & 0xFFFFFFFF, seed >> 32])]
+
+
+def inject_followers_at(k):
+    """the decisions on which the leader-follower tests draw the followers themselves (the others leave them to the Philox stream)"""
+    return k % 3 == 1
+
+
+def external_steps(shape, protocol="LF"):
+    """decisions the external-action tests play at a shape: enough for every env of the batch to end episodes and reach the census"""
+    steps = shape.steps if protocol == "LF" else shape.ia_steps
+    return min(steps, 200)
+
+
+def external_census_needs(shape, protocol="LF"):
+    """what the external-action trajectories of a shape must reach (external census events, over all envs of the batch).  With one
+    agent nobody else can be on a masked task and nothing can send the clock back"""
+    need = set()
+    if shape.A >= 2:
+        need |= {"join_running", "join_finished", "clock_back", "depot_masked"}
+    return need
+
+
+class ExternalOracle(EnvelopeOracle):
+    """EnvelopeOracle played by caller-supplied actions.  decide(k) draws decision k of this env from external_words: a masked depot, a
+    re-visit of a feasible task the leader is a member of, a masked task with fewer than M members (running, finished, or waiting
+    with status <= 0), else a legal action; and, under leader-follower on the decisions inject_followers_at names, the followers (a
+    random subset of the current group of the size step() draws, in random order).  The draw depends on (seed, gid, k) and on the
+    state only, so the oracle-only test and the GPU test play the same trajectories.  `ext_census` collects EXTERNAL_EVENTS."""
+
+    def __init__(self, shape, b, inst, protocol="LF"):
+        super().__init__(shape, b, inst, protocol)
+        self.ext_census, self.max_joined = set(), 0
+
+    def choose(self, k):
+        """-> (action, kind) of decision k: kind is "legal" or the census event the masked action reaches"""
+        s = self.shape
+        T, M = s.T, s.M
+        w = external_words(s.seed, self.gid, k)
+        mask, L, u = self.env.mask(), self.o.leader, w[0] / 2.0 ** 32
+        kind, action = "legal", None
+        if u < EXT_DEPOT:
+            if mask[0]:
+                kind, action = "depot_masked", 0
+        elif u < EXT_JOIN:
+            st = self.env.export(M)
+            own = (st["members"] == L).any(1)
+            feas, fin = st["feasible"] > 0, st["finished"] > 0
+            if u < EXT_REVISIT:
+                js = np.flatnonzero(feas & own)
+                if len(js):
+                    kind, action = "revisit_feasible", int(js[pick_word(w[1], len(js))]) + 1
+            else:
+                free = (mask[1:] > 0) & (st["n_mem"] < M) & ~own
+                cats = [(n, np.flatnonzero(m)) for n, m in (("join_running", free & feas & ~fin), ("join_finished", free & feas & fin),
+                                                            ("join_satisfied", free & ~feas & (st["status"] <= 0))) if m.any()]
+                if cats:
+                    kind, js = cats[pick_word(w[1], len(cats))]
+                    action = int(js[pick_word(w[2], len(js))]) + 1
+        if action is None:
+            legal = np.flatnonzero(mask == 0)
+            action = int(legal[pick_word(w[3], len(legal))])
+        return action, kind
+
+    def want(self, action):
+        """-> (number of followers step() draws for `action`, the current group without the leader as a bitmask)"""
+        g = self.o.current_group() & ~(1 << self.o.leader)
+        vac = int(self.env.export(self.shape.M)["status"][action - 1]) if action else 0
+        return (min(vac - 1, bin(g).count("1")) if vac > 1 else 0), g
+
+    def draw_followers(self, k, action, fstride):
+        """-> (followers row [fstride] int32, -1 padded, for dcm_step; followers list for the oracle, None for the depot)"""
+        row = np.full(fstride, -1, np.int32)
+        if action == 0:
+            return row, None
+        want, g = self.want(action)
+        ids = [i for i in range(self.shape.A) if g >> i & 1]
+        fol = [int(x) for x in np.random.default_rng((self.shape.seed, self.gid, k)).permutation(ids)[:want]]
+        row[:want] = fol
+        return row, fol
+
+    def decide(self, k, fstride=0, inject=None):
+        """-> (action, followers row or None, followers list or None, kind) of decision k; followers under leader-follower on the
+        decisions inject_followers_at names (or as `inject` says)"""
+        action, kind = self.choose(k)
+        if self.protocol == "LF" and (inject_followers_at(k) if inject is None else inject):
+            return (action, *self.draw_followers(k, action, fstride), kind)
+        return action, None, None, kind
+
+    def apply(self, action, followers=None, next_leader=-1, kind="legal", restart_leader=-1):
+        """the decision on the oracle -> (reward, done, used_action); the census; restarts a finished episode (with `restart_leader`
+        injected when >= 0)"""
+        s, before = self.shape, self.o.current_time
+        if self.protocol == "IA":
+            r, d, ua, _ = self.o.step(action)
+        else:
+            rc, r, d, ua, _ = self.o.fused_step(action, followers, next_leader)
+            assert rc == 0, (s.name, self.gid, rc)
+        if kind != "legal":
+            self.ext_census.add(kind)
+        if kind.startswith("join_"):
+            self.max_joined = max(self.max_joined, int(self.env.export(s.M)["n_mem"][action - 1]))
+        if not d and self.o.current_time < before:
+            self.ext_census.add("clock_back")
+        if followers:
+            if len(followers) >= 2:
+                self.ext_census.add("inject_want_ge2")
+            if s.A - 1 in followers:
+                self.ext_census.add("follower_last")
+        if d:
+            self.last_metrics = np.array([self.o.episode_metrics()[0][k] for k in METRIC_KEYS])
+            self.episodes += 1
+            self._restart(restart_leader)
+        return r, d, ua
+
+
+def pick_word(word, n):
+    """uniform integer in [0, n) from a 32-bit word, as the RNG contract draws (DESIGN.md 5)"""
+    return (int(word) * n) >> 32
