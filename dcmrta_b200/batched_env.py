@@ -308,13 +308,15 @@ class BatchedTaskEnv:
     def export_state(self, envs=None):
         """Decode the records into flat per-env dicts (same field names as the reference's live state, SURVEY App. A)."""
         raw = self.export_raw()
-        return [decode_record(raw[b], self.layout) for b in (range(self.B) if envs is None else envs)]
+        dur = self.get_instances()["dur"].cpu().numpy()
+        return [decode_record(raw[b], self.layout, dur[b]) for b in (range(self.B) if envs is None else envs)]
 
 
-def decode_record(rec: np.ndarray, L: dict) -> dict:
-    """One raw dynamic record -> dict of arrays: n_mem, members[T,MC] (-1 pad), mem_arr, status, feasible, finished,
-    time_start, n_aband_task, node (-1 = depot), has_route, last_arrival, next_decision, travel_dist, assigned, returned,
-    n_aband_agent, now, and the header fields."""
+def decode_record(rec: np.ndarray, L: dict, dur) -> dict:
+    """One raw dynamic record and its env's task durations [T] -> dict of arrays: n_mem, members[T,MC] (-1 pad), mem_arr, status,
+    feasible, finished, time_start, time_finish (time_start + duration once feasible, else 0; task_env.py:257), n_aband_task,
+    node (-1 = depot), has_route, last_arrival, next_decision, travel_dist, assigned, returned, n_aband_agent, now, and the
+    header fields."""
     A, T, MC, Tp, Ap = L["A"], L["T"], L["MC"], L["Tp"], L["Ap"]
     rec = np.ascontiguousarray(rec, dtype=np.uint8)
 
@@ -332,12 +334,14 @@ def decode_record(rec: np.ndarray, L: dict) -> dict:
     aflags = arr(L["o_aflags"], np.uint8, Ap)[:A]
     node = arr(L["o_anode"], np.uint8, Ap)[:A].astype(np.int32)
     node = np.where(node == 0xFF, -1, node)
+    feasible = (tflags & 1).astype(np.uint8)
+    time_start = arr(L["o_tstart"], np.float64, Tp)[:T].copy()
     hdr = np.frombuffer(rec, dtype=_HDR_DTYPE, count=1, offset=L["o_hdr"])[0]
     return dict(
         n_mem=n_mem, members=mem, mem_arr=marr,
         status=arr(L["o_status"], np.int8, Tp)[:T].astype(np.int32),
-        feasible=(tflags & 1).astype(np.uint8), finished=((tflags >> 1) & 1).astype(np.uint8),
-        time_start=arr(L["o_tstart"], np.float64, Tp)[:T].copy(),
+        feasible=feasible, finished=((tflags >> 1) & 1).astype(np.uint8),
+        time_start=time_start, time_finish=np.where(feasible > 0, time_start + np.asarray(dur, np.float64), 0.0),
         n_aband_task=arr(L["o_tnab"], np.uint16, Tp)[:T].astype(np.int32),
         node=node, has_route=(aflags & 1).astype(np.uint8),
         last_arrival=arr(L["o_alast"], np.float64, Ap)[:A].copy(),

@@ -202,7 +202,7 @@ class TaskEnv:
     # ---- dict views -------------------------------------------------------------------------------------------------
     def _state(self):
         if self._cache is None:
-            self._cache = decode_record(self._be.export_raw()[0], self._be.layout)
+            self._cache = decode_record(self._be.export_raw()[0], self._be.layout, self._dur)
         return self._cache
 
     def _keys(self, kind):
@@ -243,7 +243,7 @@ class TaskEnv:
             if key == "time_start":
                 return float(s["time_start"][i]) if s["feasible"][i] else 0
             if key == "time_finish":
-                return float(s["time_start"][i] + self._dur[i]) if s["feasible"][i] else 0
+                return float(s["time_finish"][i]) if s["feasible"][i] else 0
             if key == "time":
                 return float(self._dur[i])
             if key == "sum_waiting_time":

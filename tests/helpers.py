@@ -299,11 +299,13 @@ def envelope_census(ev, o, A, T, M, leader, used_action, done=False, env=None):
 class EnvelopeOracle:
     """One sampled env of an envelope shape on the CPU reference, restarted as an auto-reset handle restarts it: the oracle's
     leader-follower driver (protocol "LF") or the individual-agent loop of tests/ia_oracle.py ("IA"), with the Philox draws of
-    (shape.seed, gid, episode)."""
+    (seed, gid, episode): the shape's seed and global ids unless `seed` and `first_gid` (the global id of env 0) are given."""
 
-    def __init__(self, shape, b, inst, protocol="LF"):
+    def __init__(self, shape, b, inst, protocol="LF", seed=None, first_gid=None):
         from oracle.oracle import OracleEnv
-        self.shape, self.gid, self.protocol = shape, shape.first_gid() + b, protocol
+        self.shape, self.protocol = shape, protocol
+        self.seed = shape.seed if seed is None else seed
+        self.gid = (shape.first_gid() if first_gid is None else first_gid) + b
         if protocol == "IA":
             from ia_oracle import IAOracle
             self.o = IAOracle(shape.A, inst["task_xy"], inst["depot_xy"], inst["req"], inst["dur"])
@@ -314,7 +316,7 @@ class EnvelopeOracle:
         self._restart()
 
     def _restart(self, leader=-1):
-        self.o.seed(self.shape.seed, gid=self.gid, episode=self.episodes)
+        self.o.seed(self.seed, gid=self.gid, episode=self.episodes)
         self.o.reset() if self.protocol == "IA" else self.o.fused_reset(leader)
 
     @property

@@ -15,34 +15,19 @@ from fractions import Fraction
 import numpy as np
 import pytest
 
+from dcmrta_b200._lib import ENV_ERR_ACTION, ENV_ERR_FOLLOW, ENV_ERR_LEADER, ENV_ERR_MASK, ENV_ERR_OVERFLOW
 from oracle import canon
 
+from gpu_env import (assert_metrics_match, check_obs, instances, make_env, outputs, stack_instances, step_host_equals_step,
+                     twin_handles)
 from helpers import ENVELOPE_SHAPES, ExternalOracle, envelope_shape, external_census_needs, external_steps, inject_followers_at
-from test_gpu_shape_envelope import ERR_BITS, assert_metrics_match, assert_same_records, make_env, outputs, with_finish
 
 pytestmark = pytest.mark.gpu
-ERR_OVERFLOW, ERR_ACTION, ERR_FOLLOW, ERR_LEADER = 16, 32, 64, 128
-
-
-def batch_instances(env):
-    inst = {k: v.cpu().numpy() for k, v in env.get_instances().items()}
-    return [{k: inst[k][b] for k in inst} for b in range(env.B)]
 
 
 def flags_offset(env):
     from dcmrta_b200.batched_env import _HDR_DTYPE
     return env.layout["o_hdr"] + _HDR_DTYPE.fields["flags"][1]
-
-
-def check_obs(env, orcs, skip, what):
-    """mask, agent rows and task rows of every env not in `skip` against its oracle's leader"""
-    ag, tk, mk = env.agent_obs.cpu().numpy(), env.task_obs.cpu().numpy(), env.mask_u8.cpu().numpy()
-    for b, o in enumerate(orcs):
-        if b in skip:
-            continue
-        assert np.array_equal(mk[b], o.env.mask()), (what, b, "mask")
-        assert np.array_equal(ag[b], o.env.agent_status(o.leader).astype(np.float32)), (what, b, "agent rows")
-        assert np.array_equal(tk[b], o.env.task_status(o.leader).astype(np.float32)), (what, b, "task rows")
 
 
 def step_outputs(env):
@@ -69,7 +54,7 @@ def assert_episode_metrics(got, want, M, what):
         assert got[c] == want[c], (what, c, got[c], want[c])
 
 
-def final_checks(env, orcs, insts, skip, what):
+def final_checks(env, orcs, skip, what):
     """metrics of every env's last episode, decoded state against oracle.export"""
     met = env.episode_metrics().cpu().numpy()
     states = env.export_state()
@@ -78,7 +63,7 @@ def final_checks(env, orcs, insts, skip, what):
             continue
         if o.last_metrics is not None:
             assert_episode_metrics(met[b], o.last_metrics, o.shape.M, (what, b))
-        d = canon.diff_states(with_finish(states[b], insts[b]["dur"]), o.o.export(canon.MC_CANON))
+        d = canon.diff_states(states[b], o.o.export(canon.MC_CANON))
         assert not d, (what, b, d)
 
 
@@ -86,14 +71,13 @@ def run_external(shape, protocol, steps):
     """auto-reset, DCM_POLICY_EXTERNAL, ExternalOracle's actions and followers, every env of the batch against its oracle at every
     decision; then the last episode's metrics, the state, the error bits and the step counter.  Returns (env, oracles)."""
     env = make_env(shape, protocol)
-    insts = batch_instances(env)
+    orcs = [ExternalOracle(shape, b, inst, protocol) for b, inst in enumerate(instances(env))]
     env.reset()
-    orcs = [ExternalOracle(shape, b, insts[b], protocol) for b in range(shape.B)]
     for b, o in enumerate(orcs):
         assert o.leader == int(env.leader[b]), (shape.name, b)
     for k in range(steps):
         what = (shape.name, protocol, k)
-        check_obs(env, orcs, (), what)
+        check_obs(env, orcs, range(shape.B), what)
         dec = [o.decide(k, shape.M) for o in orcs]
         acts = np.array([d[0] for d in dec], np.int32)
         rows = np.stack([d[1] for d in dec]) if dec[0][1] is not None else None
@@ -101,8 +85,8 @@ def run_external(shape, protocol, steps):
         out = step_outputs(env)
         for b, (o, (a, _, fol, kind)) in enumerate(zip(orcs, dec)):
             check_result(out, b, o, o.apply(a, fol, kind=kind), a, what)
-    final_checks(env, orcs, insts, (), (shape.name, protocol))
-    assert not (env.env_flags().cpu().numpy() & ERR_BITS).any()
+    final_checks(env, orcs, (), (shape.name, protocol))
+    assert not (env.env_flags().cpu().numpy() & ENV_ERR_MASK).any()
     assert env.total_steps() == shape.B * steps
     return env, orcs
 
@@ -129,11 +113,11 @@ def test_external_actions_ia_match_oracle(shape):
 # ---- contract bits -------------------------------------------------------------------------------------------------------------------
 # case -> (bit, least M at which it can be built).  Each case has its own env of one mixed batch.
 CONTRACT_CASES = {
-    "action_minus_one": (ERR_ACTION, 1), "action_T_plus_1": (ERR_ACTION, 1), "action_int_max": (ERR_ACTION, 1),
-    "follow_too_few": (ERR_FOLLOW, 2), "follow_too_many": (ERR_FOLLOW, 2), "follow_duplicate": (ERR_FOLLOW, 3),
-    "follow_id_ge_A": (ERR_FOLLOW, 2), "follow_other_group": (ERR_FOLLOW, 2), "follow_not_pending": (ERR_FOLLOW, 2),
-    "follow_fstride": (ERR_FOLLOW, 3),
-    "leader_outside_group": (ERR_LEADER, 1), "leader_ge_A": (ERR_LEADER, 1), "leader_restart_ge_A": (ERR_LEADER, 1),
+    "action_minus_one": (ENV_ERR_ACTION, 1), "action_T_plus_1": (ENV_ERR_ACTION, 1), "action_int_max": (ENV_ERR_ACTION, 1),
+    "follow_too_few": (ENV_ERR_FOLLOW, 2), "follow_too_many": (ENV_ERR_FOLLOW, 2), "follow_duplicate": (ENV_ERR_FOLLOW, 3),
+    "follow_id_ge_A": (ENV_ERR_FOLLOW, 2), "follow_other_group": (ENV_ERR_FOLLOW, 2), "follow_not_pending": (ENV_ERR_FOLLOW, 2),
+    "follow_fstride": (ENV_ERR_FOLLOW, 3),
+    "leader_outside_group": (ENV_ERR_LEADER, 1), "leader_ge_A": (ENV_ERR_LEADER, 1), "leader_restart_ge_A": (ENV_ERR_LEADER, 1),
     "depot_with_followers": (0, 2),
 }
 CASE_FROM = 4                           # first decision at which a case may fire (follow_other_group: when its slot comes)
@@ -259,11 +243,11 @@ def test_contract_bits_in_a_mixed_batch(name):
     cases = [c for c, (_, m) in CONTRACT_CASES.items() if M >= m]
     owner = {case_env(i): c for i, c in enumerate(cases)}
     env = make_env(shape)
-    insts = batch_instances(env)
+    insts = instances(env)
     b_og = next((b for b, c in owner.items() if c == "follow_other_group"), None)
     if b_og is not None:
         insts[b_og] = other_group_instance(insts[b_og])
-        env.load_instances(*(np.stack([i[k] for i in insts]) for k in ("task_xy", "depot_xy", "req", "dur")))
+        env.load_instances(*stack_instances(insts))
     env.reset()
     orcs = [ExternalOracle(shape, b, insts[b]) for b in range(B)]
     fired, home, cleared, expect = {}, set(), set(), np.zeros(B, np.int64)
@@ -271,7 +255,7 @@ def test_contract_bits_in_a_mixed_batch(name):
     steps = 160
     for k in range(steps):
         what = (name, k)
-        check_obs(env, orcs, (), what)
+        check_obs(env, orcs, range(B), what)
         plans = {}
         for b, c in owner.items():
             if b not in fired:
@@ -333,7 +317,7 @@ def test_contract_bits_in_a_mixed_batch(name):
                 res = o.apply(a, fol, nl, restart_leader=p.get("restart_leader", -1))
                 if owner[b] == "leader_restart_ge_A":
                     assert res[1] and o.leader == 0, (what, "the depot of the whole remaining group ends the episode")
-                    expect[b] = ERR_LEADER
+                    expect[b] = ENV_ERR_LEADER
                 elif owner[b].startswith("leader_"):
                     assert not res[1] and o.leader == nl, (what, owner[b])
                 check_result(out, b, o, res, a, what)
@@ -351,11 +335,11 @@ def test_contract_bits_in_a_mixed_batch(name):
                 home.add(b)
         assert env.total_steps() == total0 + B - len(refused), what
         for b in range(B):
-            assert flags[b] & ERR_BITS == expect[b], (what, b, owner.get(b), flags[b], expect[b])
+            assert flags[b] & ENV_ERR_MASK == expect[b], (what, b, owner.get(b), flags[b], expect[b])
     assert set(fired) == set(owner), ("cases that never fired", sorted(owner[b] for b in set(owner) - set(fired)))
     kept = [owner[b] for b in owner if CONTRACT_CASES[owner[b]][0] and b not in cleared]
     assert not kept, ("case envs whose episode did not end after their case, so no restart was seen to clear the bit", kept)
-    final_checks(env, orcs, insts, (), name)
+    final_checks(env, orcs, (), name)
     env.close()
 
 
@@ -374,7 +358,7 @@ def test_done_env_ignores_any_input(name):
         env.step(np.full(B, junk, np.int32), followers=np.full((B, 3), A + k, np.int32), next_leaders=np.full(B, A + 3, np.int32))
         rew, done, lead, ua = step_outputs(env)
         assert (done == 1).all() and (lead == -1).all() and (rew == 0).all() and (ua == -1).all(), junk
-        assert np.array_equal(env.env_flags().cpu().numpy(), flags0) and not (flags0 & ERR_BITS).any(), junk
+        assert np.array_equal(env.env_flags().cpu().numpy(), flags0) and not (flags0 & ENV_ERR_MASK).any(), junk
         assert np.array_equal(env.export_raw(), raw0), junk
     assert env.total_steps() == total0
     env.close()
@@ -396,13 +380,14 @@ def test_overflow_bit_on_its_envs_only(name):
     B, A, M = shape.B, shape.A, shape.M
     piles = {b: 0 for b in range(5, B, 25)}                         # env -> the task it piles agents on
     env = make_env(shape)
-    insts = batch_instances(env)
+    insts = instances(env)
     env.reset()
     orcs = [ExternalOracle(shape, b, insts[b]) for b in range(B)]
     over = {}
     for k in range(400):
         what = (name, k)
-        check_obs(env, orcs, over, what)
+        live = [b for b in range(B) if b not in over]
+        check_obs(env, [orcs[b] for b in live], live, what)
         inject = inject_followers_at(k)
         dec = [o.decide(k, M) if b not in piles else None for b, o in enumerate(orcs)]
         now = set()
@@ -429,7 +414,7 @@ def test_overflow_bit_on_its_envs_only(name):
                 o.apply(a, fol)
                 st, want = states[sorted(now).index(b)], o.env.export(M)
                 j = a - 1
-                assert flags[b] & ERR_OVERFLOW, (what, b)
+                assert flags[b] & ENV_ERR_OVERFLOW, (what, b)
                 assert st["node"][L] == j and st["travel_dist"][L] == want["travel_dist"][L], (what, b)
                 xy = insts[b]["task_xy"]
                 src = insts[b]["depot_xy"] if before["node"][L] < 0 else xy[before["node"][L]]
@@ -438,43 +423,29 @@ def test_overflow_bit_on_its_envs_only(name):
                 over[b] = k
                 continue
             check_result(out, b, o, o.apply(a, fol, kind=kind), a, what)
-            assert not flags[b] & ERR_BITS, (what, b, flags[b])
+            assert not flags[b] & ENV_ERR_MASK, (what, b, flags[b])
         if len(over) == len(piles):
             break
     assert set(over) == set(piles), ("envs that never overflowed", set(piles) - set(over))
-    final_checks(env, orcs, insts, over, name)
+    final_checks(env, orcs, over, name)
     env.close()
 
 
 def test_step_host_equals_step_on_masked_actions():
     """dcm_step_host (action buffers pageable and pinned on alternate calls) against dcm_step on a twin handle, with ExternalOracle's
     masked action stream at the largest shape: every output at every decision, then the raw records"""
-    import torch
     shape = envelope_shape("64A_254T_8M_B100_random")
-    B, A, T = shape.B, shape.A, shape.T
-    a, h = make_env(shape), make_env(shape)
-    insts = batch_instances(a)
-    a.reset(); h.reset()
-    orcs = [ExternalOracle(shape, b, insts[b]) for b in range(B)]
-    pinned = torch.empty(B, dtype=torch.int32).pin_memory()
-    out = dict(agent_obs=np.empty((B, A, 6), np.float32), task_obs=np.empty((B, T + 1, 5), np.float32),
-               mask=np.empty((B, T + 1), np.uint8), next_leader=np.empty(B, np.int32), reward=np.empty(B, np.float32),
-               done=np.empty(B, np.uint8))
-    for k in range(200):
-        dec = [o.decide(k, inject=False) for o in orcs]
-        acts = np.array([d[0] for d in dec], np.int32)
-        a.step(acts)
-        if k % 2:
-            pinned.copy_(torch.from_numpy(acts))
-            h.step_host(pinned, out)
-        else:
-            h.step_host(acts.copy(), out)
-        want = outputs(a)
-        for n, m in (("agent_obs", "agent_obs"), ("task_obs", "task_obs"), ("mask_u8", "mask"), ("leader", "next_leader"),
-                     ("reward", "reward"), ("done_u8", "done")):
-            assert np.array_equal(want[n], out[m]), (k, n)
-        for b, (o, (x, _, _, kind)) in enumerate(zip(orcs, dec)):
-            r, d, _ = o.apply(x, kind=kind)
-            assert out["reward"][b] == np.float32(r) and bool(out["done"][b]) == d and out["next_leader"][b] == o.leader, (k, b)
-    assert_same_records(a, h, "after 200 decisions")
-    a.close(); h.close()
+    with twin_handles(lambda: make_env(shape)) as (a, h):
+        orcs = [ExternalOracle(shape, b, inst) for b, inst in enumerate(instances(a))]
+        dec = {}
+
+        def actions(k):
+            dec[k] = [o.decide(k, inject=False) for o in orcs]
+            return [d[0] for d in dec[k]]
+
+        def against_oracle(k, out):
+            for b, (o, (x, _, _, kind)) in enumerate(zip(orcs, dec.pop(k))):
+                r, d, _ = o.apply(x, kind=kind)
+                assert out["reward"][b] == np.float32(r) and bool(out["done"][b]) == d and out["next_leader"][b] == o.leader, (k, b)
+
+        step_host_equals_step(a, h, 200, actions, pinned=True, after_step=against_oracle)

@@ -1,31 +1,25 @@
 """GPU tests of the individual-agent (IA) protocol on the fused step path (DCM_FLAG_INDIVIDUAL, BatchedTaskEnv(protocol="IA")) and of the
 batched test-set evaluation (dcmrta_b200.evaluate): against tests/golden/facade_is.npz (the real reference's run_test_IS loop), against the
 IA loop restated on the C oracle (tests/ia_oracle.py), and against the step path's own variants (serial pass, host buffers, shards)."""
+from contextlib import closing
+
 import numpy as np
 import pytest
 
+from dcmrta_b200._lib import ENV_DONE, ENV_ERR_FOLLOW, ENV_ERR_LEADER, ENV_ERR_MASK
 from oracle import canon
 from oracle.oracle import OracleEnv
 
-from helpers import GOLD, METRIC_KEYS, pickle_instances
+from gpu_env import (assert_metrics_match, check_shard_invariance, lockstep, make_env, stack_instances, step_host_equals_step, twin_handles,
+                     twin_steps)
+from helpers import GOLD, METRIC_KEYS, EnvelopeShape, pickle_instances
 from ia_oracle import IAOracle
 
 pytestmark = pytest.mark.gpu
-ERR_BITS = 0xF0                         # DCM_ENV_ERR_OVERFLOW | _ACTION | _FOLLOW | _LEADER
 
 
 def facade_is():
     return np.load(GOLD / "facade_is.npz")
-
-
-def stack(insts):
-    return (np.stack([i["task_xy"] for i in insts]), np.stack([i["depot_xy"] for i in insts]),
-            np.stack([i["req"] for i in insts]).astype(np.int32), np.stack([i["dur"] for i in insts]))
-
-
-def gpu_state(st, dur):
-    st["time_finish"] = np.where(st["feasible"] > 0, st["time_start"] + np.asarray(dur, np.float64), 0.0)
-    return st
 
 
 def nearest_task_module():
@@ -58,12 +52,6 @@ def oracle_metrics(inst, protocol, seed=0, gid=0):
     return np.array([m[k] for k in METRIC_KEYS])
 
 
-def assert_metrics_match(got, want, what):
-    np.testing.assert_allclose(got, want, rtol=1e-12, atol=0, err_msg=what)
-    for c in (0, 1, 2, 3, 5, 6, 7):                     # everything but waiting_time is bit-exact (tests/test_gpu_parity.py)
-        assert got[c] == want[c], (what, METRIC_KEYS[c])
-
-
 def test_replay_reference_run_test_is_through_dcm_step():
     """The three recorded IA episodes in one batch of three, external actions, leaders chosen by the kernel: at every decision the acting
     agent, the clock, the observation digest and the state digest; then the metrics and no contract bit."""
@@ -75,7 +63,7 @@ def test_replay_reference_run_test_is_through_dcm_step():
     B, A, T = len(ids), 20, 50
     n = np.array([len(z[f"{i}/agent"]) for i in ids])
     env = BatchedTaskEnv(B, A, T, M=5, protocol="IA")
-    env.load_instances(*stack(insts))
+    env.load_instances(*stack_instances(insts))
     env.reset()
     for k in range(int(n.max())):
         ag, tk, mk = env.agent_obs.cpu().numpy(), env.task_obs.cpu().numpy(), env.mask_u8.cpu().numpy()
@@ -84,10 +72,10 @@ def test_replay_reference_run_test_is_through_dcm_step():
         act = np.zeros(B, np.int32)
         for b, i in enumerate(ids):
             if k >= n[b]:
-                assert states[b]["flags"] & 1 and leaders[b] == -1, (i, k)
+                assert states[b]["flags"] & ENV_DONE and leaders[b] == -1, (i, k)
                 continue
             assert leaders[b] == z[f"{i}/agent"][k], (i, k)
-            st = gpu_state(states[b], insts[b]["dur"])
+            st = states[b]
             assert st["now"] == z[f"{i}/now"][k], (i, k)
             assert canon.obs_digest(mk[b], ag[b], tk[b]) == int(z[f"{i}/dig_obs"][k]), (i, k)
             assert canon.state_digest(st) == int(z[f"{i}/dig_state"][k]), (i, k)
@@ -97,7 +85,7 @@ def test_replay_reference_run_test_is_through_dcm_step():
         for b in range(B):
             if k < n[b]:
                 assert bool(done[b]) == (k == n[b] - 1), (ids[b], k)
-    assert not (env.env_flags().cpu().numpy() & ERR_BITS).any()
+    assert not (env.env_flags().cpu().numpy() & ENV_ERR_MASK).any()
     met = env.episode_metrics().cpu().numpy()
     states = env.export_state()
     for b, i in enumerate(ids):
@@ -114,124 +102,40 @@ def test_replay_reference_run_test_is_through_dcm_step():
 def test_inkernel_ia_policy_matches_oracle(policy):
     """In-kernel random / greedy IA with auto-reset against the CPU IA loop on the same Philox contract: a sample of a batch of 1,003
     checked at every decision (observations, reward, done, the next acting agent) over at least two episodes each."""
-    from dcmrta_b200 import BatchedTaskEnv
-    B, A, T, STEPS = 1003, 20, 50, 640
-    env = BatchedTaskEnv(B, A, T, M=5, auto_reset=True, seed=4321, first_gid=7_000, protocol="IA")
-    env.generate(max_duration=5.0, random_duration=(policy == "greedy"))
-    inst = {k: v.cpu().numpy() for k, v in env.get_instances().items()}
-    env.reset()
+    shape = EnvelopeShape(20, 50, 5, 1003, policy, None, 640, "", [])
     sample = [0, 1, 2, 31, 32, 500, 1001, 1002]
-    orcs = []
-    for b in sample:
-        o = IAOracle(A, inst["task_xy"][b], inst["depot_xy"][b], inst["req"][b], inst["dur"][b])
-        o.seed(4321, gid=7_000 + b, episode=0)
-        assert o.reset() == int(env.leader[b]) == 0
-        orcs.append(o)
-    episodes = [0] * len(sample)
-    last = [None] * len(sample)
-    for k in range(STEPS):
-        ag, tk, mk = env.agent_obs[sample].cpu().numpy(), env.task_obs[sample].cpu().numpy(), env.mask_u8[sample].cpu().numpy()
-        for q, o in enumerate(orcs):
-            a = o.leader
-            assert np.array_equal(mk[q], o.mask()), (policy, sample[q], k)
-            assert np.array_equal(ag[q], o.agent_status(a).astype(np.float32)), (policy, sample[q], k)
-            assert np.array_equal(tk[q], o.task_status(a).astype(np.float32)), (policy, sample[q], k)
-        env.step(policy=policy)
-        rew, done, lead = env.reward[sample].cpu().numpy(), env.done_u8[sample].cpu().numpy(), env.leader[sample].cpu().numpy()
-        for q, o in enumerate(orcs):
-            r, d, _, _ = o.step(-1 if policy == "random" else -2)
-            assert rew[q] == np.float32(r), (policy, sample[q], k)
-            assert bool(done[q]) == d, (policy, sample[q], k)
-            if d:
-                last[q] = o.episode_metrics()[0]
-                episodes[q] += 1
-                o.seed(4321, gid=7_000 + sample[q], episode=episodes[q])
-                o.reset()
-            assert lead[q] == o.leader, (policy, sample[q], k)
-    assert min(episodes) >= 2
-    met = env.episode_metrics()[sample].cpu().numpy()
-    for q in range(len(sample)):
-        assert_metrics_match(met[q], np.array([last[q][key] for key in METRIC_KEYS]), (policy, sample[q]))
-    states = env.export_state(sample)
-    for q, o in enumerate(orcs):
-        assert not canon.diff_states(gpu_state(states[q], inst["dur"][sample[q]]), o.export(canon.MC_CANON)), (policy, sample[q])
-    assert not (env.env_flags().cpu().numpy() & ERR_BITS).any()
-    assert env.total_steps() == B * STEPS
-    env.close()
+    with closing(make_env(shape, "IA", seed=4321, first_gid=7_000)) as env:
+        env.reset()
+        assert (env.leader[sample] == 0).all()                          # an IA episode starts with agent 0
+        lockstep(env, shape, sample, shape.ia_steps, seed=4321, first_gid=7_000)
 
 
 @pytest.mark.parametrize("shape,policy", [((20, 50), "random"), ((20, 50), "greedy"), ((30, 100), "random"), ((50, 200), "greedy")])
-def test_ia_fused_pass_equals_serial_pass(shape, policy, monkeypatch):
+def test_ia_fused_pass_equals_serial_pass(shape, policy):
     """IA: the default pass against DCM_PASS_SERIAL (k_step, episode kernel, k_obs one after the other) on 4,099 envs, raw records of
     every env and every output at checkpoints; one shape per mask width (k_step_ia<1>, <2>, <4>)."""
-    from dcmrta_b200 import BatchedTaskEnv
     A, T = shape
     B = 4099
-    fused = BatchedTaskEnv(B, A, T, auto_reset=True, seed=13, first_gid=5, protocol="IA")
-    monkeypatch.setenv("DCM_PASS_SERIAL", "1")
-    other = BatchedTaskEnv(B, A, T, auto_reset=True, seed=13, first_gid=5, protocol="IA")
-    monkeypatch.delenv("DCM_PASS_SERIAL")
-    for e in (fused, other):
-        e.generate(max_duration=5.0, random_duration=(policy == "greedy"))
-        e.reset()
-    ended = 0
     steps = 10 * (A + T)                                            # about four IA episodes per env at every shape (50A/200T: ~650 decisions each)
-    for k in range(steps):
-        fused.step(policy=policy)
-        other.step(policy=policy)
-        ended += int(fused.done_u8.sum())
-        if k % 50 == 49 or k < 3 or k == steps - 1:
-            for name in ("reward", "leader", "done_u8", "used_action", "agent_obs", "task_obs", "mask_u8"):
-                assert np.array_equal(getattr(fused, name).cpu().numpy(), getattr(other, name).cpu().numpy()), (name, k)
-            a, b = fused.export_raw(), other.export_raw()
-            assert np.array_equal(a, b), (k, np.flatnonzero((a != b).any(1))[:8])
-    assert ended > 2 * B                                            # restarts were exercised
-    assert np.array_equal(fused.episode_metrics().cpu().numpy(), other.episode_metrics().cpu().numpy())
-    assert not (fused.env_flags().cpu().numpy() & ERR_BITS).any()
-    fused.close(); other.close()
+    sh = EnvelopeShape(A, T, 5, B, policy, None, steps, "", [])
+    with twin_handles(lambda: make_env(sh, "IA", seed=13, first_gid=5), "DCM_PASS_SERIAL") as (fused, other):
+        ended = twin_steps(fused, other, policy, steps, lambda k: k % 50 == 49 or k < 3 or k == steps - 1)
+        assert ended > 2 * B                                        # restarts were exercised
+        assert not (fused.env_flags().cpu().numpy() & ENV_ERR_MASK).any()
 
 
 def test_ia_step_host_matches_device_step():
-    from dcmrta_b200 import BatchedTaskEnv
-    B, A, T = 1003, 20, 50
-    dev = BatchedTaskEnv(B, A, T, auto_reset=True, seed=23, first_gid=3, protocol="IA")
-    host = BatchedTaskEnv(B, A, T, auto_reset=True, seed=23, first_gid=3, protocol="IA")
-    for e in (dev, host):
-        e.generate(max_duration=5.0)
-        e.reset()
-    out = {"next_leader": np.empty(B, np.int32), "reward": np.empty(B, np.float32), "done": np.empty(B, np.uint8),
-           "agent_obs": np.empty((B, A, 6), np.float32), "task_obs": np.empty((B, T + 1, 5), np.float32), "mask": np.empty((B, T + 1), np.uint8)}
-    restarts = 0
-    for k in range(450):
-        dev.step(policy="random")
-        host.step_host(np.ascontiguousarray(dev.used_action.cpu().numpy().astype(np.int32)), out)
-        assert np.array_equal(out["next_leader"], dev.leader.cpu().numpy()), k
-        assert np.array_equal(out["reward"], dev.reward.cpu().numpy()), k
-        assert np.array_equal(out["done"], dev.done_u8.cpu().numpy()), k
-        assert np.array_equal(out["agent_obs"], dev.agent_obs.cpu().numpy()), k
-        assert np.array_equal(out["task_obs"], dev.task_obs.cpu().numpy()), k
-        assert np.array_equal(out["mask"], dev.mask_u8.cpu().numpy()), k
-        restarts += int(out["done"].sum())
-        assert (out["next_leader"][out["done"] > 0] == 0).all(), k             # a restarted IA episode starts with agent 0
-    assert restarts > B
-    assert np.array_equal(dev.export_raw(), host.export_raw())
-    dev.close(); host.close()
+    shape = EnvelopeShape(20, 50, 5, 1003, "random", None, 450, "", [])
+
+    def restarts_with_agent_0(k, out):                              # a restarted IA episode starts with agent 0
+        assert (out["next_leader"][out["done"] > 0] == 0).all(), k
+
+    with twin_handles(lambda: make_env(shape, "IA", seed=23, first_gid=3)) as (dev, host):
+        assert step_host_equals_step(dev, host, shape.ia_steps, after_step=restarts_with_agent_0) > shape.B
 
 
 def test_ia_shard_invariance():
-    from dcmrta_b200 import BatchedTaskEnv
-    A, T = 20, 50
-    big = BatchedTaskEnv(64, A, T, auto_reset=True, seed=7, first_gid=0, protocol="IA")
-    small = BatchedTaskEnv(16, A, T, auto_reset=True, seed=7, first_gid=32, protocol="IA")
-    for e in (big, small):
-        e.generate()
-        e.reset()
-    for _ in range(300):
-        big.step(policy="random")
-        small.step(policy="random")
-    assert np.array_equal(big.export_raw()[32:48], small.export_raw())
-    assert np.array_equal(big.task_obs[32:48].cpu().numpy(), small.task_obs.cpu().numpy())
-    big.close(); small.close()
+    check_shard_invariance("IA", 300)
 
 
 def test_ia_contract_bits():
@@ -241,29 +145,29 @@ def test_ia_contract_bits():
     inst = pickle_instances()
     insts = [inst[0], inst[1], inst[2]]
     env = BatchedTaskEnv(3, 20, 50, M=5, protocol="IA")
-    env.load_instances(*stack(insts))
+    env.load_instances(*stack_instances(insts))
     env.reset(leaders=np.array([0, 4, -1], np.int32))
     flags = env.env_flags().cpu().numpy()
-    assert not flags[0] & 128 and flags[1] & 128 and not flags[2] & 128
+    assert not flags[0] & ENV_ERR_LEADER and flags[1] & ENV_ERR_LEADER and not flags[2] & ENV_ERR_LEADER
     assert env.leader.cpu().numpy().tolist() == [0, 0, 0]
     env.reset()
     fol = np.full((3, 4), -1, np.int32)
     fol[0, 0] = 1                                                        # env 0: a follower under IA
     env.step(np.array([1, 1, 1], np.int32), fol, np.array([-1, 2, 1], np.int32))
     flags = env.env_flags().cpu().numpy()
-    assert flags[0] & 64 and not flags[1] & 64 and not flags[2] & 64
+    assert flags[0] & ENV_ERR_FOLLOW and not flags[1] & ENV_ERR_FOLLOW and not flags[2] & ENV_ERR_FOLLOW
     assert int(env.used_action[0]) == -1 and env.export_state([0])[0]["has_route"].sum() == 0     # env 0 did not step
-    assert flags[1] & 128 and not flags[2] & 128                         # agent 1 acts next, not agent 2
+    assert flags[1] & ENV_ERR_LEADER and not flags[2] & ENV_ERR_LEADER                         # agent 1 acts next, not agent 2
     assert env.leader.cpu().numpy()[1:].tolist() == [1, 1]
     env.close()
 
     lf = BatchedTaskEnv(2, 20, 50, M=5, seed=3)
-    lf.load_instances(*stack(insts[:2]))
+    lf.load_instances(*stack_instances(insts[:2]))
     lf.reset()
     raw = lf.export_raw()
     assert all(bin(s["group"]).count("1") == 20 for s in lf.export_state())
     ia = BatchedTaskEnv(2, 20, 50, M=5, protocol="IA")
-    ia.load_instances(*stack(insts[:2]))
+    ia.load_instances(*stack_instances(insts[:2]))
     ia.import_raw(raw)
     leader = lf.leader.cpu().numpy()
     ia.step(np.array([1, 0], np.int32))                                  # env 0: a task of requirement > 1; env 1: the depot (Q11 in LF)
@@ -274,7 +178,7 @@ def test_ia_contract_bits():
     assert ia.leader.cpu().numpy().tolist() == [0 if leader[0] else 1, 0 if leader[1] else 1]
     d = np.hypot(*(insts[0]["task_xy"][0] - insts[0]["depot_xy"]))
     assert float(ia.reward[0]) == pytest.approx(-d / 0.2, rel=1e-6) and float(ia.reward[1]) == 0.0
-    assert not (ia.env_flags().cpu().numpy() & ERR_BITS).any()
+    assert not (ia.env_flags().cpu().numpy() & ENV_ERR_MASK).any()
     lf.step(np.array([1, 0], np.int32))                                  # the same records under LF move a coalition / the whole group
     assert [s["has_route"].sum() for s in lf.export_state()] == [int(insts[0]["req"][0]), 20]
     lf.close(); ia.close()

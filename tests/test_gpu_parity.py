@@ -4,28 +4,22 @@
     synthetic instances at the bench's full batch size).
 Bar (BASELINE.json north_star): discrete state bit-exact; times/distances/rewards within 1e-5 relative.  The fp64 event
 clock makes the float state bit-exact too, so the digests are compared exactly; REL documents the contractual tolerance."""
+from contextlib import closing
+
 import numpy as np
 import pytest
 
+from dcmrta_b200._lib import ENV_DONE, ENV_ERR_MASK, ENV_FINISHED, ENV_STUCK
 from oracle import canon
 from oracle.oracle import OracleEnv
 
-from helpers import METRIC_KEYS, ctasd, pickle_instances, pickle_traces, quirk_instance, quirk_traces, sweep_instance, sweep_traces
+from gpu_env import (assert_same_outputs, assert_same_records, check_shard_invariance, instances, lockstep, make_env, stack_instances,
+                     step_host_equals_step, twin_handles, twin_steps)
+from helpers import (METRIC_KEYS, EnvelopeShape, ctasd, pickle_instances, pickle_traces, quirk_instance, quirk_traces, sweep_instance,
+                     sweep_traces)
 
 pytestmark = pytest.mark.gpu
 REL = 1e-5
-
-
-def gpu_state(env, b, inst):
-    """decode env b and add the derived time_finish (= fl(time_start + time) once feasible, task_env.py:257)."""
-    s = env.export_state([b])[0]
-    s["time_finish"] = np.where(s["feasible"] > 0, s["time_start"] + np.asarray(inst["dur"], np.float64), 0.0)
-    return s
-
-
-def stack_instances(insts):
-    return (np.stack([i["task_xy"] for i in insts]), np.stack([i["depot_xy"] for i in insts]),
-            np.stack([i["req"] for i in insts]).astype(np.int32), np.stack([i["dur"] for i in insts]))
 
 
 def replay_batch(insts, eps, tr, max_wait=10.0):
@@ -56,12 +50,11 @@ def replay_batch(insts, eps, tr, max_wait=10.0):
         states = env.export_state()
         for b in range(B):
             if k >= n[b]:
-                assert states[b]["flags"] & 1, f"env {b} should be done after {n[b]} decisions"
+                assert states[b]["flags"] & ENV_DONE, f"env {b} should be done after {n[b]} decisions"
                 continue
             e = eps[b]
             assert leaders[b] == e["leader"][k]
             st = states[b]
-            st["time_finish"] = np.where(st["feasible"] > 0, st["time_start"] + insts[b]["dur"], 0.0)
             assert st["now"] == e["now"][k], (e["name"], k)
             if canon.obs_digest(mk[b], ag[b], tk[b]) != int(e["dig_obs"][k]):
                 o = oracle_at(b, k)
@@ -91,7 +84,7 @@ def replay_batch(insts, eps, tr, max_wait=10.0):
                 assert rew[b] == np.float32(eps[b]["reward"][k]), (eps[b]["name"], k)
                 assert bool(done[b]) == (k == n[b] - 1), (eps[b]["name"], k)
     flags = env.env_flags().cpu().numpy()
-    assert not (flags & 0xF0).any(), "contract-violation bits set during a legal replay"
+    assert not (flags & ENV_ERR_MASK).any(), "contract-violation bits set during a legal replay"
     met = env.episode_metrics().cpu().numpy()
     states = env.export_state()
     for b in range(B):
@@ -99,9 +92,7 @@ def replay_batch(insts, eps, tr, max_wait=10.0):
         np.testing.assert_allclose(met[b], gold, rtol=1e-12, atol=0, err_msg=eps[b]["name"])
         for c in (0, 1, 2, 3, 5, 6, 7):                      # everything but waiting_time is bit-exact
             assert met[b, c] == gold[c], (eps[b]["name"], METRIC_KEYS[c])
-        st = states[b]
-        st["time_finish"] = np.where(st["feasible"] > 0, st["time_start"] + insts[b]["dur"], 0.0)
-        assert canon.state_digest(st) == eps[b]["final_digest"], eps[b]["name"]
+        assert canon.state_digest(states[b]) == eps[b]["final_digest"], eps[b]["name"]
     env.close()
     return met
 
@@ -146,7 +137,7 @@ def test_replay_quirk_fixtures():
     fol = np.full((1, 8), -1, np.int32); f = tr.followers(ep, 0); fol[0, :len(f)] = f
     env.step(np.array([int(ep["action"][0])], np.int32), fol, np.array([-1], np.int32))
     flags = int(env.env_flags()[0])
-    assert flags & 1 and flags & 4 and not flags & 2          # DONE | STUCK, not FINISHED
+    assert flags & ENV_DONE and flags & ENV_STUCK and not flags & ENV_FINISHED
     env.close()
 
 
@@ -171,7 +162,7 @@ def test_ctasd_routes_known_answer():
     env.set_params(max_wait=100.0)                   # execute_by_route leaves max_waiting_time = 100 (task_env.py:564)
     met = env.compute_metrics().cpu().numpy()
     flags = env.env_flags().cpu().numpy()
-    assert not (flags & 0xF0).any()
+    assert not (flags & ENV_ERR_MASK).any()
     states = env.export_state()
     for b, g in enumerate(gold):
         for k, v in g["csv"].items():
@@ -180,9 +171,7 @@ def test_ctasd_routes_known_answer():
             assert met[b, METRIC_KEYS.index(k)] == g["ref_here"][k], (b, k)
         assert met[b, 4] == pytest.approx(g["ref_here"]["waiting_time"], rel=1e-13)
         assert states[b]["finished"].tolist() == g["finished"]
-        st = states[b]
-        st["time_finish"] = np.where(st["feasible"] > 0, st["time_start"] + inst[b]["dur"], 0.0)
-        assert str(canon.state_digest(st)) == g["final_digest"], b
+        assert str(canon.state_digest(states[b])) == g["final_digest"], b
     env.close()
 
 
@@ -190,270 +179,110 @@ def test_ctasd_routes_known_answer():
 def test_inkernel_policy_matches_oracle_on_synthetic(policy):
     """In-kernel Philox policies + generator vs the oracle running the same RNG contract, synthetic 20A/50T instances,
     auto-reset across several episodes; sample of envs out of a batch that is not a multiple of the CTA size."""
-    from dcmrta_b200 import BatchedTaskEnv
-    B, A, T, STEPS = 1003, 20, 50, 400
-    env = BatchedTaskEnv(B, A, T, M=5, auto_reset=True, seed=1234, first_gid=10_000)
-    env.generate(max_duration=5.0, random_duration=(policy == "greedy"))
-    inst = {k: v.cpu().numpy() for k, v in env.get_instances().items()}
-    env.reset()
-    sample = [0, 1, 2, 3, 4, 500, 1001, 1002]
-    orcs = []
-    for b in sample:
-        o = OracleEnv.make(A, inst["task_xy"][b], inst["depot_xy"][b], inst["req"][b], inst["dur"][b])
-        o.seed(1234, gid=10_000 + b, episode=0)
-        assert o.fused_reset() == int(env.leader[b])
-        orcs.append(o)
-    episodes = [0] * len(sample)
-    last_metrics = [None] * len(sample)
-    for k in range(STEPS):
-        ag, tk, mk = env.agent_obs[sample].cpu().numpy(), env.task_obs[sample].cpu().numpy(), env.mask_u8[sample].cpu().numpy()
-        for q, o in enumerate(orcs):
-            l = o.leader
-            assert np.array_equal(mk[q], o.mask()), (policy, sample[q], k)
-            assert np.array_equal(ag[q], o.agent_status(l).astype(np.float32)), (policy, sample[q], k)
-            assert np.array_equal(tk[q], o.task_status(l).astype(np.float32)), (policy, sample[q], k)
-        env.step(policy=policy)
-        rew, done, lead = env.reward[sample].cpu().numpy(), env.done_u8[sample].cpu().numpy(), env.leader[sample].cpu().numpy()
-        for q, o in enumerate(orcs):
-            rc, r, d, _, _ = o.fused_step(-1 if policy == "random" else -2)
-            assert rc == 0
-            assert rew[q] == np.float32(r)
-            assert bool(done[q]) == d, (policy, sample[q], k)
-            if d:
-                last_metrics[q] = o.episode_metrics()[0]
-                episodes[q] += 1
-                o.seed(1234, gid=10_000 + sample[q], episode=episodes[q])
-                o.fused_reset()
-            assert lead[q] == o.leader, (policy, sample[q], k)
-    assert min(episodes) >= 2
-    assert env.total_episodes() >= sum(episodes)                     # dcm_total_episodes: every accounted episode of the batch (bench.py's phase report)
-    met = env.episode_metrics()[sample].cpu().numpy()
-    for q in range(len(sample)):
-        gold = np.array([last_metrics[q][key] for key in METRIC_KEYS])
-        np.testing.assert_allclose(met[q], gold, rtol=1e-12, atol=0)
-    states = env.export_state(sample)
-    for q, o in enumerate(orcs):
-        st = states[q]
-        st["time_finish"] = np.where(st["feasible"] > 0, st["time_start"] + inst["dur"][sample[q]], 0.0)
-        assert not canon.diff_states(st, o.export(canon.MC_CANON)), (policy, sample[q])
-    assert env.total_steps() == B * STEPS
-    env.close()
+    shape = EnvelopeShape(20, 50, 5, 1003, policy, 400, None, "", [])
+    with closing(make_env(shape, seed=1234, first_gid=10_000)) as env:
+        env.reset()
+        orcs = lockstep(env, shape, [0, 1, 2, 3, 4, 500, 1001, 1002], shape.steps, seed=1234, first_gid=10_000)
+        assert env.total_episodes() >= sum(o.episodes for o in orcs)     # dcm_total_episodes: every accounted episode of the batch (bench.py's phase report)
 
 
 def test_shard_invariance():
-    """SURVEY 8(e): the trajectory of global env k does not depend on the batch it lives in."""
-    from dcmrta_b200 import BatchedTaskEnv
-    A, T = 20, 50
-    big = BatchedTaskEnv(64, A, T, auto_reset=True, seed=7, first_gid=0)
-    big.generate()
-    big.reset()
-    small = BatchedTaskEnv(16, A, T, auto_reset=True, seed=7, first_gid=32)
-    small.generate()
-    small.reset()
-    for _ in range(200):
-        big.step(policy="random")
-        small.step(policy="random")
-    a, b = big.export_raw()[32:48], small.export_raw()
-    assert np.array_equal(a, b)
-    assert np.array_equal(big.task_obs[32:48].cpu().numpy(), small.task_obs.cpu().numpy())
-    big.close(); small.close()
+    """SURVEY 8(e): the trajectory of global env k does not depend on the batch it lives in (leader-follower, 200 decisions)."""
+    check_shard_invariance("LF", 200)
 
 
 @pytest.mark.parametrize("variant", ["DCM_PASS_SERIAL"])
 @pytest.mark.parametrize("shape,policy", [((20, 50), "random"), ((20, 50), "greedy"), ((10, 20), "random"), ((50, 200), "random"), ((30, 100), "greedy")])
-def test_fused_pass_equals_split_kernels(shape, policy, variant, monkeypatch):
+def test_fused_pass_equals_split_kernels(shape, policy, variant):
     """The default pass (k_step, then k_episode on a side stream writing the restarted envs' observations from registers
     beside k_obs) against the three kernels one after the other with k_obs building every observation from memory: raw records (every field, bookkeeping bits included), observations, rewards, leaders and metrics identical on a batch
     that is not a multiple of the tile size."""
-    from dcmrta_b200 import BatchedTaskEnv
-    A, T = shape
     B = 4099
-    fused = BatchedTaskEnv(B, A, T, auto_reset=True, seed=11, first_gid=5)
-    monkeypatch.setenv(variant, "1")
-    other = BatchedTaskEnv(B, A, T, auto_reset=True, seed=11, first_gid=5)
-    monkeypatch.delenv(variant)
-    for e in (fused, other):
-        e.generate(max_duration=5.0, random_duration=(policy == "greedy"))
-        e.reset()
-    assert fused.launch_count() == other.launch_count()
-    keys = [k for k in fused.export_state([0])[0].keys()]
-    for k in range(600):
-        fused.step(policy=policy)
-        other.step(policy=policy)
-        if k % 50 == 49 or k < 3:
-            assert np.array_equal(fused.reward.cpu().numpy(), other.reward.cpu().numpy()), k
-            assert np.array_equal(fused.leader.cpu().numpy(), other.leader.cpu().numpy()), k
-            assert np.array_equal(fused.done_u8.cpu().numpy(), other.done_u8.cpu().numpy()), k
-            assert np.array_equal(fused.used_action.cpu().numpy(), other.used_action.cpu().numpy()), k
-            assert np.array_equal(fused.agent_obs.cpu().numpy(), other.agent_obs.cpu().numpy()), k
-            assert np.array_equal(fused.task_obs.cpu().numpy(), other.task_obs.cpu().numpy()), k
-            assert np.array_equal(fused.mask_u8.cpu().numpy(), other.mask_u8.cpu().numpy()), k
-            a, b = fused.export_raw(), other.export_raw()
-            if not np.array_equal(a, b):
-                bad = int(np.argwhere((a != b).any(1))[0, 0])
-                sa, sb = fused.export_state([bad])[0], other.export_state([bad])[0]
-                diff = [key for key in keys if not np.array_equal(np.asarray(sa[key]), np.asarray(sb[key]), equal_nan=True)]
-                raise AssertionError(f"decision {k}: env {bad} differs in {diff}")
-    ma, mb = fused.episode_metrics().cpu().numpy(), other.episode_metrics().cpu().numpy()
-    assert np.array_equal(ma, mb)
-    assert fused.total_steps() == other.total_steps() == B * 600
-    fused.close(); other.close()
+    sh = EnvelopeShape(*shape, 5, B, policy, 600, None, "", [])
+    with twin_handles(lambda: make_env(sh, seed=11, first_gid=5), variant) as (fused, other):
+        assert fused.launch_count() == other.launch_count()
+        twin_steps(fused, other, policy, sh.steps, lambda k: k % 50 == 49 or k < 3)
+        assert fused.total_steps() == other.total_steps() == B * sh.steps
 
 
 @pytest.mark.parametrize("variant", [None, "DCM_OBS_RESET_BY_EPISODE", "DCM_OBS_CHUNKED"])
-def test_step_host_matches_device_step(variant, monkeypatch):
+def test_step_host_matches_device_step(variant):
     """dcm_step_host (host buffers; next_leader / reward / done leave for the host when k_step ends, beside the episode and
     observation kernels) against dcm_step with device buffers replaying the same actions: every output of every decision,
     restarts included (the first leader and the first observation of a restarted episode come from k_step / k_obs_tile in the
-    default pass and from the episode kernel in the variants)."""
-    from dcmrta_b200 import BatchedTaskEnv
-    B, A, T = 1003, 20, 50
-    dev = BatchedTaskEnv(B, A, T, auto_reset=True, seed=21, first_gid=3)
-    dev.generate(max_duration=5.0)
-    dev.reset()
-    if variant:                                                                # read when the handle launches its first observation kernel
-        monkeypatch.setenv(variant, "1")
-    host = BatchedTaskEnv(B, A, T, auto_reset=True, seed=21, first_gid=3)
-    host.generate(max_duration=5.0)
-    host.reset()
-    if variant:
-        monkeypatch.delenv(variant)
-    out = {"next_leader": np.empty(B, np.int32), "reward": np.empty(B, np.float32), "done": np.empty(B, np.uint8),
-           "agent_obs": np.empty((B, A, 6), np.float32), "task_obs": np.empty((B, T + 1, 5), np.float32), "mask": np.empty((B, T + 1), np.uint8)}
-    restarts = 0
-    import torch
-    pinned = torch.empty(B, dtype=torch.int32).pin_memory()
-    for k in range(450):
-        dev.step(policy="random")
-        acts = np.ascontiguousarray(dev.used_action.cpu().numpy().astype(np.int32))
-        if k % 2:                                                              # pinned buffer: the step kernel reads the actions in place; pageable: staged copy
-            import torch
-            pinned[:] = torch.from_numpy(acts)
-            host.step_host(pinned, out)
-        else:
-            host.step_host(acts, out)
-        assert np.array_equal(out["next_leader"], dev.leader.cpu().numpy()), k
-        assert np.array_equal(out["reward"], dev.reward.cpu().numpy()), k
-        assert np.array_equal(out["done"], dev.done_u8.cpu().numpy()), k
-        assert np.array_equal(out["agent_obs"], dev.agent_obs.cpu().numpy()), k
-        assert np.array_equal(out["task_obs"], dev.task_obs.cpu().numpy()), k
-        assert np.array_equal(out["mask"], dev.mask_u8.cpu().numpy()), k
-        restarts += int(out["done"].sum())
-        assert (out["next_leader"] >= 0).all(), k                              # auto-reset: every env has a leader after every decision
-    assert restarts > B                                                        # the restart path was exercised
-    assert np.array_equal(dev.export_raw(), host.export_raw())
-    dev.close(); host.close()
+    default pass and from the episode kernel in the variants, which the host-buffer handle is created with)."""
+    shape = EnvelopeShape(20, 50, 5, 1003, "random", 450, None, "", [])
+
+    def every_env_has_a_leader(k, out):                                          # auto-reset: after every decision
+        assert (out["next_leader"] >= 0).all(), k
+
+    with twin_handles(lambda: make_env(shape, seed=21, first_gid=3), variant) as (dev, host):
+        restarts = step_host_equals_step(dev, host, shape.steps, pinned=True, after_step=every_env_has_a_leader)
+        assert restarts > shape.B                                                # the restart path was exercised
 
 
-def test_regenerate_restarts_on_fresh_instances(monkeypatch):
+def test_regenerate_restarts_on_fresh_instances():
     """DCM_FLAG_REGENERATE: an env whose episode ended restarts on a NEW instance drawn in the episode kernel's registers (same
     Philox streams as dcm_generate, instance counter + 1), and that kernel writes the first observation of the new episode
     beside k_obs_tile.  Checked against (a) the serial pass, where k_obs builds that observation from memory after the
     restart, and (b) the closed form of a reset observation on the instance read back from the device."""
     from dcmrta_b200 import BatchedTaskEnv
     B, A, T = 1003, 20, 50
-    env = BatchedTaskEnv(B, A, T, auto_reset=True, regenerate=True, seed=31, first_gid=9)
-    monkeypatch.setenv("DCM_PASS_SERIAL", "1")
-    ser = BatchedTaskEnv(B, A, T, auto_reset=True, regenerate=True, seed=31, first_gid=9)
-    monkeypatch.delenv("DCM_PASS_SERIAL")
-    for e in (env, ser):
+
+    def make():
+        e = BatchedTaskEnv(B, A, T, auto_reset=True, regenerate=True, seed=31, first_gid=9)
         e.generate(max_duration=5.0)
-        e.reset()
-    first = {k: v.cpu().numpy().copy() for k, v in env.get_instances().items()}
-    restarted = np.zeros(B, bool)
-    for k in range(450):
-        env.step(policy="random")
-        ser.step(policy="random")
-        done = env.done_u8.cpu().numpy().astype(bool)
-        assert np.array_equal(done, ser.done_u8.cpu().numpy().astype(bool)), k
-        assert np.array_equal(env.leader.cpu().numpy(), ser.leader.cpu().numpy()), k
-        assert np.array_equal(env.reward.cpu().numpy(), ser.reward.cpu().numpy()), k
-        ag, tk, mk = env.agent_obs.cpu().numpy(), env.task_obs.cpu().numpy(), env.mask_u8.cpu().numpy()
-        assert np.array_equal(ag, ser.agent_obs.cpu().numpy()), k
-        assert np.array_equal(tk, ser.task_obs.cpu().numpy()), k
-        assert np.array_equal(mk, ser.mask_u8.cpu().numpy()), k
-        if done.any():
-            inst = {kk: v.cpu().numpy() for kk, v in env.get_instances().items()}
-            for b in np.flatnonzero(done)[:8]:
+        return e
+
+    with twin_handles(make, "DCM_PASS_SERIAL") as (env, ser):
+        first_xy = stack_instances(instances(env))[0]
+        restarted = np.zeros(B, bool)
+
+        def reset_observations(k):
+            done = env.done_u8.cpu().numpy().astype(bool)
+            ag, tk, mk = env.agent_obs.cpu().numpy(), env.task_obs.cpu().numpy(), env.mask_u8.cpu().numpy()
+            ended = np.flatnonzero(done)[:8]
+            for b, inst in zip(ended, instances(env, ended)):
                 assert not ag[b].any(), (k, b)                                         # nobody has a route (:165-180)
                 want = np.zeros((T + 1, 5), np.float32)
-                want[1:, 0] = inst["req"][b]; want[1:, 1] = inst["req"][b]; want[1:, 2] = inst["dur"][b].astype(np.float32)
-                want[1:, 3:] = (inst["task_xy"][b] - inst["depot_xy"][b]).astype(np.float32)
+                want[1:, 0] = inst["req"]; want[1:, 1] = inst["req"]; want[1:, 2] = inst["dur"].astype(np.float32)
+                want[1:, 3:] = (inst["task_xy"] - inst["depot_xy"]).astype(np.float32)
                 assert np.array_equal(tk[b], want), (k, b)                              # :182-190 seen from the depot
                 assert mk[b, 0] == 1 and not mk[b, 1:].any(), (k, b)                    # only the depot is masked
-            restarted |= done
-    assert restarted.sum() > B // 2
-    last = {k: v.cpu().numpy() for k, v in env.get_instances().items()}
-    moved = (last["task_xy"] != first["task_xy"]).any(axis=(1, 2))
-    assert np.array_equal(moved, restarted)                                             # new instances exactly where an episode ended
-    assert (last["task_xy"] >= 0).all() and (last["task_xy"] < 1).all() and (last["depot_xy"] >= 0).all() and (last["depot_xy"] < 1).all()
-    assert last["req"].min() >= 1 and last["req"].max() <= 5 and (last["dur"] == 5.0).all()
-    assert np.array_equal(env.export_raw(), ser.export_raw())
-    env.close(); ser.close()
+            restarted[done] = True
+
+        twin_steps(env, ser, "random", 450, lambda k: True, after_step=reset_observations)
+        assert restarted.sum() > B // 2
+        xy, depot, req, dur = stack_instances(instances(env))
+        moved = (xy != first_xy).any(axis=(1, 2))
+        assert np.array_equal(moved, restarted)                                         # new instances exactly where an episode ended
+        assert (xy >= 0).all() and (xy < 1).all() and (depot >= 0).all() and (depot < 1).all()
+        assert req.min() >= 1 and req.max() <= 5 and (dur == 5.0).all()
 
 
-def test_bench_configuration_at_its_own_size(monkeypatch):
+def test_bench_configuration_at_its_own_size():
     """The configuration the headline number is measured on (BASELINE configs[2]: 65,536 synthetic 20A/50T envs, in-kernel random
     policy, auto-reset) checked AT THAT SIZE through its steady state (k_step appends ~450 ended envs per pass to the episode list,
     2,048 observation blocks share the SMs with the episode blocks):
       * 64 random envs against the oracle at every one of 340 decisions -- observations, mask, reward, done, next leader;
       * the default pass against the serial pass (DCM_PASS_SERIAL: k_step, k_episode_list, k_obs one after the other on one
         stream, observations always built from memory) on every output at checkpoints and on the raw records of all envs."""
-    from dcmrta_b200 import BatchedTaskEnv
-    B, A, T, STEPS = 65536, 20, 50, 340
-    env = BatchedTaskEnv(B, A, T, M=5, auto_reset=True, seed=1234, first_gid=0)
-    monkeypatch.setenv("DCM_PASS_SERIAL", "1")
-    ser = BatchedTaskEnv(B, A, T, M=5, auto_reset=True, seed=1234, first_gid=0)
-    monkeypatch.delenv("DCM_PASS_SERIAL")
-    for e in (env, ser):
-        e.generate(max_duration=5.0)
-        e.reset()
+    import torch
+    shape = EnvelopeShape(20, 50, 5, 65536, "random", 340, None, "", [])
+    B, STEPS = shape.B, shape.steps
     rng = np.random.default_rng(5)
     sample = sorted(int(x) for x in rng.choice(B, 64, replace=False))
     sample[0], sample[-1] = 0, B - 1
-    import torch
-    sidx = torch.as_tensor(sample, device=env.device)
-    inst = {k: v[sidx].cpu().numpy() for k, v in env.get_instances().items()}
-    orcs = []
-    for q, b in enumerate(sample):
-        o = OracleEnv.make(A, inst["task_xy"][q], inst["depot_xy"][q], inst["req"][q], inst["dur"][q])
-        o.seed(1234, gid=b, episode=0)
-        assert o.fused_reset() == int(env.leader[b])
-        orcs.append(o)
-    episodes = [0] * len(sample)
-    ended_total = 0
-    for k in range(STEPS):
-        ag, tk, mk = env.agent_obs[sidx].cpu().numpy(), env.task_obs[sidx].cpu().numpy(), env.mask_u8[sidx].cpu().numpy()
-        for q, o in enumerate(orcs):
-            l = o.leader
-            assert np.array_equal(mk[q], o.mask()), (sample[q], k)
-            assert np.array_equal(ag[q], o.agent_status(l).astype(np.float32)), (sample[q], k)
-            assert np.array_equal(tk[q], o.task_status(l).astype(np.float32)), (sample[q], k)
-        env.step(policy="random")
-        ser.step(policy="random")
-        rew, done, lead = env.reward[sidx].cpu().numpy(), env.done_u8[sidx].cpu().numpy(), env.leader[sidx].cpu().numpy()
-        for q, o in enumerate(orcs):
-            rc, r, d, _, _ = o.fused_step(-1)
-            assert rc == 0 and rew[q] == np.float32(r) and bool(done[q]) == d, (sample[q], k)
-            if d:
-                episodes[q] += 1
-                o.seed(1234, gid=sample[q], episode=episodes[q])
-                o.fused_reset()
-            assert lead[q] == o.leader, (sample[q], k)
-        if k % 20 == 19 or k >= STEPS - 3:
-            ended_total += int(env.done_u8.sum())
-            for name in ("reward", "leader", "done_u8", "used_action", "agent_obs", "task_obs", "mask_u8"):
-                assert torch.equal(getattr(env, name), getattr(ser, name)), (name, k)
-    assert min(episodes) >= 1 and ended_total > 20 * 100            # the steady state was reached: hundreds of episode ends per pass
-    a, b = env.export_raw(), ser.export_raw()
-    if not np.array_equal(a, b):
-        bad = np.flatnonzero((a != b).any(1))
-        raise AssertionError(f"{len(bad)} envs differ between the default and the serial pass, first: {bad[:8]}")
-    assert torch.equal(env.episode_metrics(), ser.episode_metrics())
-    states = env.export_state(sample)
-    for q, o in enumerate(orcs):
-        st = states[q]
-        st["time_finish"] = np.where(st["feasible"] > 0, st["time_start"] + inst["dur"][q], 0.0)
-        assert not canon.diff_states(st, o.export(canon.MC_CANON)), sample[q]
-    assert env.total_steps() == B * STEPS
-    env.close(); ser.close()
+    with twin_handles(lambda: make_env(shape, seed=1234, first_gid=0), "DCM_PASS_SERIAL") as (env, ser):
+        ended = []
+
+        def serial_pass(k):
+            ser.step(policy="random")
+            if k % 20 == 19 or k >= STEPS - 3:
+                ended.append(int(env.done_u8.sum()))
+                assert_same_outputs(env, ser, k)
+
+        lockstep(env, shape, sample, STEPS, seed=1234, first_gid=0, min_episodes=1, metrics=False, after_step=serial_pass)
+        assert sum(ended) > 20 * 100                                # the steady state was reached: hundreds of episode ends per pass
+        assert_same_records(env, ser, "default against serial pass")
+        assert torch.equal(env.episode_metrics(), ser.episode_metrics())

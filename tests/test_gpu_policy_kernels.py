@@ -342,7 +342,7 @@ def _peaked(net, gain=3.0):
 @pytest.mark.parametrize("name", ["1A_1T_1M_B33_random", "20A_50T", "64A_254T_8M_B100_random"])
 def test_every_kernel_call_of_a_forward(name, peaked):
     from dcmrta_b200.policy_fused import FusedPolicy
-    from test_gpu_shape_envelope import make_env
+    from gpu_env import make_env
     from test_policy_fused import _net
     shape = EnvelopeShape(20, 50, 5, 64, "random", 0, None, "", []) if name == "20A_50T" else envelope_shape(name)
     env = make_env(shape)

@@ -9,14 +9,14 @@ import ctypes as C
 import numpy as np
 import pytest
 
+from dcmrta_b200._lib import ENV_DONE, ENV_ERR_ACTION, ENV_ERR_MASK, ENV_ERR_OVERFLOW, ENV_FINISHED, ENV_STUCK
 from oracle import canon
 
+from gpu_env import instances
 from helpers import (ENVELOPE_SHAPES, METRIC_KEYS, ROUTE_MAX_DURATION, envelope_shape, make_routes, pack_routes, route_batch_sizes,
                      route_family, route_oracle, route_seed)
 
 pytestmark = pytest.mark.gpu
-ERR_BITS = 0xF0                         # DCM_ENV_ERR_OVERFLOW | _ACTION | _FOLLOW | _LEADER
-ERR_OVERFLOW, ERR_ACTION = 16, 32
 
 
 def route_env(shape, B, protocol="LF", velocity=0.2):
@@ -25,9 +25,8 @@ def route_env(shape, B, protocol="LF", velocity=0.2):
     env = BatchedTaskEnv(B, shape.A, shape.T, M=shape.M, seed=shape.seed, first_gid=shape.first_gid(), protocol=protocol,
                          velocity=velocity)
     env.generate(max_duration=ROUTE_MAX_DURATION, random_duration=shape.random_duration)
-    got = {k: v.cpu().numpy() for k, v in env.get_instances().items()}
     env.reset()
-    return env, [{k: got[k][b] for k in got} for b in range(B)]
+    return env, instances(env)
 
 
 def batch_routes(shape, insts):
@@ -48,15 +47,13 @@ def check_against_oracle(env, insts, makespan, played, envs, velocity=0.2):
         what = (env.A, env.T, env.M, env.B, b)
         o, want_mk = route_oracle(A, insts[b], played[b], velocity)
         assert mk[b] == want_mk, (what, mk[b], want_mk)
-        st = states[q]
-        st["time_finish"] = np.where(st["feasible"] > 0, st["time_start"] + np.asarray(insts[b]["dur"], np.float64), 0.0)
         ref = o.export(canon.MC_CANON)
-        d = canon.diff_states(st, ref)
+        d = canon.diff_states(states[q], ref)
         assert not d, (what, d)
         f = int(flags[b])
-        assert f & 1, (what, f)                                               # DONE, always
-        assert bool(f & 2) == ref["env_finished"], (what, f)
-        assert bool(f & 4) == o.stuck, (what, f)
+        assert f & ENV_DONE, (what, f)                                        # always
+        assert bool(f & ENV_FINISHED) == ref["env_finished"], (what, f)
+        assert bool(f & ENV_STUCK) == o.stuck, (what, f)
         ends.add("finished" if ref["env_finished"] else ("stuck" if o.stuck else "clock_cap"))
         want = o.episode_metrics()[0]
         for c in (0, 1, 2, 3, 5, 6):
@@ -81,7 +78,7 @@ def test_routes_match_oracle(shape, B):
     routes, rlen = pack_routes(R, shape.A)
     mk = env.execute_by_route(routes, rlen)
     flags, ends = check_against_oracle(env, insts, mk, R, list(range(B)))
-    assert not (flags & ERR_BITS).any()
+    assert not (flags & ENV_ERR_MASK).any()
     if B == max(route_batch_sizes(shape)) and shape.M > 1:                 # the batch tests/test_routes_oracle.py takes the census of
         assert {"finished", "stuck", "clock_cap"} <= ends, ends
     env.close()
@@ -113,9 +110,9 @@ def test_route_errors_stay_in_their_env(name):
     ok = [b for b in range(B) if b not in overflow]
     flags, _ = check_against_oracle(env, insts, mk, played, ok)
     for b in range(B):
-        want = ERR_OVERFLOW if b in overflow else (ERR_ACTION if b in bad else 0)
-        assert flags[b] & ERR_BITS == want, (name, b, flags[b])
-        assert flags[b] & 1
+        want = ENV_ERR_OVERFLOW if b in overflow else (ENV_ERR_ACTION if b in bad else 0)
+        assert flags[b] & ENV_ERR_MASK == want, (name, b, flags[b])
+        assert flags[b] & ENV_DONE
     env.close()
 
 
@@ -179,7 +176,7 @@ def test_route_lengths_beyond_the_row_stride():
     flags, _ = check_against_oracle(env, insts, mk, played, list(range(B)))
     long_envs = {b for b, _ in long}
     for b in range(B):
-        assert flags[b] & ERR_BITS == (ERR_ACTION if b in long_envs else 0), (b, flags[b])
+        assert flags[b] & ENV_ERR_MASK == (ENV_ERR_ACTION if b in long_envs else 0), (b, flags[b])
     env.close()
 
 
@@ -190,7 +187,7 @@ def test_routes_at_a_non_default_velocity():
     R = batch_routes(shape, insts)
     mk = env.execute_by_route(*pack_routes(R, shape.A))
     flags, _ = check_against_oracle(env, insts, mk, R, list(range(64)), velocity=0.35)
-    assert not (flags & ERR_BITS).any()
+    assert not (flags & ENV_ERR_MASK).any()
     env.close()
 
 

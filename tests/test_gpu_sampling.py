@@ -6,12 +6,13 @@ import math
 import numpy as np
 import pytest
 
+from dcmrta_b200._lib import ENV_ERR_MASK
+
 from helpers import GOLD, METRIC_KEYS
 from test_sampling_rule import kth_allowed, rule64, sampler_word
 
 pytestmark = pytest.mark.gpu
 NS = (1, 2, 31, 32, 33, 51, 64, 65, 255, 256)
-ERR_BITS = 0xF0
 SENTINEL = 0x5A5A5A5A
 
 
@@ -278,7 +279,7 @@ def play(protocol, B, first_gid, runner, sampler=(31, 0), horizon=600):
                leader=np.where(ep.active[:L].cpu().numpy(), ep.leader[:L].cpu().numpy(), -1),
                metrics=ep.metrics.cpu().numpy(), inst={k: v.cpu().numpy() for k, v in env.get_instances().items()},
                flags=env.env_flags().cpu().numpy())
-    assert not (out["flags"] & ERR_BITS).any()
+    assert not (out["flags"] & ENV_ERR_MASK).any()
     env.close()
     return out
 
@@ -417,7 +418,7 @@ def test_attention_net_samples_legal_actions(amp):
     env.load_instances(sets["task_xy"][inst], sets["depot_xy"][inst], sets["req"][inst], sets["dur"][inst])
     ep = BatchedRollout(env, 560).run(net, "sample", amp=amp, sampler=(2, 0))
     assert bool(ep.ended.all())
-    assert not (env.env_flags().cpu().numpy() & ERR_BITS).any()
+    assert not (env.env_flags().cpu().numpy() & ENV_ERR_MASK).any()
     act, mask, active = ep.action.long(), ep.mask, ep.active
     chosen = mask.gather(2, act.unsqueeze(2)).squeeze(2)
     assert int(chosen[active].sum()) == 0 and int(active.sum()) > 50 * K * 50

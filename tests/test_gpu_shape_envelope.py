@@ -4,39 +4,19 @@ where the kernels change code path: one, two or four 64-bit task-mask words and 
 k_obs, the second 16-entry staging chunk of the step's scans, 8-member coalitions, partial tiles of envs, and metric sums over more than
 248 tasks (NumPy splits those twice).  The shapes, their trajectories' census and the CPU side of the same runs are in tests/helpers.py
 and tests/test_shape_envelope_oracle.py.  The whole file takes about 16 s on one B200."""
+from contextlib import closing
+
 import numpy as np
 import pytest
 
-from oracle import canon
+from dcmrta_b200._lib import ENV_DONE, ENV_ERR_MASK, ENV_FINISHED, ENV_STUCK
 
-from helpers import ENVELOPE_SHAPES, METRIC_KEYS, EnvelopeOracle, device_instance, envelope_shape
+from gpu_env import (assert_metrics_match, assert_same_outputs, assert_same_records, check_obs, instances, lockstep, make_env,
+                     stack_instances, twin_handles, twin_steps)
+from helpers import ENVELOPE_SHAPES, EnvelopeOracle, EnvelopeShape, device_instance, envelope_shape
 
 pytestmark = pytest.mark.gpu
-ERR_BITS = 0xF0                         # DCM_ENV_ERR_OVERFLOW | _ACTION | _FOLLOW | _LEADER
 OBS_TILE_AGENTS = 20
-
-
-def make_env(shape, protocol="LF", auto_reset=True):
-    from dcmrta_b200 import BatchedTaskEnv
-    env = BatchedTaskEnv(shape.B, shape.A, shape.T, M=shape.M, auto_reset=auto_reset, seed=shape.seed, first_gid=shape.first_gid(),
-                         protocol=protocol)
-    env.generate(max_duration=5.0, random_duration=shape.random_duration)
-    return env
-
-
-def sampled_instances(env, sample):
-    return [{k: v[b].cpu().numpy() for k, v in env.get_instances().items()} for b in sample]
-
-
-def with_finish(st, dur):
-    st["time_finish"] = np.where(st["feasible"] > 0, st["time_start"] + np.asarray(dur, np.float64), 0.0)
-    return st
-
-
-def assert_metrics_match(got, want, what):
-    np.testing.assert_allclose(got, want, rtol=1e-12, atol=0, err_msg=str(what))      # waiting_time: the documented order difference
-    for c in (0, 1, 2, 3, 5, 6, 7):
-        assert got[c] == want[c], (what, METRIC_KEYS[c], got[c], want[c])
 
 
 def obs_tile_switch(A=OBS_TILE_AGENTS):
@@ -68,7 +48,7 @@ def test_device_generator_is_the_restated_one():
     trajectories this file checks"""
     for shape in (ENVELOPE_SHAPES[0], envelope_shape("64A_254T_8M_B100_random"), envelope_shape("33A_129T_5M_B100_greedy")):
         env = make_env(shape)
-        for b, got in zip(shape.sample(), sampled_instances(env, shape.sample())):
+        for b, got in zip(shape.sample(), instances(env, shape.sample())):
             want = device_instance(shape.A, shape.T, shape.M, shape.seed, shape.first_gid() + b, random_duration=shape.random_duration)
             for k in ("task_xy", "depot_xy", "req", "dur"):
                 assert np.array_equal(got[k], want[k]), (shape.name, b, k)
@@ -76,121 +56,47 @@ def test_device_generator_is_the_restated_one():
 
 
 def run_lockstep(shape, protocol, steps):
-    """in-kernel policy with auto-reset against the oracle on a sample of the batch, every decision: mask, agent rows, task rows, reward,
-    done, next leader; then the metrics of the last episode, the state and the error bits.  Returns (env, oracles)."""
-    env = make_env(shape, protocol)
-    sample = shape.sample()
-    insts = sampled_instances(env, sample)
-    env.reset()
-    orcs = [EnvelopeOracle(shape, b, inst, protocol) for b, inst in zip(sample, insts)]
-    for q, o in enumerate(orcs):
-        assert o.leader == int(env.leader[sample[q]]), (shape.name, sample[q])
-    for k in range(steps):
-        ag, tk, mk = env.agent_obs[sample].cpu().numpy(), env.task_obs[sample].cpu().numpy(), env.mask_u8[sample].cpu().numpy()
-        for q, o in enumerate(orcs):
-            what = (shape.name, protocol, sample[q], k)
-            assert np.array_equal(mk[q], o.env.mask()), what
-            assert np.array_equal(ag[q], o.env.agent_status(o.leader).astype(np.float32)), what
-            assert np.array_equal(tk[q], o.env.task_status(o.leader).astype(np.float32)), what
-        env.step(policy=shape.policy)
-        rew, done, lead = env.reward[sample].cpu().numpy(), env.done_u8[sample].cpu().numpy(), env.leader[sample].cpu().numpy()
-        for q, o in enumerate(orcs):
-            what = (shape.name, protocol, sample[q], k)
-            r, d, _ = o.step()
-            assert rew[q] == np.float32(r), what
-            assert bool(done[q]) == d, what
-            assert lead[q] == o.leader, what
-    assert min(o.episodes for o in orcs) >= (1 if shape.T > 200 else 2)
-    met = env.episode_metrics()[sample].cpu().numpy()
-    for q, o in enumerate(orcs):
-        assert_metrics_match(met[q], o.last_metrics, (shape.name, protocol, sample[q]))
-    states = env.export_state(sample)
-    for q, o in enumerate(orcs):
-        d = canon.diff_states(with_finish(states[q], insts[q]["dur"]), o.o.export(canon.MC_CANON))
-        assert not d, (shape.name, protocol, sample[q], d)
-    assert not (env.env_flags().cpu().numpy() & ERR_BITS).any()
-    assert env.total_steps() == shape.B * steps
-    return env, orcs
+    """in-kernel policy with auto-reset against the oracle on the shape's sample (gpu_env.lockstep).  -> the oracles"""
+    with closing(make_env(shape, protocol)) as env:
+        env.reset()
+        return lockstep(env, shape, shape.sample(), steps, min_episodes=1 if shape.T > 200 else 2)
 
 
 @pytest.mark.parametrize("shape", ENVELOPE_SHAPES, ids=lambda s: s.name)
 def test_envelope_matches_oracle(shape):
     """leader-follower, and the census events the shape is listed for"""
-    env, orcs = run_lockstep(shape, "LF", shape.steps)
+    orcs = run_lockstep(shape, "LF", shape.steps)
     missing = set(shape.census) - set.union(*(o.census for o in orcs))
     assert not missing, (shape.name, missing)
-    env.close()
 
 
 @pytest.mark.parametrize("shape", [s for s in ENVELOPE_SHAPES if s.ia_steps], ids=lambda s: s.name)
 def test_envelope_ia_matches_oracle(shape):
     """the individual-agent protocol (tests/ia_oracle.py's loop) at the shapes of the table that run it"""
-    run_lockstep(shape, "IA", shape.ia_steps)[0].close()
-
-
-def outputs(env):
-    return {n: getattr(env, n).cpu().numpy() for n in ("reward", "leader", "done_u8", "used_action", "agent_obs", "task_obs", "mask_u8")}
-
-
-def assert_same_records(a, b, what):
-    ra, rb = a.export_raw(), b.export_raw()
-    assert np.array_equal(ra, rb), (what, np.flatnonzero((ra != rb).any(1))[:8])
-
-
-def twin_handles(shape, variant, monkeypatch, B):
-    """two handles on the same instances and draws, the second created with the environment switch `variant` set"""
-    from dcmrta_b200 import BatchedTaskEnv
-    mk = lambda: BatchedTaskEnv(B, shape.A, shape.T, M=shape.M, auto_reset=True, seed=shape.seed, first_gid=shape.first_gid())
-    a = mk()
-    monkeypatch.setenv(variant, "1")
-    b = mk()
-    monkeypatch.delenv(variant)
-    for e in (a, b):
-        e.generate(max_duration=5.0, random_duration=shape.random_duration)
-        e.reset()
-    return a, b
+    run_lockstep(shape, "IA", shape.ia_steps)
 
 
 @pytest.mark.parametrize("which", ["tile_last", "chunked_first", "64A_254T_8M"])
-def test_envelope_default_pass_equals_serial_pass(which, monkeypatch):
+def test_envelope_default_pass_equals_serial_pass(which):
     """the default pass against DCM_PASS_SERIAL (k_step, episode kernel and the chunked k_obs one after the other): every output at
     checkpoints and the raw records of every env, on the last shape k_obs_tile serves at 20 agents, the first it does not, and the
     largest shape"""
-    from helpers import EnvelopeShape
     if which == "64A_254T_8M":
-        shape, B, steps = envelope_shape("64A_254T_8M_B100_random"), 1003, 700
+        shape = EnvelopeShape(64, 254, 8, 1003, "random", 700, None, "", [])      # the table's largest shape at ten times its batch
     else:
-        t = obs_tile_switch() + (which == "chunked_first")
-        shape, B, steps = EnvelopeShape(OBS_TILE_AGENTS, t, 5, 4099, "random", 0, None, "", []), 4099, 500
-    a, b = twin_handles(shape, "DCM_PASS_SERIAL", monkeypatch, B)
-    ended = 0
-    for k in range(steps):
-        a.step(policy=shape.policy)
-        b.step(policy=shape.policy)
-        ended += int(a.done_u8.sum())
-        if k % 50 == 49 or k < 3 or k == steps - 1:
-            oa, ob = outputs(a), outputs(b)
-            for n in oa:
-                assert np.array_equal(oa[n], ob[n]), (which, n, k)
-            assert_same_records(a, b, (which, k))
-    assert ended > B                                                      # restarts were exercised
-    assert np.array_equal(a.episode_metrics().cpu().numpy(), b.episode_metrics().cpu().numpy())
-    assert not (a.env_flags().cpu().numpy() & ERR_BITS).any()
-    a.close(); b.close()
+        shape = EnvelopeShape(OBS_TILE_AGENTS, obs_tile_switch() + (which == "chunked_first"), 5, 4099, "random", 500, None, "", [])
+    with twin_handles(lambda: make_env(shape), "DCM_PASS_SERIAL") as (a, b):
+        ended = twin_steps(a, b, shape.policy, shape.steps, lambda k: k % 50 == 49 or k < 3 or k == shape.steps - 1)
+        assert ended > shape.B                                              # restarts were exercised
+        assert not (a.env_flags().cpu().numpy() & ENV_ERR_MASK).any()
 
 
-def test_step_without_next_decision_scratch_equals_default(monkeypatch):
+def test_step_without_next_decision_scratch_equals_default():
     """24 agents, the largest count whose next_decision rows the step keeps in shared memory: DCM_STEP_NO_NDS=1 (rows from global
     memory) leaves every raw record as the default does"""
-    shape = envelope_shape("24A_64T_8M_B100_random")
-    a, b = twin_handles(shape, "DCM_STEP_NO_NDS", monkeypatch, 1003)
-    for k in range(400):
-        a.step(policy=shape.policy)
-        b.step(policy=shape.policy)
-        if k % 100 == 99:
-            assert_same_records(a, b, k)
-            assert np.array_equal(a.agent_obs.cpu().numpy(), b.agent_obs.cpu().numpy()), k
-    a.close(); b.close()
+    shape = EnvelopeShape(24, 64, 8, 1003, "random", 400, None, "", [])        # the table's 24-agent shape at ten times its batch
+    with twin_handles(lambda: make_env(shape), "DCM_STEP_NO_NDS") as (a, b):
+        twin_steps(a, b, shape.policy, shape.steps, lambda k: k % 100 == 99)
 
 
 @pytest.mark.parametrize("name", ["2A_3T_3M_B100_random", "7A_63T_2M_B100_greedy", "64A_249T_3M_B100_greedy", "64A_254T_8M_B100_random"])
@@ -204,9 +110,8 @@ def test_envelope_granular_path(name):
     shape = envelope_shape(name)
     env = make_env(shape, auto_reset=False)
     sample = shape.sample()
-    insts = sampled_instances(env, sample)
+    orcs = [EnvelopeOracle(shape, b, inst) for b, inst in zip(sample, instances(env, sample))]
     env.reset()
-    orcs = [EnvelopeOracle(shape, b, inst) for b, inst in zip(sample, insts)]
     B, A = shape.B, shape.A
     ended = [False] * len(sample)
     k = 0
@@ -218,14 +123,8 @@ def test_envelope_granular_path(name):
                 if trial == 0:
                     leaders[:] = A - 1
                 env.build_obs(leaders)
-                ag, tk, mk = env.agent_obs[sample].cpu().numpy(), env.task_obs[sample].cpu().numpy(), env.mask_u8[sample].cpu().numpy()
-                for q, o in enumerate(orcs):
-                    if ended[q]:
-                        continue
-                    l, what = int(leaders[sample[q]]), (name, sample[q], k, trial)
-                    assert np.array_equal(mk[q], o.env.mask()), what
-                    assert np.array_equal(ag[q], o.env.agent_status(l).astype(np.float32)), what
-                    assert np.array_equal(tk[q], o.env.task_status(l).astype(np.float32)), what
+                playing = [q for q in range(len(sample)) if not ended[q]]
+                check_obs(env, [orcs[q] for q in playing], [sample[q] for q in playing], (name, k, trial), leader=leaders)
             env.build_obs(np.where(live >= 0, live, 0).astype(np.int32))       # what the step wrote, for the policy of the next step
         env.step(policy=shape.policy)
         done = env.done_u8[sample].cpu().numpy()
@@ -243,9 +142,10 @@ def test_envelope_granular_path(name):
     met = env.compute_metrics()[sample].cpu().numpy()
     for q, o in enumerate(orcs):
         finished, stuck = o.first_end
-        assert flags[q] & 7 == 1 | (2 if finished else 0) | (4 if stuck else 0), (name, sample[q], flags[q])
+        want = ENV_DONE | (ENV_FINISHED if finished else 0) | (ENV_STUCK if stuck else 0)
+        assert flags[q] & (ENV_DONE | ENV_FINISHED | ENV_STUCK) == want, (name, sample[q], flags[q])
         assert_metrics_match(met[q], o.last_metrics, (name, sample[q]))
-    assert not (env.env_flags().cpu().numpy() & ERR_BITS).any()
+    assert not (env.env_flags().cpu().numpy() & ENV_ERR_MASK).any()
     env.close()
 
 
@@ -259,16 +159,13 @@ def test_export_import_at_the_largest_shape():
     for _ in range(150):
         a.step(policy=shape.policy)
     b = BatchedTaskEnv(shape.B, shape.A, shape.T, M=shape.M, auto_reset=True, seed=shape.seed, first_gid=shape.first_gid())
-    inst = {k: v.cpu().numpy() for k, v in a.get_instances().items()}
-    b.load_instances(inst["task_xy"], inst["depot_xy"], inst["req"], inst["dur"])
+    b.load_instances(*stack_instances(instances(a)))
     b.import_raw(a.export_raw())
     assert_same_records(a, b, "after import")
     for k in range(100):
         a.step(policy=shape.policy)
         b.step(policy=shape.policy)
-        oa, ob = outputs(a), outputs(b)
-        for n in oa:
-            assert np.array_equal(oa[n], ob[n]), (n, k)
+        assert_same_outputs(a, b, k)
     assert_same_records(a, b, "after 100 decisions")
     assert np.array_equal(a.episode_metrics().cpu().numpy(), b.episode_metrics().cpu().numpy())
     a.close(); b.close()
